@@ -187,6 +187,30 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ our arm
+DUMP_SAMPLE = 1 << 18      # elements --dump-outputs keeps of a larger tensor: 40 tensors of at most 1 MB
+
+
+def dump_outputs(out_dir, losses, model):
+    """What the last timed step computed, as float32 DIR/<name>.npy: `losses` (verb, nouns, gt-nouns loss) and, for
+    every trainable tensor, `param.<name>` (the weights after the optimizer step) and `grad.<name>` (rank 0's gradient
+    buffer).  A tensor of more than DUMP_SAMPLE elements is reduced to a fixed, seeded sample of that many flat
+    elements, in index order."""
+    import numpy as np
+    import torch
+    arrays = {"losses": losses}
+    for name, p in model.named_parameters():
+        if p.requires_grad:
+            arrays["param." + name] = p
+            arrays["grad." + name] = p.grad
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -230,6 +254,18 @@ def run_ours(args):
     sharded = world > 1 and not args.replicated_optimizer
     opt = parallel.FlatAdamax(flat, lr=0.002, max_norm=1.0, group=dist.group.WORLD if sharded else None)
     params = [p for p in model.parameters() if p.requires_grad]
+    # --dump-outputs: the last timed step starts again from the seeded initial weights and optimizer state.  The steps
+    # before it are as many as the pre-heat's time allows, and atomic / split-K reduce-add sums have no fixed order, so
+    # the state they leave differs from run to run; the state they start from does not.  The copies back (~0.5 GB) fall
+    # inside the timed window, once.
+    dump_state = None
+    if args.dump_outputs:
+        dump_state = [(t, t.clone()) for t in (flat.flat_param, opt.exp_avg, opt.exp_inf, opt.scratch)]
+
+    def restore_dump_state():
+        for t, saved in dump_state:
+            t.copy_(saved)
+        flat.version += 1                                       # the packed bf16 weights are stale
 
     Bg = args.batch
     lo, hi = parallel.shard_range(Bg, rank, world)
@@ -260,14 +296,17 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, k):
+    def timed(fn, k, before_last=None):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         t0 = time.perf_counter()
-        for _ in range(k):
-            fn()
+        for i in range(k):
+            if i == k - 1 and before_last is not None:
+                before_last()
+            out = fn()
         timed.host_issue_ms = (time.perf_counter() - t0) * 1e3   # host time to QUEUE the k steps (no sync inside)
+        timed.last_out = out
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -285,6 +324,9 @@ def run_ours(args):
         run_resident = lambda: step(resident)
     for _ in range(max(3, args.warmup)):
         run_resident()
+    if dump_state is not None:
+        # the dropout seed counter exists from the first step on and advances by one per step
+        dump_state += [(t, t.clone()) for t in model._seed_state.values()]
     # pre-heat: the same step, back to back for >= args.preheat seconds, so that the timed region starts in the
     # sustained clock / power state at every N (a 0.1 s window after an idle GPU runs at boost clocks)
     t_probe = timed(run_resident, 2) / 2
@@ -300,8 +342,10 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     n0 = lib.srg_launch_count()
-    total_ms = timed(run_resident, args.steps)
+    total_ms = timed(run_resident, args.steps, restore_dump_state if dump_state is not None else None)
     host_issue_ms = timed.host_issue_ms / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, timed.last_out, model)
     launches = (lib.srg_launch_count() - n0)
     if use_graph:
         launches = gstep.launches * args.steps
@@ -435,7 +479,13 @@ def main():
                     help="N > 1: all-reduce the gradient and run clip + Adamax on every rank (round-1 scheme)")
     ap.add_argument("--graph", action="store_true", help="replay the whole training step from one CUDA graph")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the losses, weights and gradients of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
