@@ -121,6 +121,32 @@ int srg_verb_forward(srg_handle* h, const float* feat, int B, const uint8_t* kee
                      const int64_t* drop_seed, int64_t drop_stream, float* logits, int64_t ldl, int precision,
                      int save_for_backward, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Row-wise top-k + log-softmax: for each of `rows` rows of logits [rows, ldl], the k largest of the first n columns in
+ * descending order (ties go to the lower column, as torch.argmax and a stable descending sort) and their log-softmax
+ * over those n columns (fp32, accurate expf / logf).  Columns >= n are never read, so padding may hold anything;
+ * -inf entries are allowed.  1 <= k <= 16, k <= n <= ldl.  idx int64 [rows, k], logp fp32 [rows, k]. */
+int srg_topk_logsoftmax(const float* logits, int64_t ldl, int rows, int n, int k, int64_t* idx, float* logp,
+                        void* stream);
+
+/* Top-k situation decode (a situation = a verb + one label per role of that verb).
+ * srg_situation_nouns runs the role graphs of the B*k (image, verb) pairs verbs[b*k + j] (int64 [B, k]) in eval mode
+ * (no dropout): it is srg_nouns_forward on B*k graphs whose node init reads feat[b] (fp32 [B, D]; the features are
+ * not copied k times), followed by a decode.  Per candidate:
+ *   labels     int64 [B, k, R]: top-1 label of every role slot, -1 on the pad slots (r >= role_count[verb]);
+ *   label_logp fp32  [B, k, R]: its log-softmax over the n_labels labels, 0 on the pad slots;
+ *   score      fp32  [B, k]   : (verb_logp ? verb_logp[b*k + j] : 0) + the sum of the real slots' label_logp.
+ * verb_logp (nullable) fp32 [B, k].  Out-of-range verb ids are clamped and flagged as in srg_nouns_forward
+ * (srg_check_verbs).  1 <= k <= min(16, n_verbs); both precisions.
+ * Workspace (srg_situation_workspace_bytes, enough at any 16-byte aligned address): the forward buffers of B*k role
+ * graphs plus their noun logits
+ * [B*k*R, n_labels padded to 256] fp32.  At D = 2048, R = 6, 2001 labels, B = 6144, k = 5 that is about 7.5 GB in bf16
+ * (184 k slot rows of state, operand copies and logits; estimated from the buffer list, not measured); the fp32-parity
+ * mode needs more for its split operands. */
+size_t srg_situation_workspace_bytes(srg_handle* h, int B, int k, int precision);
+int srg_situation_nouns(srg_handle* h, const float* feat, const int64_t* verbs, int B, int k, const float* role_emb,
+                        const float* verb_emb, const float* verb_logp, int64_t* labels, float* label_logp,
+                        float* score, int precision, void* workspace, size_t workspace_bytes, void* stream);
+
 /* The keep-mask the Philox path applies for (*drop_seed, drop_stream, drop_p) on a [rows, D] slot matrix, written as
  * uint8 0/1 (tests: lets the oracle replay exactly the dropout a training step used). */
 int srg_dropout_mask(const int64_t* drop_seed, int64_t drop_stream, float drop_p, int64_t rows, int D, uint8_t* keep,

@@ -41,6 +41,9 @@ SIGNATURES = {
     "srg_workspace_bytes": (_sz, [_vp, _i, _i, _i, _i]),
     "srg_nouns_forward": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _f, _vp, _i64, _vp, _i64, _i, _i, _vp, _sz, _vp]),
     "srg_verb_forward": (_i, [_vp, _vp, _i, _vp, _f, _vp, _i64, _vp, _i64, _i, _i, _vp, _sz, _vp]),
+    "srg_topk_logsoftmax": (_i, [_vp, _i64, _i, _i, _i, _vp, _vp, _vp]),
+    "srg_situation_workspace_bytes": (_sz, [_vp, _i, _i, _i]),
+    "srg_situation_nouns": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _sz, _vp]),
     "srg_dropout_mask": (_i, [_vp, _i64, _f, _i64, _i, _vp, _vp]),
     "srg_ggnn_forward": (_i, [_vp, _i, _vp, _vp, _i, _i, _i, _vp, _sz, _vp]),
     "srg_count_targets": (_i, [_vp, _vp, _i, _vp, _vp]),

@@ -837,6 +837,41 @@ size_t srg_workspace_bytes(srg_handle* h, int mode, int B, int precision, int sa
   return carve(h, mode, B, precision, save_for_backward, nullptr, mode == SRG_MODE_NOUN).bytes;
 }
 
+}  // extern "C"
+
+namespace {
+// predict_nouns minus the backbone on the B role graphs of `verb` (B = images x candidates): role graph b reads feature
+// row b / feat_rep.  Shared by srg_nouns_forward (feat_rep = 1) and srg_situation_nouns (feat_rep = k).
+int nouns_forward_body(srg_handle* h, PathBufs& pb, const float* feat, int feat_rep, const int64_t* verb, int B,
+                       const float* role_emb, const float* verb_emb, const DropSpec& ds, float* logits, int64_t ldl,
+                       int precision, int save_for_backward, cudaStream_t s) {
+  // role counts -> compact row layout (device-resident: the predicted verbs never visit the host)
+  SRG_TRY(launch_prep_rows(h->d_role_count, h->V, h->R, verb, B, h->compact, pb.rm, h->d_bad, s));
+  SRG_TRY(launch_node_init_noun(feat, role_emb, verb_emb, verb, h->d_verb2roles, h->V, B, h->R, h->D, pb.rm, feat_rep,
+                                pb.h32, pb.hb_hi[0], pb.hb_mid[0], pb.hb_lo[0], s));
+  SRG_TRY(ggnn_steps(h, SRG_MODE_NOUN, pb, pb.h32, nullptr, B, precision, save_for_backward, s));
+  return classifier_forward(h, SRG_MODE_NOUN, pb, pb.h32, ds, logits, ldl, precision, s);
+}
+
+// srg_situation_nouns' workspace: the role-graph buffers of B*k graphs (carve), then the noun logits [B*k*R, Lpad].
+// Returns the bytes a workspace at ANY 16-byte aligned address needs: carve's size of the buffers alone (used + 1024
+// bytes of slack for the 1024-byte alignment of the first buffer) plus the logits.  With ws != nullptr, *pb / *logits
+// receive the layout in `ws`: carve starts at the alignment pad a <= 1023 and ends at ws + a + used (1024-aligned), where
+// the logits begin; they end at a + used + logit_bytes < the returned size.
+size_t situation_layout(const srg_handle* h, int B, int k, int prec, void* ws, PathBufs* pb, float** logits) {
+  const int n = B * k;
+  const size_t logit_bytes = static_cast<size_t>(n) * h->R * h->Lpad * sizeof(float);
+  if (ws != nullptr) {
+    const PathBufs p = carve(h, SRG_MODE_NOUN, n, prec, 0, ws, true);   // p.bytes = a + used + 1024
+    if (pb) *pb = p;
+    if (logits) *logits = reinterpret_cast<float*>(static_cast<uint8_t*>(ws) + p.bytes - 1024);
+  }
+  return carve(h, SRG_MODE_NOUN, n, prec, 0, nullptr, true).bytes + logit_bytes;
+}
+}  // namespace
+
+extern "C" {
+
 int srg_nouns_forward(srg_handle* h, const float* feat, const int64_t* verb, int B, const float* role_emb,
                       const float* verb_emb, const uint8_t* keep, float drop_p, const int64_t* drop_seed,
                       int64_t drop_stream, float* logits, int64_t ldl, int precision, int save_for_backward,
@@ -850,13 +885,43 @@ int srg_nouns_forward(srg_handle* h, const float* feat, const int64_t* verb, int
   SRG_CHECK(feat && verb && role_emb && verb_emb && logits, "srg_nouns_forward: null argument");
   DropSpec ds;
   SRG_TRY(make_drop(keep, drop_p, drop_seed, drop_stream, &ds));
+  return nouns_forward_body(h, pb, feat, 1, verb, B, role_emb, verb_emb, ds, logits, ldl, precision, save_for_backward,
+                            static_cast<cudaStream_t>(stream));
+}
+
+int srg_topk_logsoftmax(const float* logits, int64_t ldl, int rows, int n, int k, int64_t* idx, float* logp,
+                        void* stream) {
+  SRG_CHECK(rows >= 0, "srg_topk_logsoftmax: negative row count %d", rows);
+  SRG_CHECK(rows == 0 || (logits && idx && logp), "srg_topk_logsoftmax: null argument");
+  return launch_row_topk_logsoftmax(logits, ldl, rows, n, k, idx, logp, static_cast<cudaStream_t>(stream));
+}
+
+size_t srg_situation_workspace_bytes(srg_handle* h, int B, int k, int precision) {
+  if (!h || B <= 0 || k < 1 || k > 16) return 0;
+  return situation_layout(h, B, k, precision, nullptr, nullptr, nullptr);
+}
+
+int srg_situation_nouns(srg_handle* h, const float* feat, const int64_t* verbs, int B, int k, const float* role_emb,
+                        const float* verb_emb, const float* verb_logp, int64_t* labels, float* label_logp,
+                        float* score, int precision, void* workspace, size_t workspace_bytes, void* stream) {
+  SRG_CHECK(h != nullptr, "srg_situation_nouns: null handle");
+  DeviceGuard guard_(h->device);
+  SRG_CHECK(k >= 1 && k <= 16 && k <= h->V, "srg_situation_nouns: k=%d must be in [1, min(16, n_verbs=%d)]", k, h->V);
+  SRG_CHECK(B > 0 && static_cast<int64_t>(B) * k * h->R <= (1 << 30), "srg_situation_nouns: bad batch %d", B);
+  PathBufs pb;
+  SRG_TRY(check_ws(h, SRG_MODE_NOUN, B * k, precision, 0, workspace, workspace_bytes, &pb, true));
+  float* nl = nullptr;
+  const size_t need = situation_layout(h, B, k, precision, workspace, &pb, &nl);
+  if (need > workspace_bytes)
+    return set_error(SRG_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  SRG_CHECK(h->tables_set, "srg_situation_nouns: call srg_set_tables first");
+  SRG_CHECK(h->packed_prec == precision, "srg_situation_nouns: weights are not packed for precision %d", precision);
+  SRG_CHECK(feat && verbs && role_emb && verb_emb && labels && label_logp && score, "srg_situation_nouns: null argument");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  // role counts -> compact row layout (device-resident: the predicted verbs never visit the host)
-  SRG_TRY(launch_prep_rows(h->d_role_count, h->V, h->R, verb, B, h->compact, pb.rm, h->d_bad, s));
-  SRG_TRY(launch_node_init_noun(feat, role_emb, verb_emb, verb, h->d_verb2roles, h->V, B, h->R, h->D, pb.rm, pb.h32,
-                                pb.hb_hi[0], pb.hb_mid[0], pb.hb_lo[0], s));
-  SRG_TRY(ggnn_steps(h, SRG_MODE_NOUN, pb, pb.h32, nullptr, B, precision, save_for_backward, s));
-  return classifier_forward(h, SRG_MODE_NOUN, pb, pb.h32, ds, logits, ldl, precision, s);
+  const int n = B * k;
+  SRG_TRY(nouns_forward_body(h, pb, feat, k, verbs, n, role_emb, verb_emb, DropSpec(), nl, h->Lpad, precision, 0, s));
+  SRG_TRY(launch_row_topk_logsoftmax(nl, h->Lpad, n * h->R, h->L, 1, labels, label_logp, s));
+  return launch_situation_finish(verbs, h->d_role_count, h->V, h->R, n, verb_logp, labels, label_logp, score, s);
 }
 
 int srg_verb_forward(srg_handle* h, const float* feat, int B, const uint8_t* keep, float drop_p,

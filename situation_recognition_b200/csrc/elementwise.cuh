@@ -40,11 +40,12 @@ int launch_gather_mask(const int32_t* verb2roles, const int32_t* role_count, int
 // cnt / off / meta of `rm` from the verb ids (imsitu_encoder.py:158-159 per image + an exclusive scan); one block
 int launch_prep_rows(const int32_t* role_count, int n_verbs, int R, const int64_t* verb, int B, int compact, RowMap rm,
                      int* bad, cudaStream_t s);
-// node[row(b,r), :] = relu(feat[b,:] * role_emb[verb2roles[verb[b], r], :] * verb_emb[verb[b], :])   (model.py:124-144)
-// for the rows `rm` materialises; the self-loop rows are set to 0
+// node[row(b,r), :] = relu(feat[b / feat_rep,:] * role_emb[verb2roles[verb[b], r], :] * verb_emb[verb[b], :])
+// (model.py:124-144) for the rows `rm` materialises; the self-loop rows are set to 0.  feat_rep > 1: consecutive groups
+// of feat_rep graphs share one feature row (the k candidate verbs of an image, srg_situation_nouns)
 int launch_node_init_noun(const float* feat, const float* role_emb, const float* verb_emb, const int64_t* verb,
-                          const int32_t* verb2roles, int n_verbs, int B, int R, int D, RowMap rm, float* h32,
-                          bf16* hb_hi, bf16* hb_mid, bf16* hb_lo, cudaStream_t s);
+                          const int32_t* verb2roles, int n_verbs, int B, int R, int D, RowMap rm, int feat_rep,
+                          float* h32, bf16* hb_hi, bf16* hb_mid, bf16* hb_lo, cudaStream_t s);
 // the same aggregation as launch_aggregate on the rows of `rm`, from the role counts instead of a [B,R,R] mask
 int launch_aggregate_rows(const float* h32, RowMap rm, int B, int R, int D, bf16* a_hi, bf16* a_mid, bf16* a_lo,
                           cudaStream_t s);
@@ -105,6 +106,16 @@ int launch_nouns_ce(const float* logits, int64_t ldl, int n_labels, const int64_
 int launch_verb_ce(const float* logits, int64_t ldl, int n_verbs, const int64_t* gt, int B, float inv_batch,
                    float* loss, float* dlogits, float grad_scale, const float* gscale_dev, const float* stats,
                    int stats_tiles, const float* batch_total, bf16* dlb, int n_pad, int accumulate, cudaStream_t s);
+// Per row of x [rows, ldl]: the k largest of the first n columns in descending order (ties: lower column first, as
+// torch.argmax) and their log-softmax over those n columns.  Columns >= n are never read.  1 <= k <= 16, k <= n.
+// idx int64 [rows, k], logp fp32 [rows, k].
+int launch_row_topk_logsoftmax(const float* x, int64_t ldl, int rows, int n, int k, int64_t* idx, float* logp,
+                               cudaStream_t s);
+// Decode of the situation candidates u < n_cand (verb[u]): slots r >= role_count[verb[u]] get label -1 and log-prob 0;
+// score[u] = (verb_logp ? verb_logp[u] : 0) + sum of the real slots' label log-probs.  labels / label_logp [n_cand, R]
+// hold the per-slot top-1 on entry and are finished in place.
+int launch_situation_finish(const int64_t* verb, const int32_t* role_count, int n_verbs, int R, int n_cand,
+                            const float* verb_logp, int64_t* labels, float* label_logp, float* score, cudaStream_t s);
 // fp32 [rows, ld] (first n_valid columns) -> bf16 [rows, n_pad], zero padded
 int launch_cast_pad(const float* src, int64_t ld, int rows, int n_valid, int n_pad, bf16* dst, int accumulate,
                     cudaStream_t s);

@@ -176,7 +176,7 @@ __device__ __forceinline__ void store8_split(bf16* hi, Parts parts, int64_t idx,
 __global__ void k_node_init_noun(const float* __restrict__ feat, const float* __restrict__ role_emb,
                                  const float* __restrict__ verb_emb, const int64_t* __restrict__ verb,
                                  const int32_t* __restrict__ verb2roles, int n_verbs, int B, int R, int D, RowMap rm,
-                                 float* __restrict__ h32, bf16* __restrict__ hb_hi, Parts hb_lo) {
+                                 int feat_rep, float* __restrict__ h32, bf16* __restrict__ hb_hi, Parts hb_lo) {
   const int D4 = D / 4;
   const int64_t total = static_cast<int64_t>(B + kSelfRows) * D4;
   for (int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; t < total;
@@ -196,7 +196,7 @@ __global__ void k_node_init_noun(const float* __restrict__ feat, const float* __
     const int b = u;
     int64_t v = verb[b];
     if (v < 0 || v >= n_verbs) v = 0;
-    const float4 f = *reinterpret_cast<const float4*>(feat + static_cast<int64_t>(b) * D + d);
+    const float4 f = *reinterpret_cast<const float4*>(feat + static_cast<int64_t>(b / feat_rep) * D + d);
     const float4 ve = *reinterpret_cast<const float4*>(verb_emb + v * D + d);
     const int L = rm.compact ? rm.cnt[b] : R;
     const int base = rm.off[b];
@@ -1024,6 +1024,145 @@ __global__ void k_clip_adamax(float* __restrict__ p, float* __restrict__ g, floa
 
 __global__ void k_inc(float* x) { *x += 1.0f; }
 
+// ------------------------------------------------------------------------------------------------ top-k decode
+// (v, c) ranks before (w, d): larger value, ties to the lower column (torch.argmax / a stable descending sort)
+__device__ __forceinline__ bool topk_before(float v, int c, float w, int d) { return v > w || (v == w && c < d); }
+
+template <int KMAX>
+__device__ __forceinline__ void topk_insert(float (&tv)[KMAX], int (&tc)[KMAX], float v, int c) {
+  if (!topk_before(v, c, tv[KMAX - 1], tc[KMAX - 1])) return;
+#pragma unroll
+  for (int j = 0; j < KMAX; ++j) {   // carry insertion: the candidate swaps with every entry it ranks before
+    if (topk_before(v, c, tv[j], tc[j])) {
+      const float tvj = tv[j];
+      const int tcj = tc[j];
+      tv[j] = v; tc[j] = c;
+      v = tvj; c = tcj;
+    }
+  }
+}
+
+// One warp per row.  Each lane keeps the KMAX best (value, column) pairs of the columns it reads, sorted, in registers
+// (the insertion is unrolled, so the list never leaves them), and a running (max, sum exp(x - max)) of its columns.
+// The row is read in chunks of kTopkChunk values per lane, all loads of a chunk in flight at once; the running sum is
+// rescaled once per chunk, so every column costs one expf.  Then k rounds of a warp argmax over the lane heads; the
+// winning lane pops its head.  The sentinel (-inf, INT_MAX) ranks after every real column, -inf entries included.
+// Every column < n is read exactly once; columns >= n are never read.
+constexpr int kTopkChunk = 64;
+
+template <int KMAX>
+__global__ void __launch_bounds__(kThreads)
+k_row_topk_logsoftmax(const float* __restrict__ x, int64_t ldl, int rows, int n, int k, int64_t* __restrict__ idx,
+                      float* __restrict__ logp) {
+  const int lane = threadIdx.x & 31;
+  const int warps = blockDim.x >> 5;
+  const bool vec = (ldl & 3) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0;
+  for (int row = blockIdx.x * warps + (threadIdx.x >> 5); row < rows; row += gridDim.x * warps) {
+    const float* xr = x + static_cast<int64_t>(row) * ldl;
+    float tv[KMAX];
+    int tc[KMAX];
+#pragma unroll
+    for (int j = 0; j < KMAX; ++j) { tv[j] = -INFINITY; tc[j] = INT_MAX; }
+    float m = -INFINITY, se = 0.f;
+    float v[kTopkChunk];
+    // v[i] holds column col(i) of the current chunk (-inf where the column is >= n); fold the chunk into the state
+    auto fold = [&](auto col) {
+      float cm = -INFINITY;
+#pragma unroll
+      for (int i = 0; i < kTopkChunk; ++i) {
+        cm = fmaxf(cm, v[i]);
+        topk_insert<KMAX>(tv, tc, v[i], col(i));
+      }
+      const float mn = fmaxf(m, cm);
+      if (mn > -INFINITY) {
+        float acc = 0.f;
+#pragma unroll
+        for (int i = 0; i < kTopkChunk; ++i) acc += expf(v[i] - mn);   // -inf -> 0
+        se = se * expf(m - mn) + acc;                                  // m = -inf: se is 0
+        m = mn;
+      }
+    };
+    if (vec) {   // 16-byte loads: lane reads float4 q = q0 + 32 i + lane of the row
+      const int n4 = (n + 3) >> 2;
+      for (int q0 = 0; q0 < n4; q0 += 32 * (kTopkChunk / 4)) {
+#pragma unroll
+        for (int i = 0; i < kTopkChunk / 4; ++i) {
+          const int q = q0 + 32 * i + lane;
+          float4 f = make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
+          if (4 * q + 3 < n) {
+            f = __ldg(reinterpret_cast<const float4*>(xr) + q);
+          } else if (4 * q < n) {   // the row's last, partial float4: scalar loads of the columns < n only
+            f.x = __ldg(xr + 4 * q);
+            if (4 * q + 1 < n) f.y = __ldg(xr + 4 * q + 1);
+            if (4 * q + 2 < n) f.z = __ldg(xr + 4 * q + 2);
+          }
+          v[4 * i] = f.x; v[4 * i + 1] = f.y; v[4 * i + 2] = f.z; v[4 * i + 3] = f.w;
+        }
+        fold([&](int i) { const int c = 4 * (q0 + 32 * (i >> 2) + lane) + (i & 3); return c < n ? c : INT_MAX; });
+      }
+    } else {     // any pitch / alignment: 4-byte loads, lane reads column c0 + 32 i + lane
+      for (int c0 = 0; c0 < n; c0 += 32 * kTopkChunk) {
+#pragma unroll
+        for (int i = 0; i < kTopkChunk; ++i) {
+          const int c = c0 + 32 * i + lane;
+          v[i] = (c < n) ? __ldg(xr + c) : -INFINITY;
+        }
+        fold([&](int i) { const int c = c0 + 32 * i + lane; return c < n ? c : INT_MAX; });
+      }
+    }
+    // log-sum-exp of the row from the per-lane (max, sum) pairs
+    float M = m;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) M = fmaxf(M, __shfl_xor_sync(0xffffffffu, M, o));
+    float S = (m > -INFINITY) ? se * expf(m - M) : 0.f;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) S += __shfl_xor_sync(0xffffffffu, S, o);
+    const float log_s = logf(S);
+    for (int j = 0; j < k; ++j) {
+      float bv = tv[0];
+      int bc = tc[0];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oc = __shfl_xor_sync(0xffffffffu, bc, o);
+        if (topk_before(ov, oc, bv, bc)) { bv = ov; bc = oc; }
+      }
+      if (tc[0] == bc) {                 // columns are unique within a row: exactly one lane pops its head
+#pragma unroll
+        for (int i = 0; i + 1 < KMAX; ++i) { tv[i] = tv[i + 1]; tc[i] = tc[i + 1]; }
+        tv[KMAX - 1] = -INFINITY;
+        tc[KMAX - 1] = INT_MAX;
+      }
+      if (lane == 0) {
+        idx[static_cast<int64_t>(row) * k + j] = bc;
+        logp[static_cast<int64_t>(row) * k + j] = (bv - M) - log_s;
+      }
+    }
+  }
+}
+
+__global__ void k_situation_finish(const int64_t* __restrict__ verb, const int32_t* __restrict__ role_count,
+                                   int n_verbs, int R, int n_cand, const float* __restrict__ verb_logp,
+                                   int64_t* __restrict__ labels, float* __restrict__ label_logp,
+                                   float* __restrict__ score) {
+  for (int u = blockIdx.x * blockDim.x + threadIdx.x; u < n_cand; u += gridDim.x * blockDim.x) {
+    int64_t v = verb[u];
+    if (v < 0 || v >= n_verbs) v = 0;    // clamped as in the role graph (k_prep_rows raised the flag)
+    const int n = role_count[v];
+    float s = (verb_logp != nullptr) ? verb_logp[u] : 0.f;
+    for (int r = 0; r < R; ++r) {
+      const int64_t o = static_cast<int64_t>(u) * R + r;
+      if (r < n) {
+        s += label_logp[o];
+      } else {
+        labels[o] = -1;
+        label_logp[o] = 0.f;
+      }
+    }
+    score[u] = s;
+  }
+}
+
 #define SRG_LAUNCH_CHECK()                                                                      \
   do {                                                                                          \
     g_launches.fetch_add(1, std::memory_order_relaxed);                                         \
@@ -1128,6 +1267,30 @@ int launch_verb_ce(const float* logits, int64_t ldl, int n_verbs, const int64_t*
   return SRG_OK;
 }
 
+int launch_row_topk_logsoftmax(const float* x, int64_t ldl, int rows, int n, int k, int64_t* idx, float* logp,
+                               cudaStream_t s) {
+  if (rows <= 0) return SRG_OK;
+  if (k < 1 || k > 16 || n < k || ldl < n)
+    return set_error(SRG_ERR_ARG, "topk_logsoftmax: need 1 <= k <= 16, k <= n <= ldl (k=%d, n=%d, ldl=%lld)", k, n,
+                     (long long)ldl);
+  const int blocks = grid_for(static_cast<int64_t>(rows) * 32);   // one warp per row
+  if (k == 1) k_row_topk_logsoftmax<1><<<blocks, kThreads, 0, s>>>(x, ldl, rows, n, k, idx, logp);
+  else if (k <= 4) k_row_topk_logsoftmax<4><<<blocks, kThreads, 0, s>>>(x, ldl, rows, n, k, idx, logp);
+  else if (k <= 8) k_row_topk_logsoftmax<8><<<blocks, kThreads, 0, s>>>(x, ldl, rows, n, k, idx, logp);
+  else k_row_topk_logsoftmax<16><<<blocks, kThreads, 0, s>>>(x, ldl, rows, n, k, idx, logp);
+  SRG_LAUNCH_CHECK();
+  return SRG_OK;
+}
+
+int launch_situation_finish(const int64_t* verb, const int32_t* role_count, int n_verbs, int R, int n_cand,
+                            const float* verb_logp, int64_t* labels, float* label_logp, float* score, cudaStream_t s) {
+  if (n_cand <= 0) return SRG_OK;
+  k_situation_finish<<<grid_for(n_cand), kThreads, 0, s>>>(verb, role_count, n_verbs, R, n_cand, verb_logp, labels,
+                                                          label_logp, score);
+  SRG_LAUNCH_CHECK();
+  return SRG_OK;
+}
+
 int launch_cast_pad(const float* src, int64_t ld, int rows, int n_valid, int n_pad, bf16* dst, int accumulate,
                     cudaStream_t s) {
   if (rows <= 0) return SRG_OK;
@@ -1159,12 +1322,13 @@ int launch_prep_rows(const int32_t* role_count, int n_verbs, int R, const int64_
 }
 
 int launch_node_init_noun(const float* feat, const float* role_emb, const float* verb_emb, const int64_t* verb,
-                          const int32_t* verb2roles, int n_verbs, int B, int R, int D, RowMap rm, float* h32,
-                          bf16* hb_hi, bf16* hb_mid, bf16* hb_lo, cudaStream_t s) {
+                          const int32_t* verb2roles, int n_verbs, int B, int R, int D, RowMap rm, int feat_rep,
+                          float* h32, bf16* hb_hi, bf16* hb_mid, bf16* hb_lo, cudaStream_t s) {
   if (B <= 0) return SRG_OK;
   if (R > kMaxR) return set_error(SRG_ERR_UNSUPPORTED, "max_role_count %d > %d", R, kMaxR);
+  if (feat_rep < 1) return set_error(SRG_ERR_ARG, "node_init_noun: feat_rep %d < 1", feat_rep);
   k_node_init_noun<<<grid_for(static_cast<int64_t>(B + kSelfRows) * D / 4), kThreads, 0, s>>>(
-      feat, role_emb, verb_emb, verb, verb2roles, n_verbs, B, R, D, rm, h32, hb_hi, Parts{hb_mid, hb_lo});
+      feat, role_emb, verb_emb, verb, verb2roles, n_verbs, B, R, D, rm, feat_rep, h32, hb_hi, Parts{hb_mid, hb_lo});
   SRG_LAUNCH_CHECK();
   return SRG_OK;
 }

@@ -17,6 +17,7 @@ Differences a caller can observe (all documented in DESIGN.md):
 import ctypes
 import os
 import warnings
+from collections import namedtuple
 
 import torch
 import torch.nn as nn
@@ -27,6 +28,16 @@ from .imsitu_encoder import tables_from_encoder
 
 T_STEPS = 4  # model.py:60
 _POISON_WS = os.environ.get("SRG_POISON_WS", "0") == "1"
+
+
+Situations = namedtuple("Situations", ["verbs", "verb_logp", "labels", "label_logp", "score"])
+Situations.__doc__ = """Top-k situations of a batch (FCGGNN.situations_from_features / predict_situations).
+    verbs [B,k] int64 (descending verb logit, ties to the lower id); verb_logp [B,k] fp32 log-softmax over the verbs, or
+    None when the verbs were given; labels [B,k,R] int64 top-1 label per role slot, -1 on pad slots; label_logp [B,k,R]
+    fp32 its log-softmax over the labels, 0 on pad slots; score [B,k] = verb_logp + sum over the real slots of
+    label_logp (label term only when the verbs were given)."""
+
+MAX_TOPK = 16
 
 
 def _pad256(n):
@@ -180,8 +191,12 @@ class _Engine:
         """Current stream of THIS engine's device (the caller's current device may be another GPU)."""
         return _lib.stream_ptr(self.device)
 
-    def workspace(self, mode, B, prec, save):
-        n = self.lib.srg_workspace_bytes(self.h, mode, B, prec, int(save))
+    def workspace(self, mode, B, prec, save, k=None):
+        """Uninitialised device workspace of one call; k: srg_situation_nouns on B images x k candidate verbs."""
+        if k is None:
+            n = self.lib.srg_workspace_bytes(self.h, mode, B, prec, int(save))
+        else:
+            n = self.lib.srg_situation_workspace_bytes(self.h, B, k, prec)
         ws = torch.empty(n, dtype=torch.uint8, device=self.device)
         if _POISON_WS:      # tests: every byte 0xFF = NaN as fp32 / bf16, -1 as int32: a read of a workspace location
             ws.fill_(0xFF)  # nobody wrote shows up as NaN in the results instead of hiding behind fresh (zeroed) memory
@@ -738,6 +753,63 @@ class FCGGNN(nn.Module):
         tap, side = self._tap_of(pred_nouns, stats)
         return _NounsLoss.apply(self, torch.is_grad_enabled(), pred_nouns, gt_nouns.to(pred_nouns.device), stats, tap,
                                 side)
+
+    # ---- top-k situation decode ----------------------------------------------------------------
+    @torch.no_grad()
+    def situations_from_features(self, feat_verbs, feat_nouns, k=5, verbs=None):
+        """The k best situations of each image from the backbone features ([B, D] each): the verb path, the top k
+        verbs with their log-softmax, then the role graphs of all B*k (image, verb) pairs in one call (the node init
+        reads each image's feature row k times instead of copying it) and the top-1 label of every role slot.
+        verbs ([B, k'] int64, optional): decode these candidate verbs instead (feat_verbs is then not used and may be
+        None; verb_logp is None and the score is the label term only) -- e.g. `verbs=gt_verb[:, None]` for the
+        ground-truth-verb decode of the imSitu gt-value metrics.
+
+        Inference only, in train mode too: no autograd node is built and no dropout is applied.  Honours
+        `self.precision`, and makes no host synchronisation (it can be captured in a CUDA graph).  Returns
+        `Situations`."""
+        fn = _as_feat(feat_nouns, self.D)
+        dev = fn.device
+        eng = self._engine_for(dev)
+        B = fn.shape[0]
+        if verbs is not None:
+            verbs = verbs.to(device=dev, dtype=torch.int64).contiguous()
+            if verbs.dim() != 2 or verbs.shape[0] != B:
+                raise _lib.SrgError("verbs must be [B, k] = [%d, k], got %s" % (B, tuple(verbs.shape)))
+            k = verbs.shape[1]
+        if not 1 <= k <= min(MAX_TOPK, eng.V):
+            raise _lib.SrgError("k=%d must be in [1, %d]" % (k, min(MAX_TOPK, eng.V)))
+        prec = _prec_code(self.precision)
+        eng.ensure_packed(self, prec)
+        stream = eng.stream()
+        verb_logp = None
+        if verbs is None:
+            fv = _as_feat(feat_verbs, self.D)
+            if fv.shape[0] != B:
+                raise _lib.SrgError("feat_verbs has %d rows, feat_nouns %d" % (fv.shape[0], B))
+            logits = torch.empty(B, eng.Vpad, dtype=torch.float32, device=dev)
+            ws = eng.workspace(SRG_MODE_VERB, B, prec, False)
+            _lib.check(eng.lib.srg_verb_forward(eng.h, _lib.ptr(fv), B, None, 0.0, None, 0, _lib.ptr(logits), eng.Vpad,
+                                                prec, 0, _lib.ptr(ws), ws.numel(), stream))
+            verbs = torch.empty(B, k, dtype=torch.int64, device=dev)
+            verb_logp = torch.empty(B, k, dtype=torch.float32, device=dev)
+            _lib.check(eng.lib.srg_topk_logsoftmax(_lib.ptr(logits), eng.Vpad, B, eng.V, k, _lib.ptr(verbs),
+                                                   _lib.ptr(verb_logp), stream))
+        labels = torch.empty(B, k, eng.R, dtype=torch.int64, device=dev)
+        label_logp = torch.empty(B, k, eng.R, dtype=torch.float32, device=dev)
+        score = torch.empty(B, k, dtype=torch.float32, device=dev)
+        ws = eng.workspace(SRG_MODE_NOUN, B, prec, False, k=k)
+        _lib.check(eng.lib.srg_situation_nouns(eng.h, _lib.ptr(fn), _lib.ptr(verbs), B, k, _lib.ptr(self.role_emb.weight),
+                                               _lib.ptr(self.verb_emb.weight), _lib.ptr(verb_logp), _lib.ptr(labels),
+                                               _lib.ptr(label_logp), _lib.ptr(score), prec, _lib.ptr(ws), ws.numel(),
+                                               stream))
+        return Situations(verbs, verb_logp, labels, label_logp, score)
+
+    @torch.no_grad()
+    def predict_situations(self, img, k=5, img_nouns=None):
+        """`situations_from_features` from images, through the two frozen backbones (same rules: no autograd, no
+        dropout, no host synchronisation)."""
+        fv, fn = self.extract_features(img, img_nouns)
+        return self.situations_from_features(fv, fn, k=k)
 
     # ---- GGSNN.forward drop-in (inference) ------------------------------------------------------
     def _ggsnn_forward(self, hidden_state, mask=None, verb=False):

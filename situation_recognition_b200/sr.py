@@ -14,7 +14,9 @@ ways.  Differences, all forced by the B200-first design:
   * the features of the frozen backbones on the dev / test images are cached across epochs (`features.FeatureCache`):
     the per-epoch validation (sr.py:123) runs the backbones once, not once per epoch;
   * `--no_pretrained` (extra flag) skips the ImageNet weights when there is no network; `--no_feature_cache` disables
-    the cache.
+    the cache;
+  * `--topk_situations K` (extra flag, default 0 = off) adds the standard imSitu top-k situation metrics
+    (`situations.SituationScorer`) to --evaluate_dev / --evaluate_test, and K situations per image to --test_img.
 """
 import os
 from argparse import ArgumentParser
@@ -32,6 +34,7 @@ from .imsitu_encoder import imsitu_encoder
 from .imsitu_loader import ShardedBatchSampler, imsitu_loader
 from .imsitu_scorer import imsitu_scorer
 from .model import FCGGNN
+from .situations import SituationScorer
 from .utils import format_dict, load_net
 
 
@@ -167,13 +170,16 @@ def _plot(hist, path):
     plt.clf()
 
 
-def eval(model, loader, encoder, logging=False, cache=None):
+def eval(model, loader, encoder, logging=False, cache=None, topk_situations=0):
     """sr.py:165-232.  cache (FeatureCache, optional): the frozen backbones' features of this loader's images are kept
-    across calls; once every image is cached the loader stops decoding images altogether."""
+    across calls; once every image is cached the loader stops decoding images altogether.
+    topk_situations K > 0: also decode the top-K situations of every image (and the gt-verb situation) from the same
+    backbone features and print the standard imSitu top-1 / top-K metrics after the existing lines."""
     model.eval()
     dev = next(model.parameters()).device
     sums = torch.zeros(3, device=dev)
     top1, top5 = imsitu_scorer(encoder, 1, 3), imsitu_scorer(encoder, 5, 3)
+    sit = SituationScorer(encoder, (1, topk_situations)) if topk_situations > 0 else None
     dataset = getattr(loader, "dataset", None)
     if cache is not None and dataset is not None and hasattr(dataset, "skip_images"):
         dataset.skip_images = cache.has(dataset.imgs_names)       # read by the workers this iteration starts
@@ -185,8 +191,14 @@ def eval(model, loader, encoder, logging=False, cache=None):
             if cache is not None:
                 fv, fn = cache.features(model, list(names), img.to(dev, non_blocking=True) if img.numel() else None)
                 pred_verb, pred_nouns, pred_gt_nouns = model.forward_features(fv, fn, verb)
+            elif sit is not None:      # the backbones run once for both decodes
+                fv, fn = model.extract_features(img.to(dev, non_blocking=True))
+                pred_verb, pred_nouns, pred_gt_nouns = model.forward_features(fv, fn, verb)
             else:
                 pred_verb, pred_nouns, pred_gt_nouns = model(img.to(dev, non_blocking=True), verb)
+            if sit is not None:
+                sit.add_point(model.situations_from_features(fv, fn, k=topk_situations), verb, nouns,
+                              model.situations_from_features(None, fn, verbs=verb[:, None]))
             top1.add_point_both(pred_verb, verb, pred_nouns, nouns, pred_gt_nouns)
             top5.add_point_both(pred_verb, verb, pred_nouns, nouns, pred_gt_nouns)
             sums += torch.stack([model.verb_loss(pred_verb, verb), model.nouns_loss(pred_nouns, nouns),
@@ -202,7 +214,19 @@ def eval(model, loader, encoder, logging=False, cache=None):
         top1_a, top5_a = top1.get_average_results_both(), top5.get_average_results_both()
         avg_score = _avg_score(top1_a, top5_a)
         _print_scores('val losses = [v: {:.2f}, n: {:.2f}, gt: {:.2f}]', (v, n, g), top1_a, top5_a, avg_score, '')
+    if sit is not None:
+        _print_situation_scores(_merge_scorer(sit))
     return top1, top5, val_losses, avg_score
+
+
+def _print_situation_scores(sit):
+    """The standard imSitu block: top-1 / top-K verb, value, value-all, then gt-value, gt-value-all and the mean."""
+    a = {key: 100 * x for key, x in sit.get_average_results().items()}
+    _print0('top-k situations (imSitu definitions):')
+    for k in sit.ks:
+        _print0('top-{}: verb: {:.2f}, value: {:.2f}, value-all: {:.2f}'.format(
+            k, a['verb@%d' % k], a['value@%d' % k], a['value-all@%d' % k]))
+    _print0('gt-value: {:.2f}, gt-value-all: {:.2f}, mean = {:.2f}'.format(a['gt-value'], a['gt-value-all'], a['mean']))
 
 
 def _spaces(dataset_folder):
@@ -249,6 +273,41 @@ def results(model, image, encoder, gt_verb, dataset_folder="imSitu"):
     roles = list(verbs_space[verb_name]["roles"].keys())
     labels = {roles[c]: _gloss(encoder, nouns_space, int(i)) for c, i in enumerate(nouns_tensor[:len(roles)])}
     return verb_name, verb_prob, labels, labels_prob
+
+
+def results_topk(model, image, encoder, k, gt_verb="", dataset_folder="imSitu"):
+    """The k best situations of one image: [(verb, verb probability % or None, score, {role: (gloss, label
+    probability %)})].  With a known `gt_verb` only that verb's situation.  Probabilities are softmaxes over the
+    verbs / over the labels."""
+    from PIL import Image
+    model.eval()
+    dev = next(model.parameters()).device
+    nouns_space, verbs_space = _spaces(dataset_folder)
+    img = encoder.dev_transform(Image.open(image).convert('RGB')).unsqueeze(0).to(dev)
+    fv, fn = model.extract_features(img)
+    if gt_verb and encoder.verb_list.count(gt_verb):
+        s = model.situations_from_features(fv, fn, verbs=torch.tensor([[encoder.verb_list.index(gt_verb)]], device=dev))
+    else:
+        s = model.situations_from_features(fv, fn, k=k)
+    verbs, labels, label_logp, score = s.verbs[0].tolist(), s.labels[0].tolist(), s.label_logp[0].exp().tolist(), \
+        s.score[0].tolist()
+    verb_p = s.verb_logp[0].exp().tolist() if s.verb_logp is not None else [None] * len(verbs)
+    out = []
+    for j, v in enumerate(verbs):
+        name = encoder.verb_list[v]
+        roles = list(verbs_space[name]["roles"].keys())
+        out.append((name, None if verb_p[j] is None else 100 * verb_p[j], score[j],
+                    {roles[r]: (_gloss(encoder, nouns_space, labels[j][r]), 100 * label_logp[j][r])
+                     for r in range(len(roles))}))
+    return out
+
+
+def _print_situations(sits):
+    for j, (verb, verb_p, score, roles) in enumerate(sits):
+        vp = 'given' if verb_p is None else '{:.2f}%'.format(verb_p)
+        print('situation {} ({}): {}, log-score = {:.4f}'.format(j + 1, vp, verb, score))
+        for role, (gloss, p) in roles.items():
+            print('  {} ({:.2f}%): {}'.format(role, p, gloss))
 
 
 def analize_subset(model, dev_set, encoder, size, dataset_folder="imSitu", imgset_dir="resized_256"):
@@ -325,6 +384,9 @@ def build_parser():
                         help="recompute the frozen backbones on the dev set at every epoch, like the reference")
     parser.add_argument("--torch_optimizer", action="store_true",
                         help="torch.optim.Adamax + clip_grad_norm_ + gradient all-reduce instead of the fused sharded step")
+    parser.add_argument("--topk_situations", type=int, default=0,
+                        help="K > 0: with --evaluate_dev / --evaluate_test also report the standard imSitu top-1 / top-K "
+                             "situation metrics (2 <= K <= 16); with --test_img print the K best situations (K <= 16)")
     return parser
 
 
@@ -335,7 +397,13 @@ def _loader(dataset, batch_size, shuffle, num_workers):
 
 
 def main(argv=None):
-    args = build_parser().parse_args(argv)
+    parser = build_parser()
+    args = parser.parse_args(argv)
+    if not 0 <= args.topk_situations <= 16:
+        parser.error("--topk_situations must be in [0, 16], got %d" % args.topk_situations)
+    if args.topk_situations == 1 and (args.evaluate_dev or args.evaluate_test):
+        # the block reports top-1 and top-K and the mean of those 8 numbers; K = 1 would print a different mean
+        parser.error("--topk_situations with --evaluate_dev / --evaluate_test needs K >= 2 (top-1 is always reported)")
     if not torch.cuda.is_available():
         raise SystemExit("situation_recognition_b200.sr needs a B200 GPU: the GGNN stage has no CPU path")
     if "RANK" in os.environ and int(os.environ.get("WORLD_SIZE", "1")) > 1:
@@ -397,10 +465,10 @@ def main(argv=None):
 
     if args.evaluate_dev:
         _print0('=> evaluating model with dev-set...')
-        eval(model, dev_loader, encoder, logging=True)
+        eval(model, dev_loader, encoder, logging=True, topk_situations=args.topk_situations)
     elif args.evaluate_test:
         _print0('=> evaluating model with test-set...')
-        eval(model, test_loader, encoder, logging=True)
+        eval(model, test_loader, encoder, logging=True, topk_situations=args.topk_situations)
     elif args.test_img:
         verb, verb_prob, labels, labels_prob = results(model, args.test_img, encoder, args.verb, args.dataset_folder)
         print('&' * 50)
@@ -410,6 +478,11 @@ def main(argv=None):
         print('action ({:.2f}%): {}'.format(verb_prob, verb))
         for c, (k, v) in enumerate(labels.items()):
             print('{} ({:.2f}%): {}'.format(k, labels_prob[c], v))
+        if args.topk_situations > 0:
+            with torch.no_grad():
+                sits = results_topk(model, args.test_img, encoder, args.topk_situations, args.verb, args.dataset_folder)
+            print('&' * 50)
+            _print_situations(sits)
     elif args.subset > 0:
         analize_subset(model, dev_set, encoder, args.subset, args.dataset_folder, args.imgset_dir)
     else:
