@@ -157,6 +157,15 @@ int srg_dropout_mask(const int64_t* drop_seed, int64_t drop_stream, float drop_p
 int srg_ggnn_forward(srg_handle* h, int mode, float* hidden, const float* mask, int B, int precision,
                      int save_for_backward, void* workspace, size_t workspace_bytes, void* stream);
 
+/* autograd backward of srg_ggnn_forward(..., save_for_backward = 1): `workspace`, `mask` and B must be that call's.
+ * dhidden_out: fp32 [rows, D] = dL/d(the updated states), only read.  dhidden_in (nullable): fp32 [rows, D], receives
+ * dL/d(the states passed in).  dmask (nullable, SRG_MODE_NOUN only): fp32 [B, R, R], receives dL/dmask (overwritten;
+ * deterministic).  The 14 GGSNN gradients accumulate into `g` (its classifier and embedding fields are ignored); the
+ * deferred chain rule (srg_set_deferred_chain) applies as in srg_*_backward.  bf16-packed weights only. */
+int srg_ggnn_backward(srg_handle* h, int mode, const float* dhidden_out, const float* mask, float* dmask,
+                      float* dhidden_in, int B, const srg_grads* g, void* workspace, size_t workspace_bytes,
+                      void* stream);
+
 /* FCGGNN.nouns_loss (model.py:189-201): sum over the 3 annotations of CrossEntropy(ignore_index = n_labels), each a
  * mean over its non-ignored targets.  counts: device fp32 [3] = number of non-ignored targets per annotation over the
  * GLOBAL batch (srg_count_targets, all-reduced by the caller when the batch is sharded).  loss: device fp32 scalar,

@@ -435,75 +435,40 @@ int chain_rule(srg_handle* h, const float* G_P, bf16* G_Pb, const float* s_all, 
 }
 
 // ------------------------------------------------------------------------------------------------ backward
-// dlogits (nullable) fp32 [Mfull, ldl]; dlb_ready: the bf16 gradient operand pb.dlb already holds a gradient written by
-// the loss kernels (srg_*_loss_backward with dlogits_bf16); both given: their sum.
-int path_backward(srg_handle* h, int mode, PathBufs& pb, const float* dlogits, int64_t ldl, int dlb_ready, int B,
-                  const DropSpec& ds, const srg_grads* g, cudaStream_t s) {
-  const int D = h->D, T = h->T, M = pb.M, Mf = pb.Mfull, R = h->R;
-  const int ncls = (mode == SRG_MODE_NOUN) ? h->L : h->V;
-  const int npad = (mode == SRG_MODE_NOUN) ? h->Lpad : h->Vpad;
-  const bf16* Wc = (mode == SRG_MODE_NOUN) ? h->Wcn : h->Wcv;
-  float* gWc = (mode == SRG_MODE_NOUN) ? g->Wc_noun : g->Wc_verb;
-  float* gbc = (mode == SRG_MODE_NOUN) ? g->bc_noun : g->bc_verb;
+// d/dP_x and the bias column sums of one backward call: per call (cleared here), or (deferred chain rule) shared by all
+// paths of the step
+int chain_acc(srg_handle* h, PathBufs& pb, float** G_P, float** s_all, cudaStream_t s) {
+  const int D = h->D;
+  *G_P = h->defer_chain ? h->acc_GP : pb.G_P;
+  *s_all = h->defer_chain ? h->acc_s : pb.s_all;
+  if (!h->defer_chain) {
+    SRG_CUDA(cudaMemsetAsync(*G_P, 0, sizeof(float) * 3 * D * D, s));
+    SRG_CUDA(cudaMemsetAsync(*s_all, 0, sizeof(float) * 3 * D, s));
+  }
+  return SRG_OK;
+}
+
+// The GGNN steps of a backward pass, on the stash of a save_for_backward forward: the gate derivatives of the last step
+// from dh_T = dL/dh_T fp32 [M, D] (read only; nullptr: the caller already wrote them), steps t = T-1..0, the weight
+// gradients, and the chain rule (or, deferred, only the accumulation into G_P / s_all).  mask: the [B,R,R] mask of
+// srg_ggnn_forward on dense rows, whose aggregation backward also yields dL/dmask when dmask is given (the caller clears
+// it); nullptr on a row-mapped role graph and on the verb node.  Leaves dL/d(initial states) in pb.dh.
+int ggnn_backward(srg_handle* h, int mode, PathBufs& pb, int B, const float* dh_T, const float* mask, float* dmask,
+                  float* G_P, float* s_all, const srg_grads* g, cudaStream_t s) {
+  const int D = h->D, T = h->T, M = pb.M, R = h->R;
   const int64_t ld3 = 3 * static_cast<int64_t>(D);
   const float cmul = (mode == SRG_MODE_NOUN) ? static_cast<float>(R) : 1.f;  // how often b_p enters a message
-  const bool use_drop = (ds.keep != nullptr || ds.seed != nullptr);
   const bool mapped = (pb.rm.meta != nullptr);            // role-graph path on the device-resident row layout
-  const bool gathered = use_drop || mapped;               // the classifier read pb.xd_hi (see classifier_forward)
-  const bf16* x = gathered ? pb.xd_hi : pb.hb_hi[T];
-  const int* rows_dev = mapped ? pb.rm.meta + 2 : nullptr;   // rows the tiles touch (multiple of 256)
   const int* m_dev = mapped ? pb.rm.meta : nullptr;          // rows incl. the shared pad row
 
-  // d/dP_x and the bias column sums: per call, or (deferred chain rule) shared by all paths of the step
-  const bool defer = h->defer_chain;
-  float* G_P = defer ? h->acc_GP : pb.G_P;
-  float* s_all = defer ? h->acc_s : pb.s_all;
-  if (!defer) {
-    SRG_CUDA(cudaMemsetAsync(G_P, 0, sizeof(float) * 3 * D * D, s));
-    SRG_CUDA(cudaMemsetAsync(s_all, 0, sizeof(float) * 3 * D, s));
-  }
-
-  // ---- classifier (model.py:105-111,152,168): one row per node slot
-  SRG_CHECK(dlogits != nullptr || dlb_ready, "backward: no gradient of the logits was given");
-  if (dlogits != nullptr) SRG_TRY(launch_cast_pad(dlogits, ldl, Mf, ncls, npad, pb.dlb, dlb_ready ? 1 : 0, s));
-  SRG_TRY(launch_colsum(pb.dlb, npad, Mf, ncls, gbc, 1.f, nullptr, 0.f, s));
-  SRG_TRY(wgrad(h, pb.dlb, npad, ncls, x, D, 1, Mf, Mf, nullptr, gWc, s));
-  {
-    GemmProblem p = base_problem(h, Mf, D);
-    add_seg(p, pb.dlb, Mf, npad, 0, npad);
-    p.b_mn = true;
-    p.b = mat(Wc, npad, D, D, DT_BF16);
-    p.epi = EPI_STORE_F32;
-    p.io[0] = mat(gathered ? pb.dx : pb.dh, Mf, D, D, DT_F32);
-    SRG_TRY(run_gemm(p, h->dev, s));
-  }
-
-  // dL/dh' of the last step comes from the classifier; from there on the GRU-gate derivatives of step t-1 are fused
-  // into the epilogue of the GEMM that completes dL/dh of step t (EPI_DH).
+  // dL/dh' of the last step comes from the caller; from there on the GRU-gate derivatives of step t-1 are fused into
+  // the epilogue of the GEMM that completes dL/dh of step t (EPI_DH).
   // dpre_of(t) = [dpre_h | dpre_z | dpre_r] of step t as column blocks of one [M, 3D] matrix.
   float* dh_acc = pb.dh_acc;
   auto dpre_of = [&](int t) { return pb.dpre_all + static_cast<size_t>(t) * M * ld3; };
-  if (gathered) {
-    // back through the dropout and the slot -> state-row gather, with the gate derivatives of the last step applied in
-    // the same pass for every row that has exactly one slot; the pad slots of all images add up in the shared pad row,
-    // whose derivatives (and the zero rows up to the tile boundary) follow in a launch over those few rows
-    GruPre gp;
-    gp.z = static_cast<const bf16*>(pb.st[T - 1].z);
-    gp.hc = pb.st[T - 1].hc;
-    gp.h = pb.hb_hi[T - 1];
-    gp.dpre_z = dpre_of(T - 1) + D;
-    gp.dpre_h = dpre_of(T - 1);
-    gp.ld_out = ld3;
-    gp.dh_acc = dh_acc;
-    SRG_TRY(launch_classifier_input_bwd(pb.dx, pb.rm, (mode == SRG_MODE_NOUN) ? B : Mf, (mode == SRG_MODE_NOUN) ? R : 1,
-                                        D, ds, pb.dh, gp, s));
-    if (mapped)
-      SRG_TRY(launch_gru_bwd_pre_ld(pb.dh, gp.z, gp.hc, gp.h, 256, rows_dev, pb.rm.meta + 1, D, gp.dpre_z, gp.dpre_h,
-                                    ld3, dh_acc, s));
-  } else {
-    SRG_TRY(launch_gru_bwd_pre_ld(pb.dh, static_cast<const bf16*>(pb.st[T - 1].z), pb.st[T - 1].hc, pb.hb_hi[T - 1], M,
+  if (dh_T != nullptr)
+    SRG_TRY(launch_gru_bwd_pre_ld(dh_T, static_cast<const bf16*>(pb.st[T - 1].z), pb.st[T - 1].hc, pb.hb_hi[T - 1], M,
                                   nullptr, nullptr, D, dpre_of(T - 1) + D, dpre_of(T - 1), ld3, dh_acc, s));
-  }
   for (int t = T - 1; t >= 0; --t) {
     StepBufs& st = pb.st[t];
     bf16* dp = dpre_of(t);
@@ -531,7 +496,8 @@ int path_backward(srg_handle* h, int mode, PathBufs& pb, const float* dlogits, i
     }
     // back through the aggregation, plus the r*h share:  ada[j] = e[j] + sum_i mask[i,j] da[i]
     // (verb node: the aggregation is the identity)
-    SRG_TRY(launch_aggregate_t_rows(pb.da, pb.e, pb.rm, mapped ? B : M, R, D, pb.ada, s));
+    if (mask != nullptr) SRG_TRY(launch_aggregate_t(pb.da, pb.e, mask, pb.hb_hi[t], B, R, D, pb.ada, dmask, s));
+    else SRG_TRY(launch_aggregate_t_rows(pb.da, pb.e, pb.rm, mapped ? B : M, R, D, pb.ada, s));
     const bf16* ada = pb.ada;
     {  // dL/dh_t = dh_acc + ada + [dpre_z | dpre_r] [U_z ; U_r], then the gate derivatives of step t-1
       GemmProblem p = path_problem(h, pb, D);
@@ -572,8 +538,64 @@ int path_backward(srg_handle* h, int mode, PathBufs& pb, const float* dlogits, i
   }
   pb.dh = dh_acc;  // gradient w.r.t. the initial node states
 
-  if (defer) return SRG_OK;   // srg_chain_finalize applies the chain rule once for all paths
+  if (h->defer_chain) return SRG_OK;   // srg_chain_finalize applies the chain rule once for all paths
   return chain_rule(h, G_P, pb.G_Pb, s_all, g, /*shared_dst=*/true, s);
+}
+
+// dlogits (nullable) fp32 [Mfull, ldl]; dlb_ready: the bf16 gradient operand pb.dlb already holds a gradient written by
+// the loss kernels (srg_*_loss_backward with dlogits_bf16); both given: their sum.
+int path_backward(srg_handle* h, int mode, PathBufs& pb, const float* dlogits, int64_t ldl, int dlb_ready, int B,
+                  const DropSpec& ds, const srg_grads* g, cudaStream_t s) {
+  const int D = h->D, T = h->T, Mf = pb.Mfull, R = h->R;
+  const int ncls = (mode == SRG_MODE_NOUN) ? h->L : h->V;
+  const int npad = (mode == SRG_MODE_NOUN) ? h->Lpad : h->Vpad;
+  const bf16* Wc = (mode == SRG_MODE_NOUN) ? h->Wcn : h->Wcv;
+  float* gWc = (mode == SRG_MODE_NOUN) ? g->Wc_noun : g->Wc_verb;
+  float* gbc = (mode == SRG_MODE_NOUN) ? g->bc_noun : g->bc_verb;
+  const int64_t ld3 = 3 * static_cast<int64_t>(D);
+  const bool use_drop = (ds.keep != nullptr || ds.seed != nullptr);
+  const bool mapped = (pb.rm.meta != nullptr);            // role-graph path on the device-resident row layout
+  const bool gathered = use_drop || mapped;               // the classifier read pb.xd_hi (see classifier_forward)
+  const bf16* x = gathered ? pb.xd_hi : pb.hb_hi[T];
+  const int* rows_dev = mapped ? pb.rm.meta + 2 : nullptr;   // rows the tiles touch (multiple of 256)
+
+  float *G_P = nullptr, *s_all = nullptr;
+  SRG_TRY(chain_acc(h, pb, &G_P, &s_all, s));
+
+  // ---- classifier (model.py:105-111,152,168): one row per node slot
+  SRG_CHECK(dlogits != nullptr || dlb_ready, "backward: no gradient of the logits was given");
+  if (dlogits != nullptr) SRG_TRY(launch_cast_pad(dlogits, ldl, Mf, ncls, npad, pb.dlb, dlb_ready ? 1 : 0, s));
+  SRG_TRY(launch_colsum(pb.dlb, npad, Mf, ncls, gbc, 1.f, nullptr, 0.f, s));
+  SRG_TRY(wgrad(h, pb.dlb, npad, ncls, x, D, 1, Mf, Mf, nullptr, gWc, s));
+  {
+    GemmProblem p = base_problem(h, Mf, D);
+    add_seg(p, pb.dlb, Mf, npad, 0, npad);
+    p.b_mn = true;
+    p.b = mat(Wc, npad, D, D, DT_BF16);
+    p.epi = EPI_STORE_F32;
+    p.io[0] = mat(gathered ? pb.dx : pb.dh, Mf, D, D, DT_F32);
+    SRG_TRY(run_gemm(p, h->dev, s));
+  }
+  if (gathered) {
+    // back through the dropout and the slot -> state-row gather, with the gate derivatives of the last step applied in
+    // the same pass for every row that has exactly one slot; the pad slots of all images add up in the shared pad row,
+    // whose derivatives (and the zero rows up to the tile boundary) follow in a launch over those few rows
+    bf16* dp = pb.dpre_all + static_cast<size_t>(T - 1) * pb.M * ld3;
+    GruPre gp;
+    gp.z = static_cast<const bf16*>(pb.st[T - 1].z);
+    gp.hc = pb.st[T - 1].hc;
+    gp.h = pb.hb_hi[T - 1];
+    gp.dpre_z = dp + D;
+    gp.dpre_h = dp;
+    gp.ld_out = ld3;
+    gp.dh_acc = pb.dh_acc;
+    SRG_TRY(launch_classifier_input_bwd(pb.dx, pb.rm, (mode == SRG_MODE_NOUN) ? B : Mf, (mode == SRG_MODE_NOUN) ? R : 1,
+                                        D, ds, pb.dh, gp, s));
+    if (mapped)
+      SRG_TRY(launch_gru_bwd_pre_ld(pb.dh, gp.z, gp.hc, gp.h, 256, rows_dev, pb.rm.meta + 1, D, gp.dpre_z, gp.dpre_h,
+                                    ld3, pb.dh_acc, s));
+  }
+  return ggnn_backward(h, mode, pb, B, gathered ? nullptr : pb.dh, nullptr, nullptr, G_P, s_all, g, s);
 }
 
 int ensure_pack_buffers(srg_handle* h, int split) {
@@ -1111,6 +1133,30 @@ int srg_verb_backward(srg_handle* h, const float* dlogits, int64_t ldl, int dlog
   SRG_TRY(make_drop(keep, drop_p, drop_seed, drop_stream, &ds));
   return path_backward(h, SRG_MODE_VERB, pb, dlogits, ldl, dlogits_in_workspace, B, ds, g,
                        static_cast<cudaStream_t>(stream));
+}
+
+int srg_ggnn_backward(srg_handle* h, int mode, const float* dhidden_out, const float* mask, float* dmask,
+                      float* dhidden_in, int B, const srg_grads* g, void* workspace, size_t workspace_bytes,
+                      void* stream) {
+  SRG_CHECK(h != nullptr, "srg_ggnn_backward: null handle");
+  DeviceGuard guard_(h->device);
+  SRG_CHECK(mode == SRG_MODE_NOUN || mode == SRG_MODE_VERB, "bad mode %d", mode);
+  PathBufs pb;
+  SRG_TRY(check_ws(h, mode, B, SRG_PREC_BF16, 1, workspace, workspace_bytes, &pb, false));
+  SRG_CHECK(h->packed_prec == SRG_PREC_BF16, "backward needs bf16-packed weights");
+  SRG_CHECK(dhidden_out != nullptr && g != nullptr, "srg_ggnn_backward: null argument");
+  SRG_CHECK(mode == SRG_MODE_VERB || mask != nullptr, "noun mode needs a mask");
+  SRG_CHECK(mode == SRG_MODE_NOUN || dmask == nullptr, "the verb node has no mask: dmask must be NULL");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  float *G_P = nullptr, *s_all = nullptr;
+  SRG_TRY(chain_acc(h, pb, &G_P, &s_all, s));
+  if (dmask != nullptr)
+    SRG_CUDA(cudaMemsetAsync(dmask, 0, sizeof(float) * static_cast<size_t>(B) * h->R * h->R, s));
+  SRG_TRY(ggnn_backward(h, mode, pb, B, dhidden_out, (mode == SRG_MODE_NOUN) ? mask : nullptr, dmask, G_P, s_all, g, s));
+  if (dhidden_in != nullptr)
+    SRG_CUDA(cudaMemcpyAsync(dhidden_in, pb.dh, sizeof(float) * static_cast<size_t>(pb.M) * h->D,
+                             cudaMemcpyDeviceToDevice, s));
+  return SRG_OK;
 }
 
 #ifdef SRG_EPI_TIMING

@@ -51,6 +51,11 @@ int launch_aggregate_rows(const float* h32, RowMap rm, int B, int R, int D, bf16
                           cudaStream_t s);
 // ada = e + aggregate^T(da) on the rows of `rm` (rm.cnt == nullptr: B dense rows, identity aggregation)
 int launch_aggregate_t_rows(const bf16* da, const bf16* e, RowMap rm, int B, int R, int D, bf16* ada, cudaStream_t s);
+// backward of launch_aggregate on B*R dense rows with the caller's fp32 mask [B,R,R] (any values):
+// ada[b,j] = e[b,j] + sum_i mask[b,i,j] da[b,i]; with dmask (nullable): dmask[b,i,j] += sum_d da[b,i,d] h[b,j,d], where
+// h is the state operand that entered the step.  dmask is deterministic (no atomics); without it h is not read.
+int launch_aggregate_t(const bf16* da, const bf16* e, const float* mask, const bf16* h, int B, int R, int D,
+                       bf16* ada, float* dmask, cudaStream_t s);
 // x[row] = dropout(h32[row of slot `row` under rm]) for all `rows` node slots -> bf16 hi (+ mid, lo)
 int launch_classifier_input(const float* h32, RowMap rm, int R, int64_t rows, int D, DropSpec ds, bf16* x_hi,
                             bf16* x_mid, bf16* x_lo, cudaStream_t s);

@@ -803,6 +803,111 @@ k_aggregate_t_rows(const bf16* __restrict__ da, const bf16* __restrict__ e, RowM
   }
 }
 
+// One 8-column chunk of the backward of k_aggregate for image rows [base, base + R*D) (see k_aggregate_t):
+// ada[j] = e[j] + sum_i mb[i,j] da[i]; kGrad: acc[i*kMaxR + j] += the chunk's share of da[i] . h[j].
+template <bool kGrad>
+__device__ __forceinline__ void aggregate_t_chunk(const bf16* __restrict__ da, const bf16* __restrict__ e,
+                                                  const float* __restrict__ mb, const bf16* __restrict__ h,
+                                                  int64_t base, int R, int D, bf16* __restrict__ ada, float* acc) {
+  uint4 g[kMaxR];
+#pragma unroll
+  for (int i = 0; i < kMaxR; ++i)
+    if (i < R) g[i] = *reinterpret_cast<const uint4*>(da + base + static_cast<int64_t>(i) * D);
+#pragma unroll
+  for (int j = 0; j < kMaxR; ++j) {
+    if (j < R) {
+      const uint4 ad = *reinterpret_cast<const uint4*>(e + base + static_cast<int64_t>(j) * D);
+      float a[8] = {bf16_lo_f(ad.x), bf16_hi_f(ad.x), bf16_lo_f(ad.y), bf16_hi_f(ad.y),
+                    bf16_lo_f(ad.z), bf16_hi_f(ad.z), bf16_lo_f(ad.w), bf16_hi_f(ad.w)};
+#pragma unroll
+      for (int i = 0; i < kMaxR; ++i) {
+        if (i < R) {
+          const float m = __ldg(mb + i * R + j);
+          a[0] = fmaf(m, bf16_lo_f(g[i].x), a[0]); a[1] = fmaf(m, bf16_hi_f(g[i].x), a[1]);
+          a[2] = fmaf(m, bf16_lo_f(g[i].y), a[2]); a[3] = fmaf(m, bf16_hi_f(g[i].y), a[3]);
+          a[4] = fmaf(m, bf16_lo_f(g[i].z), a[4]); a[5] = fmaf(m, bf16_hi_f(g[i].z), a[5]);
+          a[6] = fmaf(m, bf16_lo_f(g[i].w), a[6]); a[7] = fmaf(m, bf16_hi_f(g[i].w), a[7]);
+        }
+      }
+      uint4 o;
+      const uint2 lo = pack4_bf16(a[0], a[1], a[2], a[3]), hi = pack4_bf16(a[4], a[5], a[6], a[7]);
+      o.x = lo.x; o.y = lo.y; o.z = hi.x; o.w = hi.y;
+      *reinterpret_cast<uint4*>(ada + base + static_cast<int64_t>(j) * D) = o;
+      if constexpr (kGrad) {
+        const uint4 hv = *reinterpret_cast<const uint4*>(h + base + static_cast<int64_t>(j) * D);
+        const float hf[8] = {bf16_lo_f(hv.x), bf16_hi_f(hv.x), bf16_lo_f(hv.y), bf16_hi_f(hv.y),
+                             bf16_lo_f(hv.z), bf16_hi_f(hv.z), bf16_lo_f(hv.w), bf16_hi_f(hv.w)};
+#pragma unroll
+        for (int i = 0; i < kMaxR; ++i) {
+          if (i < R) {
+            float s = acc[i * kMaxR + j];
+            s = fmaf(bf16_lo_f(g[i].x), hf[0], s); s = fmaf(bf16_hi_f(g[i].x), hf[1], s);
+            s = fmaf(bf16_lo_f(g[i].y), hf[2], s); s = fmaf(bf16_hi_f(g[i].y), hf[3], s);
+            s = fmaf(bf16_lo_f(g[i].z), hf[4], s); s = fmaf(bf16_hi_f(g[i].z), hf[5], s);
+            s = fmaf(bf16_lo_f(g[i].w), hf[6], s); s = fmaf(bf16_hi_f(g[i].w), hf[7], s);
+            acc[i * kMaxR + j] = s;
+          }
+        }
+      }
+    }
+  }
+}
+
+// Backward of k_aggregate on dense rows (B images x R rows) with the caller's mask, which may be asymmetric, non-binary
+// and have self-loops:  ada[b,j] = e[b,j] + sum_i mask[b,i,j] da[b,i].  kGrad: also dmask[b,i,j] += sum_d da[b,i,d] h[b,j,d]
+// (h = the state operand that entered the step).  8 columns per thread per chunk.  Without kGrad the grid strides over
+// (image, chunk) pairs.  With kGrad one block owns an image (grid-stride over images): the R*R dot products are reduced
+// in a fixed order -- a warp butterfly, then the warps in index order -- and added by the owning block, so dmask is
+// deterministic without atomics.
+template <bool kGrad>
+__global__ void __launch_bounds__(kGrad ? 128 : 256, kGrad ? 1 : 4)
+k_aggregate_t(const bf16* __restrict__ da, const bf16* __restrict__ e, const float* __restrict__ mask,
+              const bf16* __restrict__ h, int B, int R, int D, bf16* __restrict__ ada, float* __restrict__ dmask) {
+  if constexpr (!kGrad) {
+    const int D8 = D / 8;
+    const int64_t total = static_cast<int64_t>(B) * D8;
+    for (int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; t < total;
+         t += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+      const int b = static_cast<int>(t / D8);
+      const int d = static_cast<int>(t % D8) * 8;
+      aggregate_t_chunk<false>(da, e, mask + static_cast<int64_t>(b) * R * R, nullptr,
+                               static_cast<int64_t>(b) * R * D + d, R, D, ada, nullptr);
+    }
+  } else {
+    constexpr int kAcc = kMaxR * kMaxR;
+    __shared__ float red[4][kAcc];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    for (int b = blockIdx.x; b < B; b += gridDim.x) {
+      const float* mb = mask + static_cast<int64_t>(b) * R * R;
+      float acc[kAcc];
+#pragma unroll
+      for (int k = 0; k < kAcc; ++k) acc[k] = 0.f;
+      for (int d = threadIdx.x * 8; d < D; d += blockDim.x * 8)
+        aggregate_t_chunk<true>(da, e, mb, h, static_cast<int64_t>(b) * R * D + d, R, D, ada, acc);
+#pragma unroll
+      for (int i = 0; i < kMaxR; ++i) {
+#pragma unroll
+        for (int j = 0; j < kMaxR; ++j) {
+          if (i < R && j < R) {
+            float v = acc[i * kMaxR + j];
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+            if (lane == 0) red[w][i * R + j] = v;
+          }
+        }
+      }
+      __syncthreads();
+      // R*R can exceed the block (32 threads at D = 256): each thread finishes every blockDim-th entry
+      for (int k = threadIdx.x; k < R * R; k += blockDim.x) {
+        float s = 0.f;
+        for (int q = 0; q < static_cast<int>(blockDim.x >> 5); ++q) s += red[q][k];
+        dmask[static_cast<int64_t>(b) * R * R + k] += s;
+      }
+      __syncthreads();   // red is reused by the block's next image
+    }
+  }
+}
+
 struct ColsumJobs {
   ColsumJob j[4];
 };
@@ -1348,6 +1453,23 @@ int launch_aggregate_t_rows(const bf16* da, const bf16* e, RowMap rm, int B, int
   if (R > kMaxR) return set_error(SRG_ERR_UNSUPPORTED, "max_role_count %d > %d", R, kMaxR);
   const int64_t units = (rm.cnt == nullptr) ? B : B + kSelfRows;
   k_aggregate_t_rows<<<grid_for(units * D / 8), kThreads, 0, s>>>(da, e, rm, B, R, D, ada);
+  SRG_LAUNCH_CHECK();
+  return SRG_OK;
+}
+
+int launch_aggregate_t(const bf16* da, const bf16* e, const float* mask, const bf16* h, int B, int R, int D,
+                       bf16* ada, float* dmask, cudaStream_t s) {
+  if (B <= 0) return SRG_OK;
+  if (R > kMaxR) return set_error(SRG_ERR_UNSUPPORTED, "max_role_count %d > %d", R, kMaxR);
+  if (D % 256 != 0) return set_error(SRG_ERR_ARG, "aggregate_t: D=%d must be a multiple of 256", D);
+  if (dmask != nullptr) {
+    if (h == nullptr) return set_error(SRG_ERR_ARG, "aggregate_t: dmask needs the step's state operand");
+    const int blocks = B < 148 * 16 ? B : 148 * 16;
+    k_aggregate_t<true><<<blocks, D / 8 < 128 ? D / 8 : 128, 0, s>>>(da, e, mask, h, B, R, D, ada, dmask);
+  } else {
+    k_aggregate_t<false><<<grid_for(static_cast<int64_t>(B) * D / 8), kThreads, 0, s>>>(da, e, mask, nullptr, B, R, D,
+                                                                                       ada, nullptr);
+  }
   SRG_LAUNCH_CHECK();
   return SRG_OK;
 }

@@ -2,8 +2,9 @@
 
 `FCGGNN(encoder, D_hidden_state)` keeps the reference's constructor, attribute / parameter names (= checkpoint
 keys), `forward(img, gt_verb)`, `predict_verb`, `predict_nouns`, `verb_loss`, `nouns_loss` (model.py:90-201) and
-`GGSNN(layersize).forward(hidden_state, mask, verb)` (model.py:38-86).  The arithmetic of the stage runs in
-libsrggnn.so (hand-written sm_100a kernels) through ctypes; PyTorch only owns memory, streams and autograd
+`GGSNN(layersize).forward(hidden_state, mask, verb)` (model.py:38-86), each differentiable on its own: in bf16 mode a
+caller can train through `model.ggsnn(node, mask)` with its own node init, adjacency or losses.  The arithmetic of the
+stage runs in libsrggnn.so (hand-written sm_100a kernels) through ctypes; PyTorch only owns memory, streams and autograd
 bookkeeping.  There is no CPU / eager fallback: non-CUDA inputs raise.
 
 Differences a caller can observe (all documented in DESIGN.md):
@@ -370,6 +371,70 @@ class _VerbStage(torch.autograd.Function):
         return (None, None, None, None, None, None, *[grads[n] for n in names])
 
 
+class _GGSNNStage(torch.autograd.Function):
+    """GGSNN.forward (model.py:59-86) on caller-supplied node states and mask, with its backward (bf16 only).
+    hidden: [B*R, D] (or [B, R, D]) with mask [B, R, R], or [B, D] with mask None (verb node)."""
+
+    @staticmethod
+    def forward(ctx, model, hidden, mask, *params):
+        eng = model._engine_for(hidden.device)
+        eng.ensure_packed(model, SRG_PREC_BF16)
+        h, mode, B, mk = _ggsnn_inputs(eng, hidden, mask, mask is None)
+        ws = eng.workspace(mode, B, SRG_PREC_BF16, True)
+        _lib.check(eng.lib.srg_ggnn_forward(eng.h, mode, _lib.ptr(h), _lib.ptr(mk), B, SRG_PREC_BF16, 1, _lib.ptr(ws),
+                                            ws.numel(), eng.stream()))
+        ctx.eng, ctx.ws, ctx.B, ctx.mode = eng, ws, B, mode
+        ctx.pack_gen = eng.pack_gen
+        ctx.direct = model._direct_grads()
+        ctx.live = tuple(params)          # the Parameter objects (for .grad in direct mode)
+        ctx.in_shape, ctx.in_dtype = hidden.shape, hidden.dtype
+        ctx.mask_meta = None if mask is None else (mask.device, mask.dtype)
+        ctx.save_for_backward(mk, *params)
+        return h
+
+    @staticmethod
+    def backward(ctx, dout):
+        eng = ctx.eng
+        eng.check_pack_gen(ctx.pack_gen)
+        mk, *params = ctx.saved_tensors
+        g = dout.detach().to(torch.float32).contiguous()
+        if ctx.direct:   # flat-buffer mode: the kernels accumulate straight into the (pre-zeroed) .grad views
+            grads = {n: p.grad for n, p in zip(_GGNN_FIELDS, ctx.live)}
+            eng.backward_begin(grads)
+        else:
+            grads = {n: torch.zeros_like(p) if ctx.needs_input_grad[3 + i] else None
+                     for i, (n, p) in enumerate(zip(_GGNN_FIELDS, params))}
+            eng.set_deferred(False)
+        dh = torch.empty_like(g) if ctx.needs_input_grad[1] else None
+        dm = torch.empty_like(mk) if ctx.needs_input_grad[2] else None     # no dL/dmask pass unless it is wanted
+        sg = _grad_struct(grads, eng)
+        _lib.check(eng.lib.srg_ggnn_backward(eng.h, ctx.mode, _lib.ptr(g), _lib.ptr(mk), _lib.ptr(dm), _lib.ptr(dh),
+                                             ctx.B, ctypes.byref(sg), _lib.ptr(ctx.ws), ctx.ws.numel(), eng.stream()))
+        ctx.ws = None
+        if ctx.direct:
+            eng.backward_mark()
+        dh = None if dh is None else dh.view(ctx.in_shape).to(ctx.in_dtype)
+        dm = None if dm is None else dm.to(*ctx.mask_meta)
+        return (None, dh, dm, *[None if ctx.direct else grads[n] for n in _GGNN_FIELDS])
+
+
+def _ggsnn_inputs(eng, hidden, mask, verb):
+    """(fp32 [rows, D] copy of the states, mode, B, fp32 [B, R, R] mask or None) for srg_ggnn_forward."""
+    h = hidden.detach().float().contiguous().clone()
+    if verb:
+        B, mode, mk = h.shape[0], SRG_MODE_VERB, None
+        rows = B
+    else:
+        B, mode = mask.shape[0], SRG_MODE_NOUN
+        mk = mask.detach().to(device=h.device, dtype=torch.float32).contiguous()
+        rows = B * eng.R
+        if tuple(mk.shape) != (B, eng.R, eng.R):
+            raise _lib.SrgError("mask must be [B, %d, %d], got %s" % (eng.R, eng.R, tuple(mask.shape)))
+    if h.numel() != rows * eng.D:
+        raise _lib.SrgError("hidden_state has %d elements, expected %d rows of %d" % (h.numel(), rows, eng.D))
+    return h, mode, B, mk
+
+
 def _padded_grad(g, npad):
     """fp32 [rows, n] gradient with unit column stride and a 16-byte aligned row pitch (no copy when the autograd
     engine hands back the padded view produced by the loss kernels)."""
@@ -526,7 +591,10 @@ class GGSNN(nn.Module):
         self._owner = None
 
     def forward(self, hidden_state, mask=None, verb=False):
-        """Forward-only (inference) entry with the reference signature; training goes through FCGGNN."""
+        """model.py:59-86 with the reference signature: hidden_state [B*R, D] with mask [B, R, R] (role graph), or
+        [B, D] with verb=True (verb node).  Differentiable in bf16 precision: when grad is enabled and hidden_state, mask
+        or a GGSNN parameter requires grad, the CUDA backward returns the gradients of all three (dL/dmask only when
+        mask.requires_grad).  precision='fp32' is forward-only and raises when a gradient is needed."""
         owner = self._owner() if self._owner is not None else None
         if owner is None:
             raise _lib.SrgError("GGSNN.forward needs the owning FCGGNN (it holds the CUDA engine)")
@@ -811,19 +879,25 @@ class FCGGNN(nn.Module):
         fv, fn = self.extract_features(img, img_nouns)
         return self.situations_from_features(fv, fn, k=k)
 
-    # ---- GGSNN.forward drop-in (inference) ------------------------------------------------------
+    # ---- GGSNN.forward drop-in ------------------------------------------------------------------
     def _ggsnn_forward(self, hidden_state, mask=None, verb=False):
         if not hidden_state.is_cuda:
             raise _lib.SrgError("the GGNN stage has no CPU path: hidden_state must be a CUDA tensor")
         eng = self._engine_for(hidden_state.device)
         prec = _prec_code(self.precision)
+        mask = None if verb else mask
+        params = self._ggnn_params()
+        need_grad = torch.is_grad_enabled() and any(
+            t is not None and t.requires_grad for t in [hidden_state, mask] + params)
+        if not verb and mask is None:
+            raise _lib.SrgError("GGSNN.forward on the role graph (verb=False) needs a mask")
+        if need_grad:
+            if prec != SRG_PREC_BF16:
+                raise _lib.SrgError("precision='fp32' is a forward-only parity mode; use torch.no_grad() or "
+                                    "precision='bf16'")
+            return _GGSNNStage.apply(self, hidden_state, mask, *params)
         eng.ensure_packed(self, prec)
-        h = hidden_state.detach().float().contiguous().clone()
-        if verb:
-            B, mode, mk = h.shape[0], SRG_MODE_VERB, None
-        else:
-            B, mode = mask.shape[0], SRG_MODE_NOUN
-            mk = mask.detach().to(device=h.device, dtype=torch.float32).contiguous()
+        h, mode, B, mk = _ggsnn_inputs(eng, hidden_state, mask, verb)
         ws = eng.workspace(mode, B, prec, False)
         _lib.check(eng.lib.srg_ggnn_forward(eng.h, mode, _lib.ptr(h), _lib.ptr(mk), B, prec, 0, _lib.ptr(ws),
                                             ws.numel(), eng.stream()))
