@@ -220,6 +220,23 @@ int srg_verb_backward(srg_handle* h, const float* dlogits, int64_t ldl, int dlog
                       const uint8_t* keep, float drop_p, const int64_t* drop_seed, int64_t drop_stream,
                       const srg_grads* g, void* workspace, size_t workspace_bytes, void* stream);
 
+/* srg_nouns_backward / srg_verb_backward plus the gradient w.r.t. the backbone features `feat` of the forward call:
+ * dfeat (nullable) fp32 [B, D] is OVERWRITTEN (not accumulated), like dhidden_in of srg_ggnn_backward.
+ *   nouns (model.py:124-144): node[b,r] = relu(feat[b] * role_emb[role(b,r)] * verb_emb[verb[b]]), so
+ *          dfeat[b] = sum over the real roles r of [node[b,r] > 0] * dL/dnode[b,r] * role_emb[role(b,r)] * verb_emb[verb[b]]
+ *          (pad slots contribute nothing); the embedding gradients in `g` are computed in the same pass when both
+ *          g->role_emb and g->verb_emb are set, and the pass is skipped when neither they nor dfeat are;
+ *   verb  (model.py:160): node = relu(feat), so dfeat = [node > 0] * dL/dnode.
+ * The mask [node > 0] is taken from the bf16 copy of the initial state (relu'(0) = 0, as torch).  No atomics: dfeat is
+ * deterministic.  With dfeat = NULL these are srg_nouns_backward / srg_verb_backward, launch for launch. */
+int srg_nouns_backward_feat(srg_handle* h, const float* dlogits, int64_t ldl, int dlogits_in_workspace,
+                            const float* feat, const int64_t* verb, int B, const float* role_emb, const float* verb_emb,
+                            const uint8_t* keep, float drop_p, const int64_t* drop_seed, int64_t drop_stream,
+                            const srg_grads* g, float* dfeat, void* workspace, size_t workspace_bytes, void* stream);
+int srg_verb_backward_feat(srg_handle* h, const float* dlogits, int64_t ldl, int dlogits_in_workspace, int B,
+                           const uint8_t* keep, float drop_p, const int64_t* drop_seed, int64_t drop_stream,
+                           const srg_grads* g, float* dfeat, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Deferred chain rule.  The verb node and the role graph share one GGNN (model.py:28-35, 226), so one training step
  * (sr.py:63-79) calls both backward functions with the same weights.  Their gradients w.r.t. the message-side weights
  * W_p, b_p, W_z, W_r, W_h go through the same chain rule (d/dP_x -> dW_x, dW_p, db_p; P_x = W_x W_p), which is linear

@@ -56,6 +56,10 @@ SIGNATURES = {
     "srg_nouns_backward": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _i, _vp, _vp, _vp, _f, _vp, _i64, _c.POINTER(SrgGrads),
                                 _vp, _sz, _vp]),
     "srg_verb_backward": (_i, [_vp, _vp, _i64, _i, _i, _vp, _f, _vp, _i64, _c.POINTER(SrgGrads), _vp, _sz, _vp]),
+    "srg_nouns_backward_feat": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _i, _vp, _vp, _vp, _f, _vp, _i64,
+                                     _c.POINTER(SrgGrads), _vp, _vp, _sz, _vp]),
+    "srg_verb_backward_feat": (_i, [_vp, _vp, _i64, _i, _i, _vp, _f, _vp, _i64, _c.POINTER(SrgGrads), _vp, _vp, _sz,
+                                    _vp]),
     "srg_ggnn_backward": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _c.POINTER(SrgGrads), _vp, _sz, _vp]),
     "srg_set_deferred_chain": (_i, [_vp, _i, _vp]),
     "srg_chain_finalize": (_i, [_vp, _c.POINTER(SrgGrads), _vp]),

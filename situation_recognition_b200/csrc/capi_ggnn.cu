@@ -1097,10 +1097,10 @@ int srg_chain_finalize(srg_handle* h, const srg_grads* g, void* stream) {
   return SRG_OK;
 }
 
-int srg_nouns_backward(srg_handle* h, const float* dlogits, int64_t ldl, int dlogits_in_workspace, const float* feat,
-                       const int64_t* verb, int B, const float* role_emb, const float* verb_emb, const uint8_t* keep,
-                       float drop_p, const int64_t* drop_seed, int64_t drop_stream, const srg_grads* g, void* workspace,
-                       size_t workspace_bytes, void* stream) {
+int srg_nouns_backward_feat(srg_handle* h, const float* dlogits, int64_t ldl, int dlogits_in_workspace,
+                            const float* feat, const int64_t* verb, int B, const float* role_emb, const float* verb_emb,
+                            const uint8_t* keep, float drop_p, const int64_t* drop_seed, int64_t drop_stream,
+                            const srg_grads* g, float* dfeat, void* workspace, size_t workspace_bytes, void* stream) {
   SRG_CHECK(h != nullptr, "srg_nouns_backward: null handle");
   DeviceGuard guard_(h->device);
   PathBufs pb;
@@ -1113,15 +1113,22 @@ int srg_nouns_backward(srg_handle* h, const float* dlogits, int64_t ldl, int dlo
   SRG_TRY(make_drop(keep, drop_p, drop_seed, drop_stream, &ds));
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   SRG_TRY(path_backward(h, SRG_MODE_NOUN, pb, dlogits, ldl, dlogits_in_workspace, B, ds, g, s));
-  if (g->role_emb != nullptr && g->verb_emb != nullptr)
-    SRG_TRY(launch_node_init_bwd(pb.dh, pb.hb_hi[0], feat, role_emb, verb_emb, verb, h->d_verb2roles, h->V, h->n_roles, B,
-                                 h->R, h->D, pb.rm, g->role_emb, g->verb_emb, s));
-  return SRG_OK;
+  const bool emb = (g->role_emb != nullptr && g->verb_emb != nullptr);
+  return launch_node_init_bwd(pb.dh, pb.hb_hi[0], feat, role_emb, verb_emb, verb, h->d_verb2roles, h->V, h->n_roles, B,
+                              h->R, h->D, pb.rm, emb ? g->role_emb : nullptr, emb ? g->verb_emb : nullptr, dfeat, s);
 }
 
-int srg_verb_backward(srg_handle* h, const float* dlogits, int64_t ldl, int dlogits_in_workspace, int B,
-                      const uint8_t* keep, float drop_p, const int64_t* drop_seed, int64_t drop_stream,
-                      const srg_grads* g, void* workspace, size_t workspace_bytes, void* stream) {
+int srg_nouns_backward(srg_handle* h, const float* dlogits, int64_t ldl, int dlogits_in_workspace, const float* feat,
+                       const int64_t* verb, int B, const float* role_emb, const float* verb_emb, const uint8_t* keep,
+                       float drop_p, const int64_t* drop_seed, int64_t drop_stream, const srg_grads* g, void* workspace,
+                       size_t workspace_bytes, void* stream) {
+  return srg_nouns_backward_feat(h, dlogits, ldl, dlogits_in_workspace, feat, verb, B, role_emb, verb_emb, keep, drop_p,
+                                 drop_seed, drop_stream, g, nullptr, workspace, workspace_bytes, stream);
+}
+
+int srg_verb_backward_feat(srg_handle* h, const float* dlogits, int64_t ldl, int dlogits_in_workspace, int B,
+                           const uint8_t* keep, float drop_p, const int64_t* drop_seed, int64_t drop_stream,
+                           const srg_grads* g, float* dfeat, void* workspace, size_t workspace_bytes, void* stream) {
   SRG_CHECK(h != nullptr, "srg_verb_backward: null handle");
   DeviceGuard guard_(h->device);
   PathBufs pb;
@@ -1131,8 +1138,17 @@ int srg_verb_backward(srg_handle* h, const float* dlogits, int64_t ldl, int dlog
   SRG_CHECK(dlogits == nullptr || ldl >= h->V, "srg_verb_backward: ldl %lld < n_verbs %d", (long long)ldl, h->V);
   DropSpec ds;
   SRG_TRY(make_drop(keep, drop_p, drop_seed, drop_stream, &ds));
-  return path_backward(h, SRG_MODE_VERB, pb, dlogits, ldl, dlogits_in_workspace, B, ds, g,
-                       static_cast<cudaStream_t>(stream));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  SRG_TRY(path_backward(h, SRG_MODE_VERB, pb, dlogits, ldl, dlogits_in_workspace, B, ds, g, s));
+  if (dfeat != nullptr) SRG_TRY(launch_node_init_verb_bwd(pb.dh, pb.hb_hi[0], B, h->D, dfeat, s));
+  return SRG_OK;
+}
+
+int srg_verb_backward(srg_handle* h, const float* dlogits, int64_t ldl, int dlogits_in_workspace, int B,
+                      const uint8_t* keep, float drop_p, const int64_t* drop_seed, int64_t drop_stream,
+                      const srg_grads* g, void* workspace, size_t workspace_bytes, void* stream) {
+  return srg_verb_backward_feat(h, dlogits, ldl, dlogits_in_workspace, B, keep, drop_p, drop_seed, drop_stream, g,
+                                nullptr, workspace, workspace_bytes, stream);
 }
 
 int srg_ggnn_backward(srg_handle* h, int mode, const float* dhidden_out, const float* mask, float* dmask,

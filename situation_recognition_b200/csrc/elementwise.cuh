@@ -128,11 +128,15 @@ int launch_cast_pad(const float* src, int64_t ld, int rows, int n_valid, int n_p
 // out1[c] (+= scale1 * colsum) , out2[c] (+= scale2 * colsum); X bf16 [rows, ld], first n_cols columns
 int launch_colsum(const bf16* X, int64_t ld, int rows, int n_cols, float* out1, float scale1, float* out2,
                   float scale2, cudaStream_t s);
-// node-init backward (embedding gradients), model.py:132-144
+// node-init backward of the role graph, model.py:124-144, from dh0 = dL/dnode and the bf16 copy h0b of the node's
+// initial state (relu'(0) = 0): the embedding gradients (accumulated; both pointers null: skipped) and / or
+// dfeat fp32 [B, D] = sum over the image's rows of [node > 0] dh0 * role_emb * verb_emb (overwritten; nullable)
 int launch_node_init_bwd(const float* dh0, const bf16* h0b, const float* feat, const float* role_emb,
                          const float* verb_emb, const int64_t* verb, const int32_t* verb2roles, int n_verbs,
                          int n_roles, int B, int R, int D, RowMap rm, float* d_role_emb, float* d_verb_emb,
-                         cudaStream_t s);
+                         float* dfeat, cudaStream_t s);
+// node-init backward of the verb node, model.py:160: dfeat [B, D] = h0b > 0 ? dh0 : 0 (overwritten)
+int launch_node_init_verb_bwd(const float* dh0, const bf16* h0b, int B, int D, float* dfeat, cudaStream_t s);
 
 // up to 4 column sums in one launch: out1/out2 += scale * colsum, out3 += scale3 * colsum
 struct ColsumJob {

@@ -706,11 +706,16 @@ __global__ void k_colsum(const bf16* __restrict__ X, int64_t ld, int rows, int n
   }
 }
 
+// One thread per (image, 4 columns) walks the image's real role rows.  kEmb: the embedding gradients (atomics: ~190
+// role rows receive the gradients of all node rows); kFeat: dfeat[b] = sum_r [node > 0] dh0 * role_emb * verb_emb, one
+// register accumulator and a plain store (this thread owns the output element: deterministic, no atomics).
+template <bool kEmb, bool kFeat>
 __global__ void k_node_init_bwd(const float* __restrict__ dh0, const bf16* __restrict__ h0b,
                                 const float* __restrict__ feat, const float* __restrict__ role_emb,
                                 const float* __restrict__ verb_emb, const int64_t* __restrict__ verb,
                                 const int32_t* __restrict__ verb2roles, int n_verbs, int n_roles, int B, int R,
-                                int D, RowMap rm, float* __restrict__ d_role_emb, float* __restrict__ d_verb_emb) {
+                                int D, RowMap rm, float* __restrict__ d_role_emb, float* __restrict__ d_verb_emb,
+                                float* __restrict__ dfeat) {
   const int D4 = D / 4;
   const int64_t total = static_cast<int64_t>(B) * D4;
   for (int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; t < total;
@@ -719,9 +724,11 @@ __global__ void k_node_init_bwd(const float* __restrict__ dh0, const bf16* __res
     const int d = static_cast<int>(t % D4) * 4;
     int64_t v = verb[b];
     if (v < 0 || v >= n_verbs) v = 0;   // same clamp as the forward kernels (which also raise the bad-verb flag)
-    const float4 f = *reinterpret_cast<const float4*>(feat + static_cast<int64_t>(b) * D + d);
+    float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (kEmb) f = *reinterpret_cast<const float4*>(feat + static_cast<int64_t>(b) * D + d);
     const float4 ve = *reinterpret_cast<const float4*>(verb_emb + v * D + d);
     float4 accv = make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 accf = make_float4(0.f, 0.f, 0.f, 0.f);
     const int n = rm.cnt[b];
     const int64_t base = rm.off[b];
     for (int r = 0; r < n; ++r) {
@@ -735,15 +742,39 @@ __global__ void k_node_init_bwd(const float* __restrict__ dh0, const bf16* __res
       g.z = (bf16_lo_f(hb.y) > 0.f) ? g.z : 0.f;
       g.w = (bf16_hi_f(hb.y) > 0.f) ? g.w : 0.f;
       const float4 re = *reinterpret_cast<const float4*>(role_emb + static_cast<int64_t>(idx) * D + d);
-      // ~190 embedding rows receive the gradients of all node rows: one 16-byte reduction per thread instead of four
-      atomicAdd(reinterpret_cast<float4*>(d_role_emb + static_cast<int64_t>(idx) * D + d),
-                make_float4(g.x * f.x * ve.x, g.y * f.y * ve.y, g.z * f.z * ve.z, g.w * f.w * ve.w));
-      accv.x = fmaf(g.x * f.x, re.x, accv.x);
-      accv.y = fmaf(g.y * f.y, re.y, accv.y);
-      accv.z = fmaf(g.z * f.z, re.z, accv.z);
-      accv.w = fmaf(g.w * f.w, re.w, accv.w);
+      if (kEmb) {
+        // one 16-byte reduction per thread instead of four
+        atomicAdd(reinterpret_cast<float4*>(d_role_emb + static_cast<int64_t>(idx) * D + d),
+                  make_float4(g.x * f.x * ve.x, g.y * f.y * ve.y, g.z * f.z * ve.z, g.w * f.w * ve.w));
+        accv.x = fmaf(g.x * f.x, re.x, accv.x);
+        accv.y = fmaf(g.y * f.y, re.y, accv.y);
+        accv.z = fmaf(g.z * f.z, re.z, accv.z);
+        accv.w = fmaf(g.w * f.w, re.w, accv.w);
+      }
+      if (kFeat) {
+        accf.x = fmaf(g.x * re.x, ve.x, accf.x);
+        accf.y = fmaf(g.y * re.y, ve.y, accf.y);
+        accf.z = fmaf(g.z * re.z, ve.z, accf.z);
+        accf.w = fmaf(g.w * re.w, ve.w, accf.w);
+      }
     }
-    atomicAdd(reinterpret_cast<float4*>(d_verb_emb + v * D + d), accv);
+    if (kEmb) atomicAdd(reinterpret_cast<float4*>(d_verb_emb + v * D + d), accv);
+    if (kFeat) *reinterpret_cast<float4*>(dfeat + static_cast<int64_t>(b) * D + d) = accf;
+  }
+}
+
+// verb node: node = relu(feat), so dfeat = dh0 where the initial state (its bf16 copy) is > 0, else 0
+__global__ void k_node_init_verb_bwd(const float* __restrict__ dh0, const bf16* __restrict__ h0b, int64_t n4,
+                                     float* __restrict__ dfeat) {
+  for (int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; t < n4;
+       t += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    float4 g = *reinterpret_cast<const float4*>(dh0 + t * 4);
+    const uint2 hb = *reinterpret_cast<const uint2*>(h0b + t * 4);
+    g.x = (bf16_lo_f(hb.x) > 0.f) ? g.x : 0.f;
+    g.y = (bf16_hi_f(hb.x) > 0.f) ? g.y : 0.f;
+    g.z = (bf16_lo_f(hb.y) > 0.f) ? g.z : 0.f;
+    g.w = (bf16_hi_f(hb.y) > 0.f) ? g.w : 0.f;
+    *reinterpret_cast<float4*>(dfeat + t * 4) = g;
   }
 }
 
@@ -1514,10 +1545,21 @@ int launch_dropout_mask(DropSpec ds, int64_t rows, int D, uint8_t* out, cudaStre
 int launch_node_init_bwd(const float* dh0, const bf16* h0b, const float* feat, const float* role_emb,
                          const float* verb_emb, const int64_t* verb, const int32_t* verb2roles, int n_verbs,
                          int n_roles, int B, int R, int D, RowMap rm, float* d_role_emb, float* d_verb_emb,
-                         cudaStream_t s) {
+                         float* dfeat, cudaStream_t s) {
+  const bool emb = (d_role_emb != nullptr && d_verb_emb != nullptr);
+  if (B <= 0 || (!emb && dfeat == nullptr)) return SRG_OK;
+  auto kern = emb ? (dfeat ? k_node_init_bwd<true, true> : k_node_init_bwd<true, false>) : k_node_init_bwd<false, true>;
+  kern<<<grid_for(static_cast<int64_t>(B) * D / 4), kThreads, 0, s>>>(
+      dh0, h0b, feat, role_emb, verb_emb, verb, verb2roles, n_verbs, n_roles, B, R, D, rm, d_role_emb, d_verb_emb,
+      dfeat);
+  SRG_LAUNCH_CHECK();
+  return SRG_OK;
+}
+
+int launch_node_init_verb_bwd(const float* dh0, const bf16* h0b, int B, int D, float* dfeat, cudaStream_t s) {
   if (B <= 0) return SRG_OK;
-  k_node_init_bwd<<<grid_for(static_cast<int64_t>(B) * D / 4), kThreads, 0, s>>>(
-      dh0, h0b, feat, role_emb, verb_emb, verb, verb2roles, n_verbs, n_roles, B, R, D, rm, d_role_emb, d_verb_emb);
+  const int64_t n4 = static_cast<int64_t>(B) * D / 4;
+  k_node_init_verb_bwd<<<grid_for(n4), kThreads, 0, s>>>(dh0, h0b, n4, dfeat);
   SRG_LAUNCH_CHECK();
   return SRG_OK;
 }

@@ -7,6 +7,9 @@ therefore the same in every epoch, while the reference recomputes three ResNet-1
 (model.py:116,159,175-178) -- 92 % of an end-to-end eval step on a B200.  The cache stores them once, on the GPU
 (25 200 dev images x 2 x 2048 fp32 = 413 MB), and later epochs feed `FCGGNN.forward_features` directly.
 
+The cache is only valid for frozen backbones: `sr.py --finetune_backbone` (or any caller that trains a backbone) must
+not use it, since the features then change at every optimizer step.
+
 Training features are NOT cached by the launcher: the reference trains with random crops / flips and with the backbones'
 BatchNorm layers in training mode (model.train(), sr.py:24), so those features legitimately change every epoch.
 """

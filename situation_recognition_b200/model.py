@@ -3,7 +3,9 @@
 `FCGGNN(encoder, D_hidden_state)` keeps the reference's constructor, attribute / parameter names (= checkpoint
 keys), `forward(img, gt_verb)`, `predict_verb`, `predict_nouns`, `verb_loss`, `nouns_loss` (model.py:90-201) and
 `GGSNN(layersize).forward(hidden_state, mask, verb)` (model.py:38-86), each differentiable on its own: in bf16 mode a
-caller can train through `model.ggsnn(node, mask)` with its own node init, adjacency or losses.  The arithmetic of the
+caller can train through `model.ggsnn(node, mask)` with its own node init, adjacency or losses, and the fused paths
+return dL/dfeatures, so an unfrozen backbone (`model.convnet_nouns.requires_grad_(True)`), a trainable adapter in front
+of `forward_features` or a saliency map dL/dimage get their gradients.  The arithmetic of the
 stage runs in libsrggnn.so (hand-written sm_100a kernels) through ctypes; PyTorch only owns memory, streams and autograd
 bookkeeping.  There is no CPU / eager fallback: non-CUDA inputs raise.
 
@@ -46,8 +48,9 @@ def _pad256(n):
 
 
 class resnet(nn.Module):
-    """Frozen torchvision ResNet-152 returning the 2048-d pooled features (model.py:8-35).  Stock library module,
-    not part of the CUDA path; timed separately.  Offline, the pretrained weights cannot be downloaded, so
+    """torchvision ResNet-152 returning the 2048-d pooled features (model.py:8-35), frozen as in the reference;
+    `requires_grad_(True)` fine-tunes it (the stages return dL/dfeatures).  Stock library module, not part of the CUDA
+    path; timed separately.  Offline, the pretrained weights cannot be downloaded, so
     `pretrained=None` tries and falls back to random init with a warning."""
 
     def __init__(self, out_layers, pretrained=None):
@@ -224,7 +227,7 @@ def _as_feat(x, D):
     x = x.reshape(x.shape[0], -1)
     if x.shape[1] != D:
         raise _lib.SrgError("backbone features have %d channels, expected %d" % (x.shape[1], D))
-    return x.detach().float().contiguous()
+    return x.float().contiguous()     # keeps the autograd graph: the stages return dL/dfeat when it is needed
 
 
 def _grad_struct(named, engine):
@@ -251,7 +254,8 @@ class _GradTap:
 
 
 class _NounsStage(torch.autograd.Function):
-    """predict_nouns minus the backbone (model.py:117-155)."""
+    """predict_nouns minus the backbone (model.py:117-155).  Input 2 is the fp32 [B, D] feature tensor; its gradient is
+    returned when it requires grad (and only then: otherwise the backward passes dfeat = NULL)."""
 
     @staticmethod
     def forward(ctx, model, grad_on, feat, verb, keep, seed, slot, role_emb, verb_emb, *params):
@@ -301,20 +305,21 @@ class _NounsStage(torch.autograd.Function):
             grads = {n: torch.zeros_like(p) for n, p in zip(names, (role_emb, verb_emb) + tuple(params))}
             eng.set_deferred(False)
         sg = _grad_struct(grads, eng)
-        _lib.check(eng.lib.srg_nouns_backward(eng.h, _lib.ptr(dl), ldl, int(in_ws), _lib.ptr(feat), _lib.ptr(verb), B,
-                                              _lib.ptr(role_emb), _lib.ptr(verb_emb), _lib.ptr(keep), ctx.drop_p,
-                                              _lib.ptr(seed), ctx.slot, ctypes.byref(sg), _lib.ptr(ctx.ws),
-                                              ctx.ws.numel(), eng.stream()))
+        dfeat = torch.empty_like(feat) if ctx.needs_input_grad[2] else None
+        _lib.check(eng.lib.srg_nouns_backward_feat(eng.h, _lib.ptr(dl), ldl, int(in_ws), _lib.ptr(feat), _lib.ptr(verb),
+                                                   B, _lib.ptr(role_emb), _lib.ptr(verb_emb), _lib.ptr(keep),
+                                                   ctx.drop_p, _lib.ptr(seed), ctx.slot, ctypes.byref(sg),
+                                                   _lib.ptr(dfeat), _lib.ptr(ctx.ws), ctx.ws.numel(), eng.stream()))
         ctx.ws = None
         if ctx.direct:
             eng.backward_mark()
-            return (None,) * (7 + len(names))
+            return (None, None, dfeat) + (None,) * (4 + len(names))
         out = [grads[n] for n in _GGNN_FIELDS + ["Wc_noun", "bc_noun"]]
-        return (None, None, None, None, None, None, None, grads["role_emb"], grads["verb_emb"], *out)
+        return (None, None, dfeat, None, None, None, None, grads["role_emb"], grads["verb_emb"], *out)
 
 
 class _VerbStage(torch.autograd.Function):
-    """predict_verb minus the backbone (model.py:160-168)."""
+    """predict_verb minus the backbone (model.py:160-168); dL/dfeat for input 2 as in _NounsStage."""
 
     @staticmethod
     def forward(ctx, model, grad_on, feat, keep, seed, slot, *params):
@@ -362,13 +367,15 @@ class _VerbStage(torch.autograd.Function):
             grads = {n: torch.zeros_like(p) for n, p in zip(names, params)}
             eng.set_deferred(False)
         sg = _grad_struct(grads, eng)
-        _lib.check(eng.lib.srg_verb_backward(eng.h, _lib.ptr(dl), ldl, int(in_ws), B, _lib.ptr(keep), ctx.drop_p, _lib.ptr(seed),
-                                             ctx.slot, ctypes.byref(sg), _lib.ptr(ctx.ws), ctx.ws.numel(), eng.stream()))
+        dfeat = torch.empty(B, eng.D, dtype=torch.float32, device=eng.device) if ctx.needs_input_grad[2] else None
+        _lib.check(eng.lib.srg_verb_backward_feat(eng.h, _lib.ptr(dl), ldl, int(in_ws), B, _lib.ptr(keep), ctx.drop_p,
+                                                  _lib.ptr(seed), ctx.slot, ctypes.byref(sg), _lib.ptr(dfeat),
+                                                  _lib.ptr(ctx.ws), ctx.ws.numel(), eng.stream()))
         ctx.ws = None
         if ctx.direct:
             eng.backward_mark()
-            return (None,) * (6 + len(names))
-        return (None, None, None, None, None, None, *[grads[n] for n in names])
+            return (None, None, dfeat) + (None,) * (3 + len(names))
+        return (None, None, dfeat, None, None, None, *[grads[n] for n in names])
 
 
 class _GGSNNStage(torch.autograd.Function):
@@ -696,7 +703,7 @@ class FCGGNN(nn.Module):
 
     # ---- reference API -------------------------------------------------------------------------
     def predict_nouns(self, img, gt_verb, batch_size, _mask_slot=1, _feat=None):
-        # `_feat`: backbone features computed once by forward() for both noun passes (the reference runs the frozen
+        # `_feat`: backbone features computed once by forward() for both noun passes (the reference runs the
         # convnet_nouns twice on the same images, model.py:116,176-178)
         feat = _feat if _feat is not None else _as_feat(self.convnet_nouns(img), self.D)
         if feat.shape[0] != batch_size:
@@ -739,14 +746,17 @@ class FCGGNN(nn.Module):
             self._step_seed = None
 
     def extract_features(self, img, img_nouns=None):
-        """The two frozen backbones (model.py:116,159): (feat_verbs, feat_nouns), fp32 [B, D].  Both are frozen
-        (model.py:17-18), so for a fixed image under a deterministic transform in eval mode these features never
-        change: `features.FeatureCache` keeps them across epochs (SURVEY section 8f, N3)."""
+        """The two backbones (model.py:116,159): (feat_verbs, feat_nouns), fp32 [B, D], differentiable when a backbone
+        (or the image) requires grad.  With frozen backbones (model.py:17-18, the default) the features of a fixed image
+        under a deterministic transform in eval mode never change: `features.FeatureCache` keeps them across epochs
+        (SURVEY section 8f, N3).  That cache is wrong for backbones being fine-tuned."""
         img_n = img if img_nouns is None else img_nouns
         return _as_feat(self.convnet_verbs(img), self.D), _as_feat(self.convnet_nouns(img_n), self.D)
 
     def forward_features(self, feat_verbs, feat_nouns, gt_verb):
-        """`forward` on backbone features instead of images: (pred_verb, pred_nouns, gt_pred_nouns)."""
+        """`forward` on backbone features instead of images: (pred_verb, pred_nouns, gt_pred_nouns).  In bf16 mode the
+        features get their gradients when they require grad (one tensor passed as both inputs: the sum of the three
+        paths' gradients)."""
         fv, fn = _as_feat(feat_verbs, self.D), _as_feat(feat_nouns, self.D)
         self._step_seed = None
         if self.training and self.dropout_masks is None:
@@ -757,7 +767,8 @@ class FCGGNN(nn.Module):
             self._step_seed = None
 
     def _forward_paths(self, img, img_n, gt_verb, batch_size, feat_v=None, feat_n=None):
-        # the noun backbone is frozen and deterministic in eval mode: evaluate it once for both noun passes
+        # the noun backbone is deterministic unless its BatchNorm layers train: evaluate it once for both noun passes
+        # (trainable or not: autograd sums the two passes' gradients into the one feature tensor)
         if feat_n is None and img_n.is_cuda and not (self.training and _has_batchnorm_in_train(self.convnet_nouns)):
             feat_n = _as_feat(self.convnet_nouns(img_n), self.D)
         on_cuda = (feat_v if feat_v is not None else img).is_cuda
@@ -874,7 +885,7 @@ class FCGGNN(nn.Module):
 
     @torch.no_grad()
     def predict_situations(self, img, k=5, img_nouns=None):
-        """`situations_from_features` from images, through the two frozen backbones (same rules: no autograd, no
+        """`situations_from_features` from images, through the two backbones (same rules: no autograd, no
         dropout, no host synchronisation)."""
         fv, fn = self.extract_features(img, img_nouns)
         return self.situations_from_features(fv, fn, k=k)

@@ -16,7 +16,9 @@ ways.  Differences, all forced by the B200-first design:
   * `--no_pretrained` (extra flag) skips the ImageNet weights when there is no network; `--no_feature_cache` disables
     the cache;
   * `--topk_situations K` (extra flag, default 0 = off) adds the standard imSitu top-k situation metrics
-    (`situations.SituationScorer`) to --evaluate_dev / --evaluate_test, and K situations per image to --test_img.
+    (`situations.SituationScorer`) to --evaluate_dev / --evaluate_test, and K situations per image to --test_img;
+  * `--finetune_backbone` (extra flag) trains both ResNet-152 backbones with the GGNN stage (bf16 only; the dev
+    feature cache is off, and a checkpoint resumes only under the setting it was trained with).
 """
 import os
 from argparse import ArgumentParser
@@ -95,6 +97,12 @@ def train(model, train_loader, dev_loader, optimizer, max_epoch, encoder, model_
         for k in hist:
             hist[k] = checkpoint[k]
         model.load_state_dict(checkpoint['model_state_dict'])
+        saved = sum(len(g['params']) for g in checkpoint['optimizer_state_dict']['param_groups'])
+        now = sum(len(g['params']) for g in optimizer.param_groups)
+        if saved != now:
+            raise SystemExit("cannot resume: the checkpoint's optimizer state covers %d trainable tensors, this run trains "
+                             "%d -- resume with the same --finetune_backbone setting the checkpoint was trained with"
+                             % (saved, now))
         optimizer.load_state_dict(checkpoint['optimizer_state_dict'])
     if flat is None:
         flat = parallel.attach(model)
@@ -384,6 +392,8 @@ def build_parser():
                         help="recompute the frozen backbones on the dev set at every epoch, like the reference")
     parser.add_argument("--torch_optimizer", action="store_true",
                         help="torch.optim.Adamax + clip_grad_norm_ + gradient all-reduce instead of the fused sharded step")
+    parser.add_argument("--finetune_backbone", action="store_true",
+                        help="train both ResNet-152 backbones with the GGNN stage (turns the dev feature cache off)")
     parser.add_argument("--topk_situations", type=int, default=0,
                         help="K > 0: with --evaluate_dev / --evaluate_test also report the standard imSitu top-1 / top-K "
                              "situation metrics (2 <= K <= 16); with --test_img print the K best situations (K <= 16)")
@@ -404,6 +414,8 @@ def main(argv=None):
     if args.topk_situations == 1 and (args.evaluate_dev or args.evaluate_test):
         # the block reports top-1 and top-K and the mean of those 8 numbers; K = 1 would print a different mean
         parser.error("--topk_situations with --evaluate_dev / --evaluate_test needs K >= 2 (top-1 is always reported)")
+    if args.finetune_backbone and args.precision == "fp32":
+        parser.error("--finetune_backbone needs --precision bf16 (precision fp32 is a forward-only parity mode)")
     if not torch.cuda.is_available():
         raise SystemExit("situation_recognition_b200.sr needs a B200 GPU: the GGNN stage has no CPU path")
     if "RANK" in os.environ and int(os.environ.get("WORLD_SIZE", "1")) > 1:
@@ -443,6 +455,9 @@ def main(argv=None):
         torch.manual_seed(int(seed))
     model = FCGGNN(encoder, D_hidden_state=2048, precision=args.precision,
                    pretrained=False if args.no_pretrained else None).to(dev)
+    if args.finetune_backbone:      # before attach(): the flat buffers and the optimizer cover what requires grad
+        model.convnet_verbs.requires_grad_(True)
+        model.convnet_nouns.requires_grad_(True)
     parallel.broadcast_model(model)              # every rank built its own random init: rank 0's becomes everyone's
     if seed is not None:
         torch.manual_seed(int(seed) + 1000 * rank)      # per-rank dropout streams from here on
@@ -453,7 +468,8 @@ def main(argv=None):
     else:   # sr.py:80-83,472-473 as one fused kernel over flat buffers, sharded over the ranks
         flat = parallel.attach(model, flat_params=True)
         optimizer = parallel.FlatAdamax(flat, lr=args.lr, max_norm=1.0, group=dist.group.WORLD if world > 1 else None)
-    dev_cache = None if args.no_feature_cache else FeatureCache(len(dev_set), 2048, dev)
+    # the cache holds frozen backbones' features: a fine-tuned backbone changes them at every step
+    dev_cache = None if (args.no_feature_cache or args.finetune_backbone) else FeatureCache(len(dev_set), 2048, dev)
     torch.backends.cudnn.benchmark = True
 
     if len(args.resume_model) > 1:
