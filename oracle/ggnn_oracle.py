@@ -69,6 +69,13 @@ def linear(x, w, b):
     return x @ w.t() + b
 
 
+# The GRU's activations, looked up in this module at every call.  Tests rebind these names (never torch's own functions)
+# to give the backward other derivative factors, e.g. to emulate the CUDA path's bf16 stash (tests/regimes.py).
+gate_z = torch.sigmoid
+gate_r = torch.sigmoid
+candidate = torch.tanh
+
+
 def ggsnn_forward(p, hidden_state, mask=None, verb=False, steps=T_STEPS, trace=None):
     """model.py:59-86.  p: dict with '<name>.weight' / '<name>.bias' for W_p,W_z,U_z,W_r,U_r,W_h,U_h."""
     for t in range(steps):
@@ -82,12 +89,12 @@ def ggsnn_forward(p, hidden_state, mask=None, verb=False, steps=T_STEPS, trace=N
             nb = linear(nb, p["W_p.weight"], p["W_p.bias"])                             # :74 (bias on all 6 neighbours)
             nb = torch.sum(nb, 2)                                                       # :75
             neighbours = nb.contiguous().view(batch_size * R, -1)                       # :76-77
-        z_t = torch.sigmoid(linear(neighbours, p["W_z.weight"], p["W_z.bias"]) +
-                            linear(hidden_state, p["U_z.weight"], p["U_z.bias"]))        # :80
-        r_t = torch.sigmoid(linear(neighbours, p["W_r.weight"], p["W_r.bias"]) +
-                            linear(hidden_state, p["U_r.weight"], p["U_r.bias"]))        # :81
-        h_hat = torch.tanh(linear(neighbours, p["W_h.weight"], p["W_h.bias"]) +
-                           linear(r_t * hidden_state, p["U_h.weight"], p["U_h.bias"]))   # :82-83
+        z_t = gate_z(linear(neighbours, p["W_z.weight"], p["W_z.bias"]) +
+                     linear(hidden_state, p["U_z.weight"], p["U_z.bias"]))        # :80
+        r_t = gate_r(linear(neighbours, p["W_r.weight"], p["W_r.bias"]) +
+                     linear(hidden_state, p["U_r.weight"], p["U_r.bias"]))        # :81
+        h_hat = candidate(linear(neighbours, p["W_h.weight"], p["W_h.bias"]) +
+                          linear(r_t * hidden_state, p["U_h.weight"], p["U_h.bias"]))   # :82-83
         if trace is not None:
             trace.append({"m": neighbours, "z": z_t, "r": r_t, "h_hat": h_hat, "h_in": hidden_state})
         hidden_state = (1 - z_t) * hidden_state + z_t * h_hat                            # :84
@@ -104,16 +111,17 @@ def dropout(x, keep, p):
 # --------------------------------------------------------------------------------------------------
 # FCGGNN stage (backbones bypassed: `feat` is what convnet_*(img) returns, [B, D])
 def predict_nouns(params, feat, verbs, verb2roles, role_count, keep=None, drop_p=0.5):
-    """model.py:114-155 with img_features := feat."""
+    """model.py:114-155 with img_features := feat.  Runs on feat's device (fp64 on a GPU for the large cases)."""
     B = feat.shape[0]
     R = verb2roles.shape[1]
-    role_idx = torch.from_numpy(get_role_ids_batch(verb2roles, verbs.cpu().numpy()))     # :117
+    verbs = verbs.to(feat.device)
+    role_idx = torch.from_numpy(get_role_ids_batch(verb2roles, verbs.cpu().numpy())).to(feat.device)  # :117
     f = feat.expand(R, B, feat.size(1)).transpose(0, 1).contiguous().view(B * R, -1)     # :124-129
     verb_embd = params["verb_emb.weight"][verbs]                                         # :132
     role_embd = params["role_emb.weight"][role_idx].view(B * R, -1)                      # :133-135
     v = verb_embd.expand(R, B, verb_embd.size(1)).transpose(0, 1).contiguous().view(B * R, -1)  # :137-141
     node = F.relu(f * role_embd * v)                                                     # :143-144
-    mask = torch.from_numpy(get_adj_matrix_noself(role_count, verbs.cpu().numpy(), R)).to(feat.dtype)  # :147
+    mask = torch.from_numpy(get_adj_matrix_noself(role_count, verbs.cpu().numpy(), R)).to(feat.device, feat.dtype)  # :147
     out = ggsnn_forward(_sub(params, "ggsnn."), node, mask=mask, verb=False)             # :151
     logits = linear(dropout(out, keep, drop_p), params["nouns_classifier.1.weight"],
                     params["nouns_classifier.1.bias"])                                   # :152

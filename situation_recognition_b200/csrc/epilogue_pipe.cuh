@@ -122,7 +122,8 @@ __device__ __forceinline__ void pipe_compute(const PipeCtx& c, uint32_t s, const
         for (int i = 0; i < 8; ++i) z[i] = act_sigmoid<false>(acc[g * 8 + i] + b[g][i]);
         u64_st_bf16x8(s + c.ew * kB16Warp, lane, g, z);
       }
-    } else {         // r = sigmoid(acc + b); rh = r * h
+    } else {         // r = sigmoid(acc + b); rh = r * h; the stash keeps r folded (gate_fold)
+      const bool stash = (a.flags & FLAG_STASH) != 0;
       float h[4][8];
 #pragma unroll
       for (int g = 0; g < 4; ++g) slot_ld_f32x8(sf, lane, g, h[g]);
@@ -135,7 +136,11 @@ __device__ __forceinline__ void pipe_compute(const PipeCtx& c, uint32_t s, const
           rh[i] = r[i] * h[g][i];
         }
         u64_st_bf16x8(sb(kRegB0), lane, g, rh);
-        if (a.flags & FLAG_STASH) u64_st_bf16x8(sb(kRegB1), lane, g, r);
+        if (stash) {
+#pragma unroll
+          for (int i = 0; i < 8; ++i) r[i] = gate_fold(r[i]);
+          u64_st_bf16x8(sb(kRegB1), lane, g, r);
+        }
       }
     }
   } else if constexpr (EPI == EPI_H) {
@@ -210,8 +215,10 @@ __device__ __forceinline__ void pipe_compute(const PipeCtx& c, uint32_t s, const
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
         const float d = acc[g * 8 + i];
-        dp[i] = d * h[g][i] * r[g][i] * (1.0f - r[g][i]);
-        e[i] = d * r[g][i];
+        float rv, rc;
+        gate_unfold(r[g][i], rv, rc);     // r and 1 - r from the folded stash
+        dp[i] = d * h[g][i] * rv * rc;
+        e[i] = d * rv;
       }
       u64_st_bf16x8(s0, lane, g, dp);
       u64_st_bf16x8(s1, lane, g, e);

@@ -125,6 +125,16 @@ __device__ __forceinline__ float act_sigmoid(float x) {
     return fmaf(0.5f, t, 0.5f);
   }
 }
+// The reset gate as the training forward stashes it for the backward: r folded to min(r, 1 - r), negated when r > 1/2
+// (r - 1 is exact there, and -0 stands for r = 1).  The backward needs r (1 - r); rebuilt from a bf16 r, 1 - r loses
+// its relative precision as r saturates (bf16 values in [0.5, 1) are 2^-8 apart: 1 - r = 0.01 comes back to +-20 %).
+// The folded value keeps 1 - r to bf16's 2^-9 plus the 2.5e-4 absolute error of act_sigmoid, at no extra MUFU op.
+__device__ __forceinline__ float gate_fold(float r) { return r > 0.5f ? copysignf(1.0f - r, -1.0f) : r; }
+__device__ __forceinline__ void gate_unfold(float f, float& g, float& one_minus_g) {
+  const bool hi = signbit(f);
+  g = hi ? 1.0f + f : f;
+  one_minus_g = hi ? -f : 1.0f - f;
+}
 template <bool F32>
 __device__ __forceinline__ float act_tanh(float x) {
   if constexpr (F32) {
