@@ -147,6 +147,35 @@ int srg_situation_nouns(srg_handle* h, const float* feat, const int64_t* verbs, 
                         const float* verb_emb, const float* verb_logp, int64_t* labels, float* label_logp,
                         float* score, int precision, void* workspace, size_t workspace_bytes, void* stream);
 
+/* N-best situation decode: the n highest-scoring situations of each image b over its kv candidate verbs
+ * verbs[b*kv + j] (int64 [B, kv]).  A situation is a candidate j < kv plus one label per real role slot of its verb;
+ * its score is (verb_logp ? verb_logp[b*kv + j] : 0) + l_0 + l_1 + ..., summed in fp32 in slot order (as
+ * srg_situation_nouns sums it, so the 1-best score is bit-identical to that call's best candidate), where l_r is the
+ * label's log-softmax over the n_labels labels.  Order: score descending, then lower j, then the per-slot label ranks
+ * compared lexicographically from slot 0.  A situation with a label of rank >= n in some slot has n situations before
+ * it (replace that label by a better-ranked one), so only the top n labels of each slot are searched.
+ *   out_verbs     int64 [B, n]   : the verb of each entry (out-of-range ids clamped and flagged as in srg_nouns_forward)
+ *   out_verb_logp fp32  [B, n]   : its verb_logp (nullable; written when verb_logp is given)
+ *   labels        int64 [B, n, R]: -1 on the pad slots;  label_logp fp32 [B, n, R]: l_r, 0 on the pad slots
+ *   score         fp32  [B, n]
+ *   exact         uint8 [B]      : (nullable) 1 when the list is the n-best over ALL verbs, certified by
+ *                                  score[b, n-1] >= verb_bound[b]; verb_bound fp32 [B] (nullable) is the log-prob of
+ *                                  the best verb outside the beam.  Every l_r <= 0, and adding a non-positive number
+ *                                  never increases an fp32 sum, so no situation of an outside verb scores above it.
+ *                                  NULL verb_bound: no verb is outside the beam and every exact[b] is 1.
+ * If kv < n and no candidate verb has a role, fewer than n situations exist; the entries past them hold verb -1,
+ * score -inf, labels -1 and label log-probs 0.  The partial sums are pruned to n per slot, so two situations whose
+ * scores lie within one fp32 rounding of each other may come out in the other order than an exhaustive enumeration
+ * would give.  Deterministic: repeated calls are bit-identical.
+ * 1 <= kv <= min(16, n_verbs), 1 <= n <= min(16, n_labels); both precisions.  Workspace
+ * (srg_situation_nbest_workspace_bytes, enough at any 16-byte aligned address): srg_situation_workspace_bytes(B, kv)
+ * plus the per-slot lists [B*kv*R, n] int64 + fp32 (35 MB at B = 6144, kv = 5, R = 6, n = 16). */
+size_t srg_situation_nbest_workspace_bytes(srg_handle* h, int B, int kv, int n, int precision);
+int srg_situation_nbest(srg_handle* h, const float* feat, const int64_t* verbs, int B, int kv, const float* role_emb,
+                        const float* verb_emb, const float* verb_logp, const float* verb_bound, int n,
+                        int64_t* out_verbs, float* out_verb_logp, int64_t* labels, float* label_logp, float* score,
+                        uint8_t* exact, int precision, void* workspace, size_t workspace_bytes, void* stream);
+
 /* The keep-mask the Philox path applies for (*drop_seed, drop_stream, drop_p) on a [rows, D] slot matrix, written as
  * uint8 0/1 (tests: lets the oracle replay exactly the dropout a training step used). */
 int srg_dropout_mask(const int64_t* drop_seed, int64_t drop_stream, float drop_p, int64_t rows, int D, uint8_t* keep,

@@ -44,6 +44,9 @@ SIGNATURES = {
     "srg_topk_logsoftmax": (_i, [_vp, _i64, _i, _i, _i, _vp, _vp, _vp]),
     "srg_situation_workspace_bytes": (_sz, [_vp, _i, _i, _i]),
     "srg_situation_nouns": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _sz, _vp]),
+    "srg_situation_nbest_workspace_bytes": (_sz, [_vp, _i, _i, _i, _i]),
+    "srg_situation_nbest": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp,
+                                 _sz, _vp]),
     "srg_dropout_mask": (_i, [_vp, _i64, _f, _i64, _i, _vp, _vp]),
     "srg_ggnn_forward": (_i, [_vp, _i, _vp, _vp, _i, _i, _i, _vp, _sz, _vp]),
     "srg_count_targets": (_i, [_vp, _vp, _i, _vp, _vp]),

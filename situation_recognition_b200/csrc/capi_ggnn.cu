@@ -890,6 +890,22 @@ size_t situation_layout(const srg_handle* h, int B, int k, int prec, void* ws, P
   }
   return carve(h, SRG_MODE_NOUN, n, prec, 0, nullptr, true).bytes + logit_bytes;
 }
+
+// srg_situation_nbest's workspace: situation_layout(B, kv), then the per-slot top-n lists [B*kv*R, n] as int64 label
+// ids and fp32 log-probs.  The logits end 1024-aligned (their rows are Lpad = 256 m floats), so the lists are aligned
+// too, and they end within situation_layout's 1024 bytes of alignment slack plus their own size.
+size_t nbest_layout(const srg_handle* h, int B, int kv, int nb, int prec, void* ws, PathBufs* pb, float** logits,
+                    int64_t** slot_idx, float** slot_logp) {
+  const size_t slots = static_cast<size_t>(B) * kv * h->R * nb;
+  if (ws != nullptr) {
+    float* nl = nullptr;
+    situation_layout(h, B, kv, prec, ws, pb, &nl);
+    *logits = nl;
+    *slot_idx = reinterpret_cast<int64_t*>(nl + static_cast<size_t>(B) * kv * h->R * h->Lpad);
+    *slot_logp = reinterpret_cast<float*>(*slot_idx + slots);
+  }
+  return situation_layout(h, B, kv, prec, nullptr, nullptr, nullptr) + slots * (sizeof(int64_t) + sizeof(float));
+}
 }  // namespace
 
 extern "C" {
@@ -944,6 +960,41 @@ int srg_situation_nouns(srg_handle* h, const float* feat, const int64_t* verbs, 
   SRG_TRY(nouns_forward_body(h, pb, feat, k, verbs, n, role_emb, verb_emb, DropSpec(), nl, h->Lpad, precision, 0, s));
   SRG_TRY(launch_row_topk_logsoftmax(nl, h->Lpad, n * h->R, h->L, 1, labels, label_logp, s));
   return launch_situation_finish(verbs, h->d_role_count, h->V, h->R, n, verb_logp, labels, label_logp, score, s);
+}
+
+size_t srg_situation_nbest_workspace_bytes(srg_handle* h, int B, int kv, int n, int precision) {
+  if (!h || B <= 0 || kv < 1 || kv > 16 || n < 1 || n > 16) return 0;
+  return nbest_layout(h, B, kv, n, precision, nullptr, nullptr, nullptr, nullptr, nullptr);
+}
+
+int srg_situation_nbest(srg_handle* h, const float* feat, const int64_t* verbs, int B, int kv, const float* role_emb,
+                        const float* verb_emb, const float* verb_logp, const float* verb_bound, int n,
+                        int64_t* out_verbs, float* out_verb_logp, int64_t* labels, float* label_logp, float* score,
+                        uint8_t* exact, int precision, void* workspace, size_t workspace_bytes, void* stream) {
+  SRG_CHECK(h != nullptr, "srg_situation_nbest: null handle");
+  DeviceGuard guard_(h->device);
+  SRG_CHECK(kv >= 1 && kv <= 16 && kv <= h->V, "srg_situation_nbest: kv=%d must be in [1, min(16, n_verbs=%d)]", kv,
+            h->V);
+  SRG_CHECK(n >= 1 && n <= 16 && n <= h->L, "srg_situation_nbest: n=%d must be in [1, min(16, n_labels=%d)]", n, h->L);
+  SRG_CHECK(B > 0 && static_cast<int64_t>(B) * kv * h->R <= (1 << 30), "srg_situation_nbest: bad batch %d", B);
+  PathBufs pb;
+  SRG_TRY(check_ws(h, SRG_MODE_NOUN, B * kv, precision, 0, workspace, workspace_bytes, &pb, true));
+  float* nl = nullptr;
+  int64_t* slot_idx = nullptr;
+  float* slot_logp = nullptr;
+  const size_t need = nbest_layout(h, B, kv, n, precision, workspace, &pb, &nl, &slot_idx, &slot_logp);
+  if (need > workspace_bytes)
+    return set_error(SRG_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+  SRG_CHECK(h->tables_set, "srg_situation_nbest: call srg_set_tables first");
+  SRG_CHECK(h->packed_prec == precision, "srg_situation_nbest: weights are not packed for precision %d", precision);
+  SRG_CHECK(feat && verbs && role_emb && verb_emb && out_verbs && labels && label_logp && score,
+            "srg_situation_nbest: null argument");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int nc = B * kv;
+  SRG_TRY(nouns_forward_body(h, pb, feat, kv, verbs, nc, role_emb, verb_emb, DropSpec(), nl, h->Lpad, precision, 0, s));
+  SRG_TRY(launch_row_topk_logsoftmax(nl, h->Lpad, nc * h->R, h->L, n, slot_idx, slot_logp, s));
+  return launch_situation_nbest(verbs, h->d_role_count, h->V, h->R, B, kv, n, verb_logp, verb_bound, slot_idx, slot_logp,
+                                out_verbs, out_verb_logp, labels, label_logp, score, exact, s);
 }
 
 int srg_verb_forward(srg_handle* h, const float* feat, int B, const uint8_t* keep, float drop_p,

@@ -121,6 +121,16 @@ int launch_row_topk_logsoftmax(const float* x, int64_t ldl, int rows, int n, int
 // hold the per-slot top-1 on entry and are finished in place.
 int launch_situation_finish(const int64_t* verb, const int32_t* role_count, int n_verbs, int R, int n_cand,
                             const float* verb_logp, int64_t* labels, float* label_logp, float* score, cudaStream_t s);
+// N-best decode of image b < B from its kv candidates verbs[b*kv + j] (one CTA per image, one warp per candidate):
+// the n best (score desc, then lower j, then the per-slot label ranks lexicographically) of the situations built from
+// the per-slot top-n lists slot_idx / slot_logp [B*kv*R, n].  score = (verb_logp ? verb_logp : 0) + l_0 + l_1 + ...
+// in fp32, slot order.  out_verbs [B,n], out_verb_logp [B,n] (written when both it and verb_logp are given), labels /
+// label_logp [B,n,R] (-1 / 0 on pad slots), score [B,n]; exact [B] (nullable) = no verb_bound or score[b,n-1] >=
+// verb_bound[b].  1 <= kv, n <= 16, R <= 8.
+int launch_situation_nbest(const int64_t* verbs, const int32_t* role_count, int n_verbs, int R, int B, int kv, int n,
+                           const float* verb_logp, const float* verb_bound, const int64_t* slot_idx,
+                           const float* slot_logp, int64_t* out_verbs, float* out_verb_logp, int64_t* labels,
+                           float* label_logp, float* score, uint8_t* exact, cudaStream_t s);
 // fp32 [rows, ld] (first n_valid columns) -> bf16 [rows, n_pad], zero padded
 int launch_cast_pad(const float* src, int64_t ld, int rows, int n_valid, int n_pad, bf16* dst, int accumulate,
                     cudaStream_t s);

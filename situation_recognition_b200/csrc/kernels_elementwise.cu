@@ -1205,10 +1205,25 @@ k_row_topk_logsoftmax(const float* __restrict__ x, int64_t ldl, int rows, int n,
     auto fold = [&](auto col) {
       float cm = -INFINITY;
 #pragma unroll
-      for (int i = 0; i < kTopkChunk; ++i) {
-        cm = fmaxf(cm, v[i]);
-        topk_insert<KMAX>(tv, tc, v[i], col(i));
+      for (int i = 0; i < kTopkChunk; ++i) cm = fmaxf(cm, v[i]);
+      // 1 < k <= 8: the k-th largest of the 32 lane maxima of the chunk is a value that k columns of the row reach, so
+      // a column below it is not among the k best and skips the insertion (about k columns of a chunk pass, instead of
+      // every column paying a KMAX-step insertion whenever one lane of the warp inserts).  On 184 k rows of 2001 labels
+      // (B200) this takes k = 5 from 5.3 to 3.8 ms, but k = 16 from 9.9 to 28.7 ms, so KMAX = 16 keeps the plain loop.
+      float theta = -INFINITY;
+      if constexpr (KMAX > 1 && KMAX <= 8) {
+        int rank = 0;                    // lanes with a larger maximum, ties to the lower lane: a permutation of 0..31
+        for (int l = 0; l < 32; ++l) {
+          const float o = __shfl_sync(0xffffffffu, cm, l);
+          rank += (o > cm || (o == cm && l < lane)) ? 1 : 0;
+        }
+        const unsigned sel = __ballot_sync(0xffffffffu, rank == k - 1);
+        const float t = __shfl_sync(0xffffffffu, cm, sel ? __ffs(sel) - 1 : 0);
+        if (sel) theta = t;              // always one lane (fmaxf drops NaN, so cm is never NaN); else no filter
       }
+#pragma unroll
+      for (int i = 0; i < kTopkChunk; ++i)
+        if (!(v[i] < theta)) topk_insert<KMAX>(tv, tc, v[i], col(i));
       const float mn = fmaxf(m, cm);
       if (mn > -INFINITY) {
         float acc = 0.f;
@@ -1296,6 +1311,165 @@ __global__ void k_situation_finish(const int64_t* __restrict__ verb, const int32
       }
     }
     score[u] = s;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------ n-best decode
+// An entry is (score, key) with key = (candidate j << 32) | rank tuple, the tuple 4 bits per slot, slot 0 in bits
+// 28..31, so that comparing keys compares (j, ranks) lexicographically.  (s, k) ranks before (t, l): larger score, ties
+// to the smaller key.  A NaN score ranks as -inf, so every entry ranks before the sentinel (-inf, ~0) of an empty place.
+constexpr int kNbestMax = 16;                                 // largest n and candidate count kv
+constexpr int kNbestPerLane = kNbestMax * kNbestMax / 32;     // a warp selects from at most 16 x 16 entries
+
+__device__ __forceinline__ bool nbest_before(float s, uint64_t k, float t, uint64_t l) {
+  s = (s == s) ? s : -INFINITY;
+  t = (t == t) ? t : -INFINITY;
+  return s > t || (s == t && k < l);
+}
+
+// The warp writes the `keep` best of the entries its lanes hold (lane l holds entry l + 32 q as es[q] / ek[q]; empty
+// places hold the sentinel) to os / ok in order: `keep` rounds of a warp argmax, after each the winner drops its entry.
+// Keys are unique among the real entries and keep <= their number, so every round has exactly one winner.
+__device__ __forceinline__ void nbest_warp_select(const float (&es)[kNbestPerLane], const uint64_t (&ek)[kNbestPerLane],
+                                                  int keep, float* os, uint64_t* ok) {
+  const int lane = threadIdx.x & 31;
+  unsigned alive = (1u << kNbestPerLane) - 1;
+  for (int i = 0; i < keep; ++i) {
+    float bs = -INFINITY;
+    uint64_t bk = ~0ull;
+    int bq = -1;
+#pragma unroll
+    for (int q = 0; q < kNbestPerLane; ++q)
+      if (((alive >> q) & 1u) && nbest_before(es[q], ek[q], bs, bk)) { bs = es[q]; bk = ek[q]; bq = q; }
+    const uint64_t mine = bk;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ts = __shfl_xor_sync(0xffffffffu, bs, o);
+      const uint64_t tk = __shfl_xor_sync(0xffffffffu, bk, o);
+      if (nbest_before(ts, tk, bs, bk)) { bs = ts; bk = tk; }
+    }
+    if (bq >= 0 && mine == bk) alive &= ~(1u << bq);
+    if (lane == 0) { os[i] = bs; ok[i] = bk; }
+  }
+  __syncwarp();
+}
+
+// One CTA per image b, one warp per candidate j < kv.  slot_idx / slot_logp [B*kv*R, n]: the n best labels of every
+// role slot and their log-softmax, descending (k_row_topk_logsoftmax with k = n).
+// Warp j: its list starts as the single partial (verb_logp, empty tuple); each real slot r merges the list (<= n
+// partial sums) with the slot's n labels into <= n*n sums cur + logp (one fp32 add each, so that the sums are formed
+// in slot order exactly as k_situation_finish forms them) and keeps the n best.  Then warp 0 merges the kv lists.
+__global__ void __launch_bounds__(kNbestMax * 32)
+k_situation_nbest(const int64_t* __restrict__ verbs, const int32_t* __restrict__ role_count, int n_verbs, int R,
+                  int kv, int n, const float* __restrict__ verb_logp, const float* __restrict__ verb_bound,
+                  const int64_t* __restrict__ slot_idx, const float* __restrict__ slot_logp,
+                  int64_t* __restrict__ out_verbs, float* __restrict__ out_verb_logp, int64_t* __restrict__ labels,
+                  float* __restrict__ label_logp, float* __restrict__ score, uint8_t* __restrict__ exact) {
+  __shared__ float ls[kNbestMax][kNbestMax];
+  __shared__ uint64_t lk[kNbestMax][kNbestMax];
+  __shared__ int lcnt[kNbestMax];
+  __shared__ float ws[kNbestMax];
+  __shared__ uint64_t wk[kNbestMax];
+  __shared__ int wcount;
+  const int b = blockIdx.x;
+  const int lane = threadIdx.x & 31;
+  const int j = threadIdx.x >> 5;
+  const float sentinel_s = -INFINITY;
+  const uint64_t sentinel_k = ~0ull;
+  if (j < kv) {
+    const int64_t u = static_cast<int64_t>(b) * kv + j;
+    int64_t v = verbs[u];
+    if (v < 0 || v >= n_verbs) v = 0;    // clamped as in the role graph (k_prep_rows raised the flag)
+    const int nr = role_count[v];
+    float* cs = ls[j];
+    uint64_t* ck = lk[j];
+    if (lane == 0) {
+      cs[0] = (verb_logp != nullptr) ? verb_logp[u] : 0.f;
+      ck[0] = static_cast<uint64_t>(j) << 32;
+    }
+    __syncwarp();
+    int cnt = 1;
+    for (int r = 0; r < nr; ++r) {
+      const float* lp = slot_logp + (u * R + r) * n;
+      const int m = cnt * n;
+      float es[kNbestPerLane];
+      uint64_t ek[kNbestPerLane];
+#pragma unroll
+      for (int q = 0; q < kNbestPerLane; ++q) {
+        const int c = lane + 32 * q;
+        es[q] = sentinel_s;
+        ek[q] = sentinel_k;
+        if (c < m) {
+          const int i = c / n, l = c - i * n;
+          es[q] = cs[i] + lp[l];
+          ek[q] = ck[i] | (static_cast<uint64_t>(l) << (28 - 4 * r));
+        }
+      }
+      __syncwarp();                      // every lane has read the list before the select overwrites it
+      cnt = min(n, m);
+      nbest_warp_select(es, ek, cnt, cs, ck);
+    }
+    if (lane == 0) lcnt[j] = cnt;
+  }
+  __syncthreads();
+  if (j == 0) {
+    float es[kNbestPerLane];
+    uint64_t ek[kNbestPerLane];
+    int total = 0;
+    for (int c = 0; c < kv; ++c) total += lcnt[c];
+#pragma unroll
+    for (int q = 0; q < kNbestPerLane; ++q) {
+      const int e = lane + 32 * q;
+      const int c = e / n, i = e - c * n;
+      es[q] = sentinel_s;
+      ek[q] = sentinel_k;
+      if (c < kv && i < lcnt[c]) { es[q] = ls[c][i]; ek[q] = lk[c][i]; }
+    }
+    const int keep = min(n, total);
+    nbest_warp_select(es, ek, keep, ws, wk);
+    if (lane == 0) wcount = keep;
+  }
+  __syncthreads();
+  const int keep = wcount;
+  // output entry i < keep: the winner's verb, labels and log-probs.  Entries past the last situation get verb -1, score
+  // -inf, labels -1 and label log-probs 0; that happens only when kv < n and no candidate verb has a role
+  for (int t = threadIdx.x; t < n * (R + 1); t += blockDim.x) {
+    const int i = t / (R + 1), r = t - i * (R + 1) - 1;       // r = -1: the entry's verb and score
+    const int64_t o = static_cast<int64_t>(b) * n + i;
+    if (i >= keep) {
+      if (r < 0) {
+        out_verbs[o] = -1;
+        score[o] = -INFINITY;
+        if (out_verb_logp != nullptr) out_verb_logp[o] = -INFINITY;
+      } else {
+        labels[o * R + r] = -1;
+        label_logp[o * R + r] = 0.f;
+      }
+      continue;
+    }
+    const int c = static_cast<int>(wk[i] >> 32);
+    const uint32_t tuple = static_cast<uint32_t>(wk[i]);
+    const int64_t u = static_cast<int64_t>(b) * kv + c;
+    int64_t v = verbs[u];
+    if (v < 0 || v >= n_verbs) v = 0;
+    if (r < 0) {
+      out_verbs[o] = v;
+      score[o] = ws[i];
+      if (out_verb_logp != nullptr) out_verb_logp[o] = verb_logp[u];
+    } else if (r < role_count[v]) {
+      const int rank = (tuple >> (28 - 4 * r)) & 15u;
+      labels[o * R + r] = slot_idx[(u * R + r) * n + rank];
+      label_logp[o * R + r] = slot_logp[(u * R + r) * n + rank];
+    } else {
+      labels[o * R + r] = -1;
+      label_logp[o * R + r] = 0.f;
+    }
+  }
+  // every verb outside the beam has log-prob <= verb_bound, and l_r <= 0 with monotone rounding keeps each of its
+  // situations' scores <= verb_bound; outside verbs rank after the beam's on equal scores
+  if (threadIdx.x == 0 && exact != nullptr) {
+    const float last = (keep == n) ? ws[n - 1] : -INFINITY;
+    exact[b] = (verb_bound == nullptr || last >= verb_bound[b]) ? 1 : 0;
   }
 }
 
@@ -1423,6 +1597,21 @@ int launch_situation_finish(const int64_t* verb, const int32_t* role_count, int 
   if (n_cand <= 0) return SRG_OK;
   k_situation_finish<<<grid_for(n_cand), kThreads, 0, s>>>(verb, role_count, n_verbs, R, n_cand, verb_logp, labels,
                                                           label_logp, score);
+  SRG_LAUNCH_CHECK();
+  return SRG_OK;
+}
+
+int launch_situation_nbest(const int64_t* verbs, const int32_t* role_count, int n_verbs, int R, int B, int kv, int n,
+                           const float* verb_logp, const float* verb_bound, const int64_t* slot_idx,
+                           const float* slot_logp, int64_t* out_verbs, float* out_verb_logp, int64_t* labels,
+                           float* label_logp, float* score, uint8_t* exact, cudaStream_t s) {
+  if (B <= 0) return SRG_OK;
+  if (kv < 1 || kv > kNbestMax || n < 1 || n > kNbestMax || R < 1 || R > kMaxR)
+    return set_error(SRG_ERR_ARG, "situation_nbest: need 1 <= kv, n <= %d and 1 <= R <= %d (kv=%d, n=%d, R=%d)",
+                     kNbestMax, kMaxR, kv, n, R);
+  k_situation_nbest<<<B, 32 * kv, 0, s>>>(verbs, role_count, n_verbs, R, kv, n, verb_logp, verb_bound, slot_idx,
+                                          slot_logp, out_verbs, verb_logp ? out_verb_logp : nullptr, labels,
+                                          label_logp, score, exact);
   SRG_LAUNCH_CHECK();
   return SRG_OK;
 }

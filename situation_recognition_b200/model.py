@@ -38,9 +38,12 @@ Situations.__doc__ = """Top-k situations of a batch (FCGGNN.situations_from_feat
     verbs [B,k] int64 (descending verb logit, ties to the lower id); verb_logp [B,k] fp32 log-softmax over the verbs, or
     None when the verbs were given; labels [B,k,R] int64 top-1 label per role slot, -1 on pad slots; label_logp [B,k,R]
     fp32 its log-softmax over the labels, 0 on pad slots; score [B,k] = verb_logp + sum over the real slots of
-    label_logp (label term only when the verbs were given)."""
+    label_logp (label term only when the verbs were given).
+    FCGGNN.nbest_situations_from_features returns the same fields for the n best situations of each image, which may
+    repeat a verb with other labels: verbs / verb_logp [B,n], labels / label_logp [B,n,R], score [B,n] descending."""
 
 MAX_TOPK = 16
+MAX_VERB_BEAM = MAX_TOPK - 1      # the n-best decode also reads the log-prob of the best verb outside the beam
 
 
 def _pad256(n):
@@ -195,12 +198,15 @@ class _Engine:
         """Current stream of THIS engine's device (the caller's current device may be another GPU)."""
         return _lib.stream_ptr(self.device)
 
-    def workspace(self, mode, B, prec, save, k=None):
-        """Uninitialised device workspace of one call; k: srg_situation_nouns on B images x k candidate verbs."""
+    def workspace(self, mode, B, prec, save, k=None, nbest=None):
+        """Uninitialised device workspace of one call; k: srg_situation_nouns on B images x k candidate verbs, and
+        with nbest: srg_situation_nbest of the `nbest` best situations over k candidate verbs."""
         if k is None:
             n = self.lib.srg_workspace_bytes(self.h, mode, B, prec, int(save))
-        else:
+        elif nbest is None:
             n = self.lib.srg_situation_workspace_bytes(self.h, B, k, prec)
+        else:
+            n = self.lib.srg_situation_nbest_workspace_bytes(self.h, B, k, nbest, prec)
         ws = torch.empty(n, dtype=torch.uint8, device=self.device)
         if _POISON_WS:      # tests: every byte 0xFF = NaN as fp32 / bf16, -1 as int32: a read of a workspace location
             ws.fill_(0xFF)  # nobody wrote shows up as NaN in the results instead of hiding behind fresh (zeroed) memory
@@ -882,6 +888,75 @@ class FCGGNN(nn.Module):
                                                _lib.ptr(label_logp), _lib.ptr(score), prec, _lib.ptr(ws), ws.numel(),
                                                stream))
         return Situations(verbs, verb_logp, labels, label_logp, score)
+
+    @torch.no_grad()
+    def nbest_situations_from_features(self, feat_verbs, feat_nouns, n=5, verb_beam=None, verbs=None):
+        """The n highest-scoring situations of each image from the backbone features ([B, D] each), and whether the
+        list is certified to be the n-best over all verbs.  Returns `(Situations, exact)`, `exact` bool [B].
+
+        A situation is one of the kv = verb_beam (default n, at most 15) best verbs plus one label per role of that
+        verb; its score is verb_logp + l_0 + l_1 + ... summed in fp32 in slot order, l_r the label's log-softmax over
+        the labels.  Order: score descending, then the better-ranked verb, then the per-slot label ranks compared
+        lexicographically from slot 0.  The 1-best entry is bit-identical to the best-scoring candidate of
+        `situations_from_features(k=kv)`.  Situations whose scores lie within one fp32 rounding of each other may come
+        out in either order.  exact[b]: score[b, n-1] >= the log-prob of the (kv+1)-th verb, so no situation of a verb
+        outside the beam can enter the list (every label log-prob is <= 0).
+        verbs ([B, kv'] int64, optional): decode these candidate verbs instead (feat_verbs is then not used and may be
+        None; verb_logp is None, the score is the label term only and exact is all True) -- e.g. `verbs=v[:, None]`
+        for the n best label assignments of verb v.
+
+        Same rules as `situations_from_features`: no autograd node, no dropout, no host synchronisation (it can be
+        captured in a CUDA graph), honours `self.precision`."""
+        fn = _as_feat(feat_nouns, self.D)
+        dev = fn.device
+        eng = self._engine_for(dev)
+        B = fn.shape[0]
+        if not 1 <= n <= min(MAX_TOPK, eng.L):
+            raise _lib.SrgError("n=%d must be in [1, %d]" % (n, min(MAX_TOPK, eng.L)))
+        if verbs is not None:
+            verbs = verbs.to(device=dev, dtype=torch.int64).contiguous()
+            if verbs.dim() != 2 or verbs.shape[0] != B:
+                raise _lib.SrgError("verbs must be [B, kv] = [%d, kv], got %s" % (B, tuple(verbs.shape)))
+            kv = verbs.shape[1]
+            if not 1 <= kv <= min(MAX_TOPK, eng.V):
+                raise _lib.SrgError("verbs has %d columns, must be in [1, %d]" % (kv, min(MAX_TOPK, eng.V)))
+        else:
+            kv = n if verb_beam is None else verb_beam
+            if not 1 <= kv <= min(MAX_VERB_BEAM, eng.V):
+                raise _lib.SrgError("verb_beam=%d must be in [1, %d]" % (kv, min(MAX_VERB_BEAM, eng.V)))
+        prec = _prec_code(self.precision)
+        eng.ensure_packed(self, prec)
+        stream = eng.stream()
+        verb_logp = verb_bound = None
+        if verbs is None:
+            fv = _as_feat(feat_verbs, self.D)
+            if fv.shape[0] != B:
+                raise _lib.SrgError("feat_verbs has %d rows, feat_nouns %d" % (fv.shape[0], B))
+            logits = torch.empty(B, eng.Vpad, dtype=torch.float32, device=dev)
+            ws = eng.workspace(SRG_MODE_VERB, B, prec, False)
+            _lib.check(eng.lib.srg_verb_forward(eng.h, _lib.ptr(fv), B, None, 0.0, None, 0, _lib.ptr(logits), eng.Vpad,
+                                                prec, 0, _lib.ptr(ws), ws.numel(), stream))
+            kt = min(kv + 1, eng.V)              # kt = kv: every verb is in the beam, nothing to bound
+            top = torch.empty(B, kt, dtype=torch.int64, device=dev)
+            top_logp = torch.empty(B, kt, dtype=torch.float32, device=dev)
+            _lib.check(eng.lib.srg_topk_logsoftmax(_lib.ptr(logits), eng.Vpad, B, eng.V, kt, _lib.ptr(top),
+                                                   _lib.ptr(top_logp), stream))
+            verbs, verb_logp = top[:, :kv].contiguous(), top_logp[:, :kv].contiguous()
+            if kt > kv:
+                verb_bound = top_logp[:, kv].contiguous()
+        out_verbs = torch.empty(B, n, dtype=torch.int64, device=dev)
+        out_verb_logp = None if verb_logp is None else torch.empty(B, n, dtype=torch.float32, device=dev)
+        labels = torch.empty(B, n, eng.R, dtype=torch.int64, device=dev)
+        label_logp = torch.empty(B, n, eng.R, dtype=torch.float32, device=dev)
+        score = torch.empty(B, n, dtype=torch.float32, device=dev)
+        exact = torch.empty(B, dtype=torch.bool, device=dev)             # the kernel stores one byte 0 / 1 per image
+        ws = eng.workspace(SRG_MODE_NOUN, B, prec, False, k=kv, nbest=n)
+        _lib.check(eng.lib.srg_situation_nbest(eng.h, _lib.ptr(fn), _lib.ptr(verbs), B, kv, _lib.ptr(self.role_emb.weight),
+                                               _lib.ptr(self.verb_emb.weight), _lib.ptr(verb_logp),
+                                               _lib.ptr(verb_bound), n, _lib.ptr(out_verbs), _lib.ptr(out_verb_logp),
+                                               _lib.ptr(labels), _lib.ptr(label_logp), _lib.ptr(score),
+                                               _lib.ptr(exact), prec, _lib.ptr(ws), ws.numel(), stream))
+        return Situations(out_verbs, out_verb_logp, labels, label_logp, score), exact
 
     @torch.no_grad()
     def predict_situations(self, img, k=5, img_nouns=None):

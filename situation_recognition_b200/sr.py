@@ -18,7 +18,9 @@ ways.  Differences, all forced by the B200-first design:
   * `--topk_situations K` (extra flag, default 0 = off) adds the standard imSitu top-k situation metrics
     (`situations.SituationScorer`) to --evaluate_dev / --evaluate_test, and K situations per image to --test_img;
   * `--finetune_backbone` (extra flag) trains both ResNet-152 backbones with the GGNN stage (bf16 only; the dev
-    feature cache is off, and a checkpoint resumes only under the setting it was trained with).
+    feature cache is off, and a checkpoint resumes only under the setting it was trained with);
+  * `--nbest_situations N` (extra flag, with --test_img) prints the N highest-scoring situations, which may share a
+    verb, and whether that list is certified to be the N best over all verbs.
 """
 import os
 from argparse import ArgumentParser
@@ -283,20 +285,46 @@ def results(model, image, encoder, gt_verb, dataset_folder="imSitu"):
     return verb_name, verb_prob, labels, labels_prob
 
 
+def _image_features(model, image, encoder):
+    """(device, verb features, noun features) of one image file, in eval mode."""
+    from PIL import Image
+    model.eval()
+    dev = next(model.parameters()).device
+    img = encoder.dev_transform(Image.open(image).convert('RGB')).unsqueeze(0).to(dev)
+    return (dev,) + tuple(model.extract_features(img))
+
+
 def results_topk(model, image, encoder, k, gt_verb="", dataset_folder="imSitu"):
     """The k best situations of one image: [(verb, verb probability % or None, score, {role: (gloss, label
     probability %)})].  With a known `gt_verb` only that verb's situation.  Probabilities are softmaxes over the
     verbs / over the labels."""
-    from PIL import Image
-    model.eval()
-    dev = next(model.parameters()).device
+    dev, fv, fn = _image_features(model, image, encoder)
     nouns_space, verbs_space = _spaces(dataset_folder)
-    img = encoder.dev_transform(Image.open(image).convert('RGB')).unsqueeze(0).to(dev)
-    fv, fn = model.extract_features(img)
     if gt_verb and encoder.verb_list.count(gt_verb):
         s = model.situations_from_features(fv, fn, verbs=torch.tensor([[encoder.verb_list.index(gt_verb)]], device=dev))
     else:
         s = model.situations_from_features(fv, fn, k=k)
+    return _situation_rows(s, encoder, nouns_space, verbs_space)
+
+
+NBEST_VERB_BEAM = 15     # the widest verb beam: at one image the cost does not matter, and more lists are certified
+
+
+def results_nbest(model, image, encoder, n, gt_verb="", dataset_folder="imSitu"):
+    """The n best situations of one image, as `results_topk` returns them, and whether the list is certified to be
+    the n best over all verbs.  With a known `gt_verb` the n best label assignments of that verb (always certified)."""
+    dev, fv, fn = _image_features(model, image, encoder)
+    nouns_space, verbs_space = _spaces(dataset_folder)
+    if gt_verb and encoder.verb_list.count(gt_verb):
+        s, exact = model.nbest_situations_from_features(
+            fv, fn, n=n, verbs=torch.tensor([[encoder.verb_list.index(gt_verb)]], device=dev))
+    else:
+        s, exact = model.nbest_situations_from_features(fv, fn, n=n, verb_beam=min(NBEST_VERB_BEAM,
+                                                                                   encoder.get_num_verbs()))
+    return _situation_rows(s, encoder, nouns_space, verbs_space), bool(exact[0])
+
+
+def _situation_rows(s, encoder, nouns_space, verbs_space):
     verbs, labels, label_logp, score = s.verbs[0].tolist(), s.labels[0].tolist(), s.label_logp[0].exp().tolist(), \
         s.score[0].tolist()
     verb_p = s.verb_logp[0].exp().tolist() if s.verb_logp is not None else [None] * len(verbs)
@@ -397,6 +425,9 @@ def build_parser():
     parser.add_argument("--topk_situations", type=int, default=0,
                         help="K > 0: with --evaluate_dev / --evaluate_test also report the standard imSitu top-1 / top-K "
                              "situation metrics (2 <= K <= 16); with --test_img print the K best situations (K <= 16)")
+    parser.add_argument("--nbest_situations", type=int, default=None,
+                        help="with --test_img: also print the N best situations (1 <= N <= 16), which may share a verb, "
+                             "and whether the list is certified to be the N best over all verbs")
     return parser
 
 
@@ -414,6 +445,11 @@ def main(argv=None):
     if args.topk_situations == 1 and (args.evaluate_dev or args.evaluate_test):
         # the block reports top-1 and top-K and the mean of those 8 numbers; K = 1 would print a different mean
         parser.error("--topk_situations with --evaluate_dev / --evaluate_test needs K >= 2 (top-1 is always reported)")
+    if args.nbest_situations is not None:
+        if not 1 <= args.nbest_situations <= 16:
+            parser.error("--nbest_situations must be in [1, 16], got %d" % args.nbest_situations)
+        if not args.test_img:
+            parser.error("--nbest_situations needs --test_img")
     if args.finetune_backbone and args.precision == "fp32":
         parser.error("--finetune_backbone needs --precision bf16 (precision fp32 is a forward-only parity mode)")
     if not torch.cuda.is_available():
@@ -499,6 +535,13 @@ def main(argv=None):
                 sits = results_topk(model, args.test_img, encoder, args.topk_situations, args.verb, args.dataset_folder)
             print('&' * 50)
             _print_situations(sits)
+        if args.nbest_situations is not None:
+            with torch.no_grad():
+                sits, exact = results_nbest(model, args.test_img, encoder, args.nbest_situations, args.verb,
+                                            args.dataset_folder)
+            print('&' * 50)
+            _print_situations(sits)
+            print('n-best list certified over all verbs: {}'.format('yes' if exact else 'no'))
     elif args.subset > 0:
         analize_subset(model, dev_set, encoder, args.subset, args.dataset_folder, args.imgset_dir)
     else:
