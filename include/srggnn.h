@@ -230,6 +230,60 @@ int srg_verb_loss_backward(srg_handle* h, const float* logits, int64_t ldl, cons
                            float* dlogits, void* dlogits_bf16, int accumulate, const float* stats, void* stream);
 size_t srg_workspace_dlogits_offset(srg_handle* h, int mode, int B, const void* workspace);
 
+/* Class weights, label smoothing and the reduction of the two losses: torch.nn.functional.cross_entropy(weight,
+ * label_smoothing, reduction), exactly.  For logits z over C classes, target y, class weights w (NULL = all 1),
+ * W = sum_c w_c and smoothing eps in [0, 1], the loss of one target is
+ *   l = (1 - eps) w_y (lse - z_y) + (eps / C) sum_c w_c (lse - z_c),   0 for an ignored target (nouns: y = n_labels),
+ * and dl/dz_c = (1 - eps) w_y (p_c - [c == y]) + (eps / C) (W p_c - w_c).  Reductions:
+ *   SRG_REDUCTION_MEAN : sum l / (sum of w_y over the non-ignored targets): the nouns per annotation, summed over the 3
+ *                        (counts = srg_count_targets_weighted), the verbs over the batch (batch_total =
+ *                        srg_verb_weight_total, or inv_batch when there are no class weights).  A zero denominator
+ *                        contributes 0, not NaN as torch gives.
+ *   SRG_REDUCTION_SUM  : sum l (counts, inv_batch and batch_total are not read);
+ *   SRG_REDUCTION_NONE : l per target into per_target_loss (fp32, laid out like the targets: [B] verbs, [B, 3, R] nouns;
+ *                        0 on ignored targets); `loss` may be NULL.  The backward calls take d(loss)/dl per target in
+ *                        grad_per_target (same layout), times grad_scale and *grad_out when given.
+ * per_target_loss under MEAN / SUM (nullable): receives each target's term of the scalar, and *loss += their sum in a
+ * fixed order (one more launch), so that repeated calls give bit-identical losses; NULL: per-CTA atomics, as the
+ * default options.  Only the forward calls write it.  class_weight: device fp32 [n_classes] (n_verbs or n_labels).
+ * A NULL srg_loss_opts, or one whose fields all hold their defaults (no weight, eps = 0, MEAN, no per-target pointers),
+ * runs exactly the default-option kernels.  Bad options (eps outside [0, 1], an unknown reduction, NONE without
+ * per_target_loss in a forward call or without grad_per_target in a call that writes a gradient) return an error and
+ * launch nothing. */
+enum { SRG_REDUCTION_MEAN = 0, SRG_REDUCTION_SUM = 1, SRG_REDUCTION_NONE = 2 };
+typedef struct srg_loss_opts {
+  const float* class_weight;
+  float label_smoothing;
+  int reduction;
+  float* per_target_loss;
+  const float* grad_per_target;
+} srg_loss_opts;
+
+/* Weighted denominators of the MEAN reduction, summed by one CTA in a fixed order (no atomics, so an eager step and a
+ * replayed CUDA graph get bit-identical values).  counts: device fp32 [3] = sum of class_weight[y] over the
+ * non-ignored targets of each annotation (overwritten; class_weight NULL = srg_count_targets).  total: device fp32
+ * scalar = sum of class_weight[y] over the B verbs (overwritten).  All-reduce both over the ranks of a sharded batch. */
+int srg_count_targets_weighted(srg_handle* h, const int64_t* gt_nouns, int B, const float* class_weight, float* counts,
+                               void* stream);
+int srg_verb_weight_total(srg_handle* h, const int64_t* gt_verb, int B, const float* class_weight, float* total,
+                          void* stream);
+
+/* srg_nouns_loss / srg_verb_loss / srg_*_loss_backward with options (opts nullable = those calls). */
+int srg_nouns_loss_ex(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_nouns, int B,
+                      const float* counts, float* loss, float* dlogits, float grad_scale, const float* stats,
+                      const srg_loss_opts* opts, void* stream);
+int srg_verb_loss_ex(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_verb, int B, float inv_batch,
+                     const float* batch_total, float* loss, float* dlogits, float grad_scale, const float* stats,
+                     const srg_loss_opts* opts, void* stream);
+int srg_nouns_loss_backward_ex(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_nouns, int B,
+                               const float* counts, const float* grad_out, float grad_scale, float* dlogits,
+                               void* dlogits_bf16, int accumulate, const float* stats, const srg_loss_opts* opts,
+                               void* stream);
+int srg_verb_loss_backward_ex(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_verb, int B,
+                              float inv_batch, const float* batch_total, const float* grad_out, float grad_scale,
+                              float* dlogits, void* dlogits_bf16, int accumulate, const float* stats,
+                              const srg_loss_opts* opts, void* stream);
+
 /* `stats` (nullable) of the two loss calls: the per-column-tile (row max, row sum-exp) pairs the classifier GEMM of the
  * matching forward call left in its workspace, at this byte offset; with them the loss reads each logits row once
  * instead of three times.  They are only valid for the logits that forward call produced. */

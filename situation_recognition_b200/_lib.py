@@ -26,6 +26,14 @@ class SrgGrads(_c.Structure):
     _fields_ = [(n, _vp) for n in _PARAM_FIELDS + ["role_emb", "verb_emb"]]
 
 
+SRG_REDUCTION = {"mean": 0, "sum": 1, "none": 2}
+
+
+class SrgLossOpts(_c.Structure):
+    _fields_ = [("class_weight", _vp), ("label_smoothing", _f), ("reduction", _i), ("per_target_loss", _vp),
+                ("grad_per_target", _vp)]
+
+
 # name -> (restype, argtypes); mirrors include/srggnn.h one to one
 SIGNATURES = {
     "srg_last_error": (_c.c_char_p, []),
@@ -54,6 +62,14 @@ SIGNATURES = {
     "srg_verb_loss": (_i, [_vp, _vp, _i64, _vp, _i, _f, _vp, _vp, _vp, _f, _vp, _vp]),
     "srg_nouns_loss_backward": (_i, [_vp, _vp, _i64, _vp, _i, _vp, _vp, _f, _vp, _vp, _i, _vp, _vp]),
     "srg_verb_loss_backward": (_i, [_vp, _vp, _i64, _vp, _i, _f, _vp, _vp, _f, _vp, _vp, _i, _vp, _vp]),
+    "srg_count_targets_weighted": (_i, [_vp, _vp, _i, _vp, _vp, _vp]),
+    "srg_verb_weight_total": (_i, [_vp, _vp, _i, _vp, _vp, _vp]),
+    "srg_nouns_loss_ex": (_i, [_vp, _vp, _i64, _vp, _i, _vp, _vp, _vp, _f, _vp, _c.POINTER(SrgLossOpts), _vp]),
+    "srg_verb_loss_ex": (_i, [_vp, _vp, _i64, _vp, _i, _f, _vp, _vp, _vp, _f, _vp, _c.POINTER(SrgLossOpts), _vp]),
+    "srg_nouns_loss_backward_ex": (_i, [_vp, _vp, _i64, _vp, _i, _vp, _vp, _f, _vp, _vp, _i, _vp,
+                                        _c.POINTER(SrgLossOpts), _vp]),
+    "srg_verb_loss_backward_ex": (_i, [_vp, _vp, _i64, _vp, _i, _f, _vp, _vp, _f, _vp, _vp, _i, _vp,
+                                       _c.POINTER(SrgLossOpts), _vp]),
     "srg_workspace_stats_offset": (_sz, [_vp, _i, _i, _i, _i, _vp]),
     "srg_workspace_dlogits_offset": (_sz, [_vp, _i, _i, _vp]),
     "srg_nouns_backward": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _i, _vp, _vp, _vp, _f, _vp, _i64, _c.POINTER(SrgGrads),

@@ -1049,51 +1049,133 @@ int srg_count_targets(srg_handle* h, const int64_t* gt_nouns, int B, float* coun
   return launch_count_targets(gt_nouns, B, h->R, h->L, counts, static_cast<cudaStream_t>(stream));
 }
 
+int srg_count_targets_weighted(srg_handle* h, const int64_t* gt_nouns, int B, const float* class_weight, float* counts,
+                               void* stream) {
+  SRG_CHECK(h != nullptr, "srg_count_targets_weighted: null handle");
+  DeviceGuard guard_(h->device);
+  SRG_CHECK(gt_nouns && counts, "srg_count_targets_weighted: null argument");
+  SRG_CHECK(B >= 0, "srg_count_targets_weighted: B = %d", B);
+  return launch_weighted_count(gt_nouns, static_cast<int64_t>(B) * 3 * h->R, h->R, 3, h->L, class_weight, h->L,
+                               counts, static_cast<cudaStream_t>(stream));
+}
+
+int srg_verb_weight_total(srg_handle* h, const int64_t* gt_verb, int B, const float* class_weight, float* total,
+                          void* stream) {
+  SRG_CHECK(h != nullptr, "srg_verb_weight_total: null handle");
+  DeviceGuard guard_(h->device);
+  SRG_CHECK(gt_verb && total, "srg_verb_weight_total: null argument");
+  SRG_CHECK(B >= 0, "srg_verb_weight_total: B = %d", B);
+  return launch_weighted_count(gt_verb, B, 1, 1, -100, class_weight, h->V, total, static_cast<cudaStream_t>(stream));
+}
+
+// srg_loss_opts -> CeOpts, refusing what the kernels cannot honour.  NULL = the default options.  fwd: the call writes
+// a loss (and, for "none", needs per_target_loss); grad: it writes a gradient (for "none", needs grad_per_target).
+static int loss_opts(const char* fn, const srg_loss_opts* o, bool fwd, bool grad, CeOpts* out) {
+  *out = CeOpts{};
+  if (o == nullptr) return SRG_OK;
+  SRG_CHECK(o->label_smoothing >= 0.f && o->label_smoothing <= 1.f, "%s: label_smoothing %g outside [0, 1]", fn,
+            static_cast<double>(o->label_smoothing));
+  SRG_CHECK(o->reduction == SRG_REDUCTION_MEAN || o->reduction == SRG_REDUCTION_SUM ||
+            o->reduction == SRG_REDUCTION_NONE, "%s: unknown reduction %d", fn, o->reduction);
+  if (o->reduction == SRG_REDUCTION_NONE) {
+    SRG_CHECK(!fwd || o->per_target_loss != nullptr, "%s: reduction 'none' needs per_target_loss", fn);
+    SRG_CHECK(!grad || o->grad_per_target != nullptr, "%s: reduction 'none' needs grad_per_target", fn);
+  }
+  out->cw = o->class_weight;
+  out->eps = o->label_smoothing;
+  out->reduction = o->reduction;
+  out->per_target = fwd ? o->per_target_loss : nullptr;
+  out->gpt = grad ? o->grad_per_target : nullptr;
+  return SRG_OK;
+}
+
+static bool mean_reduction(const srg_loss_opts* o) { return o == nullptr || o->reduction == SRG_REDUCTION_MEAN; }
+
+int srg_nouns_loss_ex(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_nouns, int B,
+                      const float* counts, float* loss, float* dlogits, float grad_scale, const float* stats,
+                      const srg_loss_opts* opts, void* stream) {
+  CeOpts o;
+  SRG_TRY(loss_opts("srg_nouns_loss", opts, true, dlogits != nullptr, &o));
+  SRG_CHECK(h != nullptr, "srg_nouns_loss: null handle");
+  DeviceGuard guard_(h->device);
+  const bool none = !mean_reduction(opts) && opts->reduction == SRG_REDUCTION_NONE;
+  SRG_CHECK(logits && gt_nouns && (counts || !mean_reduction(opts)) && (loss || none), "srg_nouns_loss: null argument");
+  SRG_CHECK(ldl >= h->L, "srg_nouns_loss: ldl %lld < n_labels %d", (long long)ldl, h->L);
+  return launch_nouns_ce(logits, ldl, h->L, gt_nouns, B, h->R, counts, loss, dlogits, grad_scale, nullptr, stats,
+                         h->Lpad / ((h->cg == 2) ? 256 : 128), nullptr, 0, 0, &o, static_cast<cudaStream_t>(stream));
+}
+
 int srg_nouns_loss(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_nouns, int B,
                    const float* counts, float* loss, float* dlogits, float grad_scale, const float* stats,
                    void* stream) {
-  SRG_CHECK(h != nullptr, "srg_nouns_loss: null handle");
+  return srg_nouns_loss_ex(h, logits, ldl, gt_nouns, B, counts, loss, dlogits, grad_scale, stats, nullptr, stream);
+}
+
+int srg_nouns_loss_backward_ex(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_nouns, int B,
+                               const float* counts, const float* grad_out, float grad_scale, float* dlogits,
+                               void* dlogits_bf16, int accumulate, const float* stats, const srg_loss_opts* opts,
+                               void* stream) {
+  CeOpts o;
+  SRG_TRY(loss_opts("srg_nouns_loss_backward", opts, false, true, &o));
+  SRG_CHECK(h != nullptr, "srg_nouns_loss_backward: null handle");
   DeviceGuard guard_(h->device);
-  SRG_CHECK(h && logits && gt_nouns && counts && loss, "srg_nouns_loss: null argument");
-  SRG_CHECK(ldl >= h->L, "srg_nouns_loss: ldl %lld < n_labels %d", (long long)ldl, h->L);
-  return launch_nouns_ce(logits, ldl, h->L, gt_nouns, B, h->R, counts, loss, dlogits, grad_scale, nullptr, stats,
-                         h->Lpad / ((h->cg == 2) ? 256 : 128), nullptr, 0, 0, static_cast<cudaStream_t>(stream));
+  SRG_CHECK(logits && gt_nouns && (counts || !mean_reduction(opts)) && (dlogits || dlogits_bf16),
+            "srg_nouns_loss_backward: null argument");
+  SRG_CHECK(ldl >= h->L, "srg_nouns_loss_backward: ldl %lld < n_labels %d", (long long)ldl, h->L);
+  return launch_nouns_ce(logits, ldl, h->L, gt_nouns, B, h->R, counts, nullptr, dlogits, grad_scale, grad_out, stats,
+                         h->Lpad / ((h->cg == 2) ? 256 : 128), static_cast<bf16*>(dlogits_bf16), h->Lpad, accumulate,
+                         &o, static_cast<cudaStream_t>(stream));
 }
 
 int srg_nouns_loss_backward(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_nouns, int B,
                             const float* counts, const float* grad_out, float grad_scale, float* dlogits,
                             void* dlogits_bf16, int accumulate, const float* stats, void* stream) {
-  SRG_CHECK(h != nullptr, "srg_nouns_loss_backward: null handle");
+  return srg_nouns_loss_backward_ex(h, logits, ldl, gt_nouns, B, counts, grad_out, grad_scale, dlogits, dlogits_bf16,
+                                    accumulate, stats, nullptr, stream);
+}
+
+int srg_verb_loss_ex(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_verb, int B, float inv_batch,
+                     const float* batch_total, float* loss, float* dlogits, float grad_scale, const float* stats,
+                     const srg_loss_opts* opts, void* stream) {
+  CeOpts o;
+  SRG_TRY(loss_opts("srg_verb_loss", opts, true, dlogits != nullptr, &o));
+  SRG_CHECK(h != nullptr, "srg_verb_loss: null handle");
   DeviceGuard guard_(h->device);
-  SRG_CHECK(h && logits && gt_nouns && counts && (dlogits || dlogits_bf16), "srg_nouns_loss_backward: null argument");
-  SRG_CHECK(ldl >= h->L, "srg_nouns_loss_backward: ldl %lld < n_labels %d", (long long)ldl, h->L);
-  return launch_nouns_ce(logits, ldl, h->L, gt_nouns, B, h->R, counts, nullptr, dlogits, grad_scale, grad_out, stats,
-                         h->Lpad / ((h->cg == 2) ? 256 : 128), static_cast<bf16*>(dlogits_bf16), h->Lpad, accumulate,
-                         static_cast<cudaStream_t>(stream));
+  const bool none = !mean_reduction(opts) && opts->reduction == SRG_REDUCTION_NONE;
+  SRG_CHECK(logits && gt_verb && (loss || none), "srg_verb_loss: null argument");
+  SRG_CHECK(ldl >= h->V, "srg_verb_loss: ldl %lld < n_verbs %d", (long long)ldl, h->V);
+  return launch_verb_ce(logits, ldl, h->V, gt_verb, B, inv_batch, loss, dlogits, grad_scale, nullptr, stats,
+                        h->Vpad / ((h->cg == 2) ? 256 : 128), batch_total, nullptr, 0, 0, &o,
+                        static_cast<cudaStream_t>(stream));
 }
 
 int srg_verb_loss(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_verb, int B, float inv_batch,
                   const float* batch_total, float* loss, float* dlogits, float grad_scale, const float* stats,
                   void* stream) {
-  SRG_CHECK(h != nullptr, "srg_verb_loss: null handle");
+  return srg_verb_loss_ex(h, logits, ldl, gt_verb, B, inv_batch, batch_total, loss, dlogits, grad_scale, stats,
+                          nullptr, stream);
+}
+
+int srg_verb_loss_backward_ex(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_verb, int B,
+                              float inv_batch, const float* batch_total, const float* grad_out, float grad_scale,
+                              float* dlogits, void* dlogits_bf16, int accumulate, const float* stats,
+                              const srg_loss_opts* opts, void* stream) {
+  CeOpts o;
+  SRG_TRY(loss_opts("srg_verb_loss_backward", opts, false, true, &o));
+  SRG_CHECK(h != nullptr, "srg_verb_loss_backward: null handle");
   DeviceGuard guard_(h->device);
-  SRG_CHECK(h && logits && gt_verb && loss, "srg_verb_loss: null argument");
-  SRG_CHECK(ldl >= h->V, "srg_verb_loss: ldl %lld < n_verbs %d", (long long)ldl, h->V);
-  return launch_verb_ce(logits, ldl, h->V, gt_verb, B, inv_batch, loss, dlogits, grad_scale, nullptr, stats,
-                        h->Vpad / ((h->cg == 2) ? 256 : 128), batch_total, nullptr, 0, 0,
-                        static_cast<cudaStream_t>(stream));
+  SRG_CHECK(logits && gt_verb && (dlogits || dlogits_bf16), "srg_verb_loss_backward: null argument");
+  SRG_CHECK(ldl >= h->V, "srg_verb_loss_backward: ldl %lld < n_verbs %d", (long long)ldl, h->V);
+  return launch_verb_ce(logits, ldl, h->V, gt_verb, B, inv_batch, nullptr, dlogits, grad_scale, grad_out, stats,
+                        h->Vpad / ((h->cg == 2) ? 256 : 128), batch_total, static_cast<bf16*>(dlogits_bf16), h->Vpad,
+                        accumulate, &o, static_cast<cudaStream_t>(stream));
 }
 
 int srg_verb_loss_backward(srg_handle* h, const float* logits, int64_t ldl, const int64_t* gt_verb, int B,
                            float inv_batch, const float* batch_total, const float* grad_out, float grad_scale,
                            float* dlogits, void* dlogits_bf16, int accumulate, const float* stats, void* stream) {
-  SRG_CHECK(h != nullptr, "srg_verb_loss_backward: null handle");
-  DeviceGuard guard_(h->device);
-  SRG_CHECK(h && logits && gt_verb && (dlogits || dlogits_bf16), "srg_verb_loss_backward: null argument");
-  SRG_CHECK(ldl >= h->V, "srg_verb_loss_backward: ldl %lld < n_verbs %d", (long long)ldl, h->V);
-  return launch_verb_ce(logits, ldl, h->V, gt_verb, B, inv_batch, nullptr, dlogits, grad_scale, grad_out, stats,
-                        h->Vpad / ((h->cg == 2) ? 256 : 128), batch_total, static_cast<bf16*>(dlogits_bf16), h->Vpad,
-                        accumulate, static_cast<cudaStream_t>(stream));
+  return srg_verb_loss_backward_ex(h, logits, ldl, gt_verb, B, inv_batch, batch_total, grad_out, grad_scale, dlogits,
+                                   dlogits_bf16, accumulate, stats, nullptr, stream);
 }
 
 int srg_clip_adamax(float* params, float* grads, float* exp_avg, float* exp_inf, int64_t n, float lr, float beta1,

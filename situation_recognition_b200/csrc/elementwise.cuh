@@ -101,16 +101,41 @@ int launch_pack_weight_multi(const PackJob* jobs, int n_jobs, int cols, cudaStre
 int launch_pack_bias(const float* a, const float* b, int n, int n_pad, float* dst, cudaStream_t s);
 
 int launch_count_targets(const int64_t* gt, int B, int R, int ignore_index, float* counts, cudaStream_t s);
+// out[a] = sum of cw[gt[t]] over the targets t of annotation a = (t / R) % n_ann with gt[t] != ignore_index
+// (targets outside [0, n_classes) count 0), n targets in all; overwritten.  One CTA in a fixed order, no atomics:
+// repeated calls are bit-identical.  n_ann <= 3.
+int launch_weighted_count(const int64_t* gt, int64_t n, int R, int n_ann, int ignore_index, const float* cw,
+                          int n_classes, float* out, cudaStream_t s);
+
+// Options of the cross-entropy kernels (srg_loss_opts).  With none of them given the kernels run the default-option
+// instantiation, launch for launch.
+enum { kCeMean = 0, kCeSum = 1, kCeNone = 2 };
+struct CeOpts {
+  const float* cw;          // class weights [n_classes] or null (all 1)
+  float eps;                // label smoothing in [0, 1]
+  int reduction;            // kCeMean / kCeSum / kCeNone
+  float* per_target;        // forward: kCeNone: the loss of every target; mean / sum: its term of the scalar, which
+                            // is then their sum in a fixed order
+  const float* gpt;         // kCeNone gradient: d(loss)/d(per-target loss), laid out like the targets
+};
+inline bool ce_opts_active(const CeOpts* o) {
+  return o != nullptr && (o->cw != nullptr || o->eps > 0.f || o->reduction != kCeMean || o->per_target != nullptr);
+}
+
 // one warp per logits row; loss and dlogits are both optional; the gradient is scaled by grad_scale and, when
 // gscale_dev is not null, by that device scalar as well
 // dlb (nullable, instead of dlogits): the gradient as the zero-padded bf16 [rows, n_pad] operand of the classifier's
 // backward GEMMs; accumulate: added to what dlb already holds
+// opt (nullable): class weights, label smoothing and the reduction; the option arithmetic is only compiled into the
+// instantiation that ce_opts_active(opt) selects.  Mean: counts[a] / *batch_total are the weighted denominators.
 int launch_nouns_ce(const float* logits, int64_t ldl, int n_labels, const int64_t* gt, int B, int R,
                     const float* counts, float* loss, float* dlogits, float grad_scale, const float* gscale_dev,
-                    const float* stats, int stats_tiles, bf16* dlb, int n_pad, int accumulate, cudaStream_t s);
+                    const float* stats, int stats_tiles, bf16* dlb, int n_pad, int accumulate, const CeOpts* opt,
+                    cudaStream_t s);
 int launch_verb_ce(const float* logits, int64_t ldl, int n_verbs, const int64_t* gt, int B, float inv_batch,
                    float* loss, float* dlogits, float grad_scale, const float* gscale_dev, const float* stats,
-                   int stats_tiles, const float* batch_total, bf16* dlb, int n_pad, int accumulate, cudaStream_t s);
+                   int stats_tiles, const float* batch_total, bf16* dlb, int n_pad, int accumulate, const CeOpts* opt,
+                   cudaStream_t s);
 // Per row of x [rows, ldl]: the k largest of the first n columns in descending order (ties: lower column first, as
 // torch.argmax) and their log-softmax over those n columns.  Columns >= n are never read.  1 <= k <= 16, k <= n.
 // idx int64 [rows, k], logp fp32 [rows, k].

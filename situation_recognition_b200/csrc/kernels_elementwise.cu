@@ -493,47 +493,144 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// Sums of one CTA in a fixed order (strided per thread, then a fixed tree): bit-identical on every call.
+template <int NA>
+__device__ __forceinline__ void block_sum_fixed(float (&v)[NA], float* __restrict__ out, int n_out, bool add) {
+  __shared__ float sh[NA][kThreads];
+#pragma unroll
+  for (int a = 0; a < NA; ++a) sh[a][threadIdx.x] = v[a];
+  __syncthreads();
+  for (int o = kThreads / 2; o > 0; o >>= 1) {
+    if (threadIdx.x < o) {
+#pragma unroll
+      for (int a = 0; a < NA; ++a) sh[a][threadIdx.x] += sh[a][threadIdx.x + o];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x < n_out) out[threadIdx.x] = (add ? out[threadIdx.x] : 0.f) + sh[threadIdx.x][0];
+}
+
+__global__ void k_weighted_count(const int64_t* __restrict__ gt, int64_t n, int R, int n_ann, int ignore_index,
+                                 const float* __restrict__ cw, int n_classes, float* __restrict__ out) {
+  float local[3] = {0.f, 0.f, 0.f};
+  for (int64_t t = threadIdx.x; t < n; t += kThreads) {
+    const int64_t y = gt[t];
+    if (y == ignore_index || y < 0 || y >= n_classes) continue;
+    const float w = cw != nullptr ? __ldg(cw + y) : 1.f;
+    const int a = static_cast<int>((t / R) % n_ann);
+    local[0] += a == 0 ? w : 0.f;
+    local[1] += a == 1 ? w : 0.f;
+    local[2] += a == 2 ? w : 0.f;
+  }
+  block_sum_fixed<3>(local, out, n_ann, false);
+}
+
+__global__ void k_sum_fixed(const float* __restrict__ x, int64_t n, float* __restrict__ out) {
+  float local[1] = {0.f};
+  for (int64_t t = threadIdx.x; t < n; t += kThreads) local[0] += x[t];
+  block_sum_fixed<1>(local, out, 1, true);
+}
+
 // One warp per row.  NT = number of targets per row (3 for nouns, 1 for verbs).
 //   loss += sum_a w_a * (lse - logit[t_a]);   dlogits[c] = gs * (sum_a w_a * (p_c - [c == t_a]))
-template <int NT>
+// OPT (CeOpts, torch's definition): with class weights cw (W = sum_c cw_c), smoothing eps and C classes the loss of a
+// target y is  l = (1 - eps) cw_y (lse - z_y) + (eps / C) sum_c cw_c (lse - z_c)  and its gradient
+//   dl/dz_c = (1 - eps) cw_y (p_c - [c == y]) + (eps / C) (W p_c - cw_c),
+// times the target's scale s_a: 1 / (its annotation's sum of cw_y) for the mean (0 when that sum is 0), 1 for the sum,
+// the upstream per-target gradient for none; 0 for an ignored target.
+template <int NT, bool OPT>
 __global__ void k_cross_entropy(const float* __restrict__ logits, int64_t ldl, int n_classes, int rows,
                                 const int64_t* __restrict__ gt, int R, int ignore_index,
                                 const float* __restrict__ counts, float inv_fixed, float* __restrict__ loss,
                                 float* __restrict__ dlogits, float grad_scale, const float* __restrict__ gscale_dev,
                                 const float2* __restrict__ stats, int stats_tiles,
                                 const float* __restrict__ total_dev, bf16* __restrict__ dlb, int64_t ld_b, int n_pad,
-                                int accumulate) {
+                                int accumulate, CeOpts opt) {
   // dlb (nullable): the gradient goes out as the zero-padded bf16 [rows, n_pad] operand of the classifier's backward
   // GEMMs instead of (not in addition to) the fp32 dlogits -- the fp32 gradient is then never written or re-read
   // (accumulate: add to what dlb holds, for a second loss on the same logits)
   __shared__ float s_loss[kThreads / 32];
   // total_dev: device scalar holding the GLOBAL number of rows the mean is taken over (all-reduced by the caller when
-  // the batch is sharded unevenly); overrides inv_fixed
-  if (total_dev != nullptr) inv_fixed = 1.0f / fmaxf(__ldg(total_dev), 1.0f);
+  // the batch is sharded unevenly); overrides inv_fixed.  With options it is the weighted sum, which may lie in (0, 1)
+  if (total_dev != nullptr) {
+    const float t = __ldg(total_dev);
+    inv_fixed = OPT ? (t > 0.f ? 1.0f / t : 0.f) : 1.0f / fmaxf(t, 1.0f);
+  }
   // gscale_dev: device scalar multiplied into the gradient (the incoming d(loss) of the autograd backward pass)
   if (gscale_dev != nullptr) grad_scale *= __ldg(gscale_dev);
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int warps_per_block = blockDim.x >> 5;
+  const bool want_grad = dlogits != nullptr || dlb != nullptr;
+  const bool fwd = loss != nullptr || (OPT && opt.per_target != nullptr);      // a loss is written
+  float wtot = static_cast<float>(n_classes), eps_c = 0.f;     // W and eps / C
+  if constexpr (OPT) {
+    eps_c = opt.eps / static_cast<float>(n_classes);
+    if (opt.cw != nullptr && opt.eps > 0.f) {
+      __shared__ float s_wtot;
+      if (wib == 0) {
+        float t = 0.f;
+        for (int c = lane; c < n_classes; c += 32) t += __ldg(opt.cw + c);
+        t = warp_sum(t);
+        if (lane == 0) s_wtot = t;
+      }
+      __syncthreads();
+      wtot = s_wtot;
+    }
+  }
   float my_loss = 0.f;
   for (int row = blockIdx.x * warps_per_block + wib; row < rows; row += gridDim.x * warps_per_block) {
     const float* lr = logits + static_cast<int64_t>(row) * ldl;
     int64_t tgt[NT];
     float w[NT];
     float wsum = 0.f;
+    // OPT: the target's index in gt (and in per_target / gpt), its weight cw_y, its scale s_a; the gradient's
+    // uniform term ecoef * cw_c
+    int64_t tix[NT];
+    float wy[NT], sa[NT];
+    float ecoef = 0.f;
+    bool any = false;
 #pragma unroll
     for (int a = 0; a < NT; ++a) {
       if (NT == 3) {
         const int b = row / R, r = row % R;
-        tgt[a] = gt[(static_cast<int64_t>(b) * 3 + a) * R + r];
-        w[a] = (tgt[a] != ignore_index) ? 1.0f / counts[a] : 0.f;
+        tix[a] = (static_cast<int64_t>(b) * 3 + a) * R + r;
       } else {
-        tgt[a] = gt[row];
-        w[a] = inv_fixed;
+        tix[a] = row;
       }
-      wsum += w[a];
+      tgt[a] = gt[tix[a]];
+      if constexpr (OPT) {
+        const bool valid = NT != 3 || tgt[a] != ignore_index;
+        any |= valid;
+        wy[a] = valid ? (opt.cw != nullptr ? __ldg(opt.cw + tgt[a]) : 1.f) : 0.f;
+        float s = 0.f;
+        if (valid) {
+          if (opt.reduction == kCeNone) s = opt.gpt != nullptr ? opt.gpt[tix[a]] : 0.f;
+          else if (opt.reduction == kCeSum) s = 1.f;
+          else if (NT == 3) s = counts[a] > 0.f ? 1.0f / counts[a] : 0.f;
+          else s = inv_fixed;
+        }
+        sa[a] = s;
+        w[a] = s * (1.f - opt.eps) * wy[a];              // coefficient of -[c == y] in the gradient
+        wsum += s * ((1.f - opt.eps) * wy[a] + eps_c * wtot);   // coefficient of p_c
+        ecoef += s * eps_c;                                // coefficient of -cw_c
+      } else {
+        if (NT == 3) w[a] = (tgt[a] != ignore_index) ? 1.0f / counts[a] : 0.f;
+        else w[a] = inv_fixed;
+        wsum += w[a];
+      }
     }
-    if (wsum == 0.f && dlogits == nullptr && dlb == nullptr) continue;  // fully ignored row contributes nothing
-    float mx = -INFINITY, se = 0.f;
+    if constexpr (OPT) {
+      if (!any && !want_grad) {          // every target ignored: its per-target losses are 0
+        if (lane == 0 && opt.per_target != nullptr)
+#pragma unroll
+          for (int a = 0; a < NT; ++a) opt.per_target[tix[a]] = 0.f;
+        continue;
+      }
+    } else {
+      if (wsum == 0.f && !want_grad) continue;  // fully ignored row contributes nothing
+    }
+    float mx = -INFINITY, se = 0.f, swd = 0.f;   // swd (OPT, eps > 0): sum_c cw_c (mx - z_c)
+    const bool need_swd = OPT && opt.eps > 0.f && fwd;
     if (stats != nullptr) {
       // the classifier GEMM already reduced every 128/256-column tile of this row to (max, sum exp(x - max)):
       // combine the per-tile pairs instead of reading the logits row two more times
@@ -541,18 +638,52 @@ __global__ void k_cross_entropy(const float* __restrict__ logits, int64_t ldl, i
       if (lane < stats_tiles) st = stats[static_cast<int64_t>(row) * stats_tiles + lane];
       mx = warp_max(st.x);
       se = warp_sum(st.y > 0.f ? st.y * __expf(st.x - mx) : 0.f);
+      if constexpr (OPT) {
+        if (need_swd) {                   // the smoothing term needs the whole row: one pass
+          for (int c = lane; c < n_classes; c += 32)
+            swd += (opt.cw != nullptr ? __ldg(opt.cw + c) : 1.f) * (mx - lr[c]);
+          swd = warp_sum(swd);
+        }
+      }
     } else {
       for (int c = lane; c < n_classes; c += 32) mx = fmaxf(mx, lr[c]);
       mx = warp_max(mx);
-      for (int c = lane; c < n_classes; c += 32) se += __expf(lr[c] - mx);
+      if constexpr (OPT) {
+        for (int c = lane; c < n_classes; c += 32) {
+          const float x = lr[c];
+          se += __expf(x - mx);
+          if (need_swd) swd += (opt.cw != nullptr ? __ldg(opt.cw + c) : 1.f) * (mx - x);
+        }
+        swd = warp_sum(swd);
+      } else {
+        for (int c = lane; c < n_classes; c += 32) se += __expf(lr[c] - mx);
+      }
       se = warp_sum(se);
     }
     const float lse = mx + __logf(se);
     if (lane == 0) {
+      if constexpr (OPT) {
+        if (fwd) {
+          // sum_c cw_c (lse - z_c) = sum_c cw_c (mx - z_c) + W log(se): no cancellation between large terms
+          const float smooth = opt.eps > 0.f ? eps_c * (swd + wtot * __logf(se)) : 0.f;
 #pragma unroll
-      for (int a = 0; a < NT; ++a)
-        if (w[a] != 0.f) my_loss += w[a] * (lse - lr[tgt[a]]);
+          for (int a = 0; a < NT; ++a) {
+            const bool valid = NT != 3 || tgt[a] != ignore_index;
+            const float l = valid ? (1.f - opt.eps) * wy[a] * (lse - lr[tgt[a]]) + smooth : 0.f;
+            const float term = opt.reduction == kCeNone ? l : sa[a] * l;    // (none: sa is the gradient's)
+            if (opt.per_target != nullptr) opt.per_target[tix[a]] = term;
+            my_loss += opt.reduction == kCeNone ? 0.f : term;
+          }
+        }
+      } else {
+#pragma unroll
+        for (int a = 0; a < NT; ++a)
+          if (w[a] != 0.f) my_loss += w[a] * (lse - lr[tgt[a]]);
+      }
     }
+    // the gradient's uniform term: grad_scale * ecoef * cw_c (OPT, eps > 0)
+    const float eg = ecoef * grad_scale;
+    const bool grad_row = OPT ? (wsum != 0.f || ecoef != 0.f) : (wsum != 0.f);
     if (dlb != nullptr) {
       bf16* br = dlb + static_cast<int64_t>(row) * ld_b;
       const float inv_se = 1.0f / se;
@@ -560,7 +691,7 @@ __global__ void k_cross_entropy(const float* __restrict__ logits, int64_t ldl, i
       // n_pad is a multiple of 128 here (the classifier pads to 256 columns); logits rows are 16-byte aligned
       for (int c = lane * 4; c < n_pad; c += 128) {
         float g[4] = {0.f, 0.f, 0.f, 0.f};
-        if (c < n_classes && wsum != 0.f) {
+        if (c < n_classes && grad_row) {
           float x[4];
           if (c + 4 <= ldl && ((reinterpret_cast<uintptr_t>(lr) & 15) == 0) && (ldl & 3) == 0) {
             const float4 v = *reinterpret_cast<const float4*>(lr + c);
@@ -576,6 +707,7 @@ __global__ void k_cross_entropy(const float* __restrict__ logits, int64_t ldl, i
 #pragma unroll
               for (int a = 0; a < NT; ++a)
                 if (w[a] != 0.f && tgt[a] == c + k) v -= w[a] * grad_scale;
+              if constexpr (OPT) v -= eg * (opt.cw != nullptr ? __ldg(opt.cw + c + k) : 1.f);
               g[k] = v;
             }
           }
@@ -600,11 +732,12 @@ __global__ void k_cross_entropy(const float* __restrict__ logits, int64_t ldl, i
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
             float v = 0.f;
-            if (c + k < n_classes && wsum != 0.f) {
+            if (c + k < n_classes && grad_row) {
               v = ws * __expf(g[k] - mx) * inv_se;
 #pragma unroll
               for (int a = 0; a < NT; ++a)
                 if (w[a] != 0.f && tgt[a] == c + k) v -= w[a] * grad_scale;
+              if constexpr (OPT) v -= eg * (opt.cw != nullptr ? __ldg(opt.cw + c + k) : 1.f);
             }
             g[k] = v;
           }
@@ -613,11 +746,12 @@ __global__ void k_cross_entropy(const float* __restrict__ logits, int64_t ldl, i
       } else {
         for (int c = lane; c < ldl; c += 32) {
           float g = 0.f;
-          if (c < n_classes && wsum != 0.f) {
+          if (c < n_classes && grad_row) {
             g = ws * __expf(lr[c] - mx) * inv_se;
 #pragma unroll
             for (int a = 0; a < NT; ++a)
               if (w[a] != 0.f && tgt[a] == c) g -= w[a] * grad_scale;
+            if constexpr (OPT) g -= eg * (opt.cw != nullptr ? __ldg(opt.cw + c) : 1.f);
           }
           dr[c] = g;
         }
@@ -629,7 +763,8 @@ __global__ void k_cross_entropy(const float* __restrict__ logits, int64_t ldl, i
   if (threadIdx.x == 0) {
     float t = 0.f;
     for (int i = 0; i < warps_per_block; ++i) t += s_loss[i];
-    if (t != 0.f && loss != nullptr) atomicAdd(loss, t);
+    // OPT with per_target: the scalar is their fixed-order sum (k_sum_fixed), not these per-CTA atomics
+    if (t != 0.f && loss != nullptr && !(OPT && opt.per_target != nullptr)) atomicAdd(loss, t);
   }
 }
 
@@ -1546,35 +1681,65 @@ int launch_count_targets(const int64_t* gt, int B, int R, int ignore_index, floa
   return SRG_OK;
 }
 
+int launch_weighted_count(const int64_t* gt, int64_t n, int R, int n_ann, int ignore_index, const float* cw,
+                          int n_classes, float* out, cudaStream_t s) {
+  if (n_ann < 1 || n_ann > 3 || R < 1) return set_error(SRG_ERR_ARG, "weighted_count: bad shape");
+  k_weighted_count<<<1, kThreads, 0, s>>>(gt, n, R, n_ann, ignore_index, cw, n_classes, out);
+  SRG_LAUNCH_CHECK();
+  return SRG_OK;
+}
+
+// the default-option or the option instantiation of k_cross_entropy, then (options, mean / sum with per-target
+// terms) their fixed-order sum into *loss
+template <int NT>
+static int launch_ce(int blocks, const float* logits, int64_t ldl, int n_classes, int rows, const int64_t* gt, int R,
+                     int ignore_index, const float* counts, float inv_fixed, float* loss, float* dlogits,
+                     float grad_scale, const float* gscale_dev, const float2* stats, int stats_tiles,
+                     const float* total_dev, bf16* dlb, int n_pad, int accumulate, const CeOpts* opt, cudaStream_t s) {
+  if (!ce_opts_active(opt)) {
+    k_cross_entropy<NT, false><<<blocks, kThreads, 0, s>>>(logits, ldl, n_classes, rows, gt, R, ignore_index, counts,
+                                                           inv_fixed, loss, dlogits, grad_scale, gscale_dev, stats,
+                                                           stats_tiles, total_dev, dlb, n_pad, n_pad, accumulate,
+                                                           CeOpts{});
+    SRG_LAUNCH_CHECK();
+    return SRG_OK;
+  }
+  k_cross_entropy<NT, true><<<blocks, kThreads, 0, s>>>(logits, ldl, n_classes, rows, gt, R, ignore_index, counts,
+                                                        inv_fixed, loss, dlogits, grad_scale, gscale_dev, stats,
+                                                        stats_tiles, total_dev, dlb, n_pad, n_pad, accumulate, *opt);
+  SRG_LAUNCH_CHECK();
+  if (loss != nullptr && opt->per_target != nullptr && opt->reduction != kCeNone) {
+    k_sum_fixed<<<1, kThreads, 0, s>>>(opt->per_target, static_cast<int64_t>(rows) * NT, loss);
+    SRG_LAUNCH_CHECK();
+  }
+  return SRG_OK;
+}
+
 int launch_nouns_ce(const float* logits, int64_t ldl, int n_labels, const int64_t* gt, int B, int R,
                     const float* counts, float* loss, float* dlogits, float grad_scale, const float* gscale_dev,
-                    const float* stats, int stats_tiles, bf16* dlb, int n_pad, int accumulate, cudaStream_t s) {
+                    const float* stats, int stats_tiles, bf16* dlb, int n_pad, int accumulate, const CeOpts* opt,
+                    cudaStream_t s) {
   const int rows = B * R;
   if (rows <= 0) return SRG_OK;
   int blocks = (rows + 7) / 8;
   if (blocks > 148 * 8) blocks = 148 * 8;
   if (stats_tiles > 32) stats = nullptr;
-  k_cross_entropy<3><<<blocks, kThreads, 0, s>>>(logits, ldl, n_labels, rows, gt, R, n_labels, counts, 0.f, loss,
-                                                dlogits, grad_scale, gscale_dev,
-                                                reinterpret_cast<const float2*>(stats), stats_tiles, nullptr, dlb, n_pad,
-                                                n_pad, accumulate);
-  SRG_LAUNCH_CHECK();
-  return SRG_OK;
+  return launch_ce<3>(blocks, logits, ldl, n_labels, rows, gt, R, n_labels, counts, 0.f, loss, dlogits, grad_scale,
+                      gscale_dev, reinterpret_cast<const float2*>(stats), stats_tiles, nullptr, dlb, n_pad, accumulate,
+                      opt, s);
 }
 
 int launch_verb_ce(const float* logits, int64_t ldl, int n_verbs, const int64_t* gt, int B, float inv_batch,
                    float* loss, float* dlogits, float grad_scale, const float* gscale_dev, const float* stats,
-                   int stats_tiles, const float* batch_total, bf16* dlb, int n_pad, int accumulate, cudaStream_t s) {
+                   int stats_tiles, const float* batch_total, bf16* dlb, int n_pad, int accumulate, const CeOpts* opt,
+                   cudaStream_t s) {
   if (B <= 0) return SRG_OK;
   int blocks = (B + 7) / 8;
   if (blocks > 148 * 8) blocks = 148 * 8;
   if (stats_tiles > 32) stats = nullptr;
-  k_cross_entropy<1><<<blocks, kThreads, 0, s>>>(logits, ldl, n_verbs, B, gt, 1, -100, nullptr, inv_batch, loss,
-                                                dlogits, grad_scale, gscale_dev,
-                                                reinterpret_cast<const float2*>(stats), stats_tiles, batch_total, dlb,
-                                                n_pad, n_pad, accumulate);
-  SRG_LAUNCH_CHECK();
-  return SRG_OK;
+  return launch_ce<1>(blocks, logits, ldl, n_verbs, B, gt, 1, -100, nullptr, inv_batch, loss, dlogits, grad_scale,
+                      gscale_dev, reinterpret_cast<const float2*>(stats), stats_tiles, batch_total, dlb, n_pad,
+                      accumulate, opt, s);
 }
 
 int launch_row_topk_logsoftmax(const float* x, int64_t ldl, int rows, int n, int k, int64_t* idx, float* logp,

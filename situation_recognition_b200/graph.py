@@ -22,10 +22,17 @@ class GraphedTrainStep:
     `optimizer` must be capturable: parallel.FlatAdamax (fused clip + Adamax kernel) or
     torch.optim.Adamax(..., capturable=True).  Inputs may live on the host
     (pinned) or on the device; they are copied into the graph's static buffers before each replay.
+    verb_loss_kwargs / nouns_loss_kwargs: the training objective's `weight`, `label_smoothing` and `reduction`
+    ("mean" or "sum") of verb_loss and of both nouns_loss calls.  The captured step reads the weight tensors in place.
     """
 
-    def __init__(self, model, optimizer, flat, batch, clip=1.0, warmup=3):
+    def __init__(self, model, optimizer, flat, batch, clip=1.0, warmup=3, verb_loss_kwargs=None,
+                 nouns_loss_kwargs=None):
         self.model, self.opt, self.flat, self.clip = model, optimizer, flat, clip
+        self.verb_kw, self.nouns_kw = dict(verb_loss_kwargs or {}), dict(nouns_loss_kwargs or {})
+        for kw in (self.verb_kw, self.nouns_kw):
+            if kw.get("reduction", "mean") not in ("mean", "sum"):
+                raise ValueError("GraphedTrainStep back-propagates a scalar loss: reduction must be 'mean' or 'sum'")
         dev = next(model.parameters()).device
         enc = model.encoder
         R = enc.get_max_role_count()
@@ -43,9 +50,9 @@ class GraphedTrainStep:
         m = self.model
         self.flat.zero()
         pred_verb, pred_nouns, gt_pred_nouns = m(a, v, img_nouns=b)
-        vl = m.verb_loss(pred_verb, v)
-        nl = m.nouns_loss(pred_nouns, n)
-        gl = m.nouns_loss(gt_pred_nouns, n)
+        vl = m.verb_loss(pred_verb, v, **self.verb_kw)
+        nl = m.nouns_loss(pred_nouns, n, **self.nouns_kw)
+        gl = m.nouns_loss(gt_pred_nouns, n, **self.nouns_kw)
         (vl + nl).backward()
         if getattr(self.opt, "world", 1) <= 1:      # a sharded FlatAdamax reduce-scatters the gradient itself
             self.flat.all_reduce()

@@ -478,88 +478,171 @@ def _rows_view(logits, n):
     return x, rows, ld
 
 
+class _LossOpts:
+    """Validated `weight` / `label_smoothing` / `reduction` of one verb_loss / nouns_loss call (torch's
+    F.cross_entropy keywords), or None from `make` when all three hold their defaults: the loss then runs the
+    default-option kernels, launch for launch.  Everything is checked here, before any engine call."""
+
+    def __init__(self, weight, eps, reduction):
+        self.weight, self.eps, self.reduction = weight, eps, reduction
+        self.red = _lib.SRG_REDUCTION[reduction]
+        # the denominators' cache key: a new weight tensor, or an in-place change of this one, is never stale
+        self.wkey = None if weight is None else (weight.data_ptr(), weight._version)
+
+    @staticmethod
+    def make(weight, label_smoothing, reduction, n_classes, device, what):
+        if reduction not in _lib.SRG_REDUCTION:
+            raise ValueError("%s: reduction must be 'mean', 'sum' or 'none', got %r" % (what, reduction))
+        eps = float(label_smoothing)
+        if not 0.0 <= eps <= 1.0:
+            raise ValueError("%s: label_smoothing must be in [0, 1], got %r" % (what, label_smoothing))
+        if weight is not None:
+            if not isinstance(weight, torch.Tensor):
+                raise _lib.SrgError("%s: weight must be a tensor, got %s" % (what, type(weight).__name__))
+            if weight.requires_grad:
+                raise _lib.SrgError("%s: weight is data and must not require grad (pass weight.detach())" % what)
+            if weight.dim() != 1 or weight.numel() != n_classes:
+                raise _lib.SrgError("%s: weight must have shape [%d], got %s" % (what, n_classes, tuple(weight.shape)))
+            if weight.dtype != torch.float32:
+                raise _lib.SrgError("%s: weight must be float32, got %s" % (what, weight.dtype))
+            if weight.device != device:
+                raise _lib.SrgError("%s: weight is on %s, the logits on %s" % (what, weight.device, device))
+        if weight is None and eps == 0.0 and reduction == "mean":
+            return None
+        return _LossOpts(None if weight is None else weight.contiguous(), eps, reduction)
+
+    def struct(self, per_target=None, grad_per_target=None):
+        return _lib.SrgLossOpts(_lib.ptr(self.weight), self.eps, self.red, _lib.ptr(per_target),
+                                _lib.ptr(grad_per_target))
+
+
 class _NounsLoss(torch.autograd.Function):
     """FCGGNN.nouns_loss (model.py:189-201).  Forward only reads what the loss needs (with the classifier's per-tile
     softmax statistics: the three target logits of a row); the gradient is produced in backward, already multiplied by
-    the incoming d(loss), in one pass over the logits."""
+    the incoming d(loss), in one pass over the logits.  opts (_LossOpts or None): class weights, label smoothing and
+    the reduction; with "none" the loss is [B, 3, R] and backward takes any upstream gradient of that shape."""
 
     @staticmethod
-    def forward(ctx, model, grad_on, logits, gt_nouns, stats, tap, side):
+    def forward(ctx, model, grad_on, logits, gt_nouns, stats, tap, side, opts):
         eng = model._engine_for(logits.device)
         x, rows, ld = _rows_view(logits, eng.L)
         if x.data_ptr() != logits.data_ptr():
             stats = side = None                    # the logits were copied / converted: neither applies
         B = rows // eng.R
         gt = gt_nouns.detach().to(torch.int64).contiguous()
-        # the denominators depend on the targets only: nouns_loss(pred_nouns, gt) and nouns_loss(gt_pred_nouns, gt) of
-        # one step (sr.py:69-70) share them, which also halves the small all-reduces of a sharded step
-        key = (gt.data_ptr(), gt._version, tuple(gt.shape), torch.cuda.current_stream(gt.device).cuda_stream)
-        cached = model._counts_cache
-        if cached is not None and cached[0] == key:
-            counts = cached[1]
-        else:
-            counts = torch.empty(3, dtype=torch.float32, device=logits.device)
-            _lib.check(eng.lib.srg_count_targets(eng.h, _lib.ptr(gt), B, _lib.ptr(counts), eng.stream()))
-            if model.loss_group is not None:
-                torch.distributed.all_reduce(counts, group=model.loss_group)
-            model._counts_cache = (key, counts, gt)     # holding gt keeps its address from being reused
-        loss = torch.zeros((), dtype=torch.float32, device=logits.device)
-        _lib.check(eng.lib.srg_nouns_loss(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), B, _lib.ptr(counts), _lib.ptr(loss),
-                                          None, 1.0, ctypes.c_void_p(stats[1]) if stats else None,
-                                          eng.stream()))
+        counts = None
+        if opts is None or opts.red == _lib.SRG_REDUCTION["mean"]:
+            # the denominators depend on the targets (and the class weights) only: nouns_loss(pred_nouns, gt) and
+            # nouns_loss(gt_pred_nouns, gt) of one step (sr.py:69-70) share them, which also halves the small
+            # all-reduces of a sharded step
+            wkey = None if opts is None else opts.wkey
+            key = (gt.data_ptr(), gt._version, tuple(gt.shape), torch.cuda.current_stream(gt.device).cuda_stream, wkey)
+            cached = model._counts_cache
+            if cached is not None and cached[0] == key:
+                counts = cached[1]
+            else:
+                counts = torch.empty(3, dtype=torch.float32, device=logits.device)
+                if wkey is None:
+                    _lib.check(eng.lib.srg_count_targets(eng.h, _lib.ptr(gt), B, _lib.ptr(counts), eng.stream()))
+                else:
+                    _lib.check(eng.lib.srg_count_targets_weighted(eng.h, _lib.ptr(gt), B, _lib.ptr(opts.weight),
+                                                                  _lib.ptr(counts), eng.stream()))
+                if model.loss_group is not None:
+                    torch.distributed.all_reduce(counts, group=model.loss_group)
+                # holding gt (and the weight) keeps their addresses from being reused
+                model._counts_cache = (key, counts, gt, None if opts is None else opts.weight)
+        st = ctypes.c_void_p(stats[1]) if stats else None
+        if opts is None:
+            loss = torch.zeros((), dtype=torch.float32, device=logits.device)
+            _lib.check(eng.lib.srg_nouns_loss(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), B, _lib.ptr(counts),
+                                              _lib.ptr(loss), None, 1.0, st, eng.stream()))
+        elif opts.reduction == "none":
+            loss = torch.empty(B, 3, eng.R, dtype=torch.float32, device=logits.device)
+            _lib.check(eng.lib.srg_nouns_loss_ex(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), B, _lib.ptr(counts), None, None,
+                                                 1.0, st, ctypes.byref(opts.struct(per_target=loss)), eng.stream()))
+        else:   # the per-target terms are summed in a fixed order: bit-identical losses from call to call
+            loss = torch.zeros((), dtype=torch.float32, device=logits.device)
+            terms = torch.empty(B * 3 * eng.R, dtype=torch.float32, device=logits.device)
+            _lib.check(eng.lib.srg_nouns_loss_ex(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), B, _lib.ptr(counts),
+                                                 _lib.ptr(loss), None, 1.0, st,
+                                                 ctypes.byref(opts.struct(per_target=terms)), eng.stream()))
         if grad_on and (ctx.needs_input_grad[2] or ctx.needs_input_grad[5]):
             ctx.save_for_backward(x, gt, counts)
-            ctx.eng, ctx.geom, ctx.shape, ctx.stats = eng, (rows, ld, B), tuple(logits.shape), stats
+            ctx.eng, ctx.geom, ctx.shape, ctx.stats, ctx.opts = eng, (rows, ld, B), tuple(logits.shape), stats, opts
             ctx.side = side if (side is not None and ctx.needs_input_grad[5] and ld == eng.Lpad) else None
         return loss
 
     @staticmethod
     def backward(ctx, gout):
         x, gt, counts = ctx.saved_tensors
-        eng, (rows, ld, B), stats, side = ctx.eng, ctx.geom, ctx.stats, ctx.side
+        eng, (rows, ld, B), stats, side, opts = ctx.eng, ctx.geom, ctx.stats, ctx.side, ctx.opts
         gout = gout.detach().to(torch.float32).contiguous()
         st = ctypes.c_void_p(stats[1]) if stats else None
         ctx.stats = None
+        per_target = opts is not None and opts.reduction == "none"
+        o = None if opts is None else ctypes.byref(opts.struct(grad_per_target=gout if per_target else None))
+        gscale = None if per_target else _lib.ptr(gout)
         if side is not None:     # straight into the stage's bf16 operand buffer; the tap carries the dependency
-            _lib.check(eng.lib.srg_nouns_loss_backward(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), B, _lib.ptr(counts),
-                                                       _lib.ptr(gout), 1.0, None, ctypes.c_void_p(side.ptr),
-                                                       int(side.written), st, eng.stream()))
+            _lib.check(eng.lib.srg_nouns_loss_backward_ex(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), B, _lib.ptr(counts),
+                                                          gscale, 1.0, None, ctypes.c_void_p(side.ptr),
+                                                          int(side.written), st, o, eng.stream()))
             side.written = True
-            return None, None, None, None, None, gout.new_zeros(1), None
+            return None, None, None, None, None, gout.new_zeros(1), None, None
         dl = torch.empty(rows, ld, dtype=torch.float32, device=x.device)
-        _lib.check(eng.lib.srg_nouns_loss_backward(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), B, _lib.ptr(counts),
-                                                   _lib.ptr(gout), 1.0, _lib.ptr(dl), None, 0, st, eng.stream()))
-        return None, None, dl[:, :eng.L].view(ctx.shape), None, None, None, None
+        _lib.check(eng.lib.srg_nouns_loss_backward_ex(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), B, _lib.ptr(counts),
+                                                      gscale, 1.0, _lib.ptr(dl), None, 0, st, o, eng.stream()))
+        return None, None, dl[:, :eng.L].view(ctx.shape), None, None, None, None, None
 
 
 class _VerbLoss(torch.autograd.Function):
-    """FCGGNN.verb_loss (model.py:182-187); same split between forward and backward as _NounsLoss."""
+    """FCGGNN.verb_loss (model.py:182-187); same split between forward and backward, and the same options, as
+    _NounsLoss ("none": a [B] loss)."""
 
     @staticmethod
-    def forward(ctx, model, grad_on, logits, gt_verb, stats, tap, side):
+    def forward(ctx, model, grad_on, logits, gt_verb, stats, tap, side, opts):
         eng = model._engine_for(logits.device)
         x, rows, ld = _rows_view(logits, eng.V)
         if x.data_ptr() != logits.data_ptr():
             stats = side = None
         gt = gt_verb.detach().to(torch.int64).contiguous()
-        loss = torch.zeros((), dtype=torch.float32, device=logits.device)
         # The mean is over the GLOBAL batch (the reference computes the loss on the gathered logits of all replicas,
         # sr.py:66-68).  Shards may be unequal (tail batch of an epoch), so rows * world is NOT the denominator: the
         # caller states the global batch (model.global_batch), or the local batch sizes are all-reduced on the stream.
+        # With class weights the denominator is the global sum of the targets' weights, which only the all-reduce of
+        # the local sums gives.
         inv, total = 1.0 / rows, None
-        if model.loss_group is not None:
+        if opts is not None and opts.weight is not None and opts.red == _lib.SRG_REDUCTION["mean"]:
+            total = torch.empty(1, dtype=torch.float32, device=logits.device)
+            _lib.check(eng.lib.srg_verb_weight_total(eng.h, _lib.ptr(gt), rows, _lib.ptr(opts.weight),
+                                                     _lib.ptr(total), eng.stream()))
+            if model.loss_group is not None:
+                torch.distributed.all_reduce(total, group=model.loss_group)
+        elif model.loss_group is not None and (opts is None or opts.red == _lib.SRG_REDUCTION["mean"]):
             if model.global_batch is not None:
                 inv = 1.0 / float(model.global_batch)
             else:
                 total = torch.full((1,), float(rows), dtype=torch.float32, device=logits.device)
                 torch.distributed.all_reduce(total, group=model.loss_group)
-        _lib.check(eng.lib.srg_verb_loss(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), rows, inv, _lib.ptr(total),
-                                         _lib.ptr(loss), None, 1.0, ctypes.c_void_p(stats[1]) if stats else None,
-                                         eng.stream()))
+        st = ctypes.c_void_p(stats[1]) if stats else None
+        if opts is None:
+            loss = torch.zeros((), dtype=torch.float32, device=logits.device)
+            _lib.check(eng.lib.srg_verb_loss(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), rows, inv, _lib.ptr(total),
+                                             _lib.ptr(loss), None, 1.0, st, eng.stream()))
+        elif opts.reduction == "none":
+            loss = torch.empty(rows, dtype=torch.float32, device=logits.device)
+            _lib.check(eng.lib.srg_verb_loss_ex(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), rows, inv, _lib.ptr(total), None,
+                                                None, 1.0, st, ctypes.byref(opts.struct(per_target=loss)),
+                                                eng.stream()))
+        else:
+            loss = torch.zeros((), dtype=torch.float32, device=logits.device)
+            terms = torch.empty(rows, dtype=torch.float32, device=logits.device)
+            _lib.check(eng.lib.srg_verb_loss_ex(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), rows, inv, _lib.ptr(total),
+                                                _lib.ptr(loss), None, 1.0, st,
+                                                ctypes.byref(opts.struct(per_target=terms)), eng.stream()))
         if grad_on and (ctx.needs_input_grad[2] or ctx.needs_input_grad[5]):
             saved = (x, gt) if total is None else (x, gt, total)
             ctx.save_for_backward(*saved)
-            ctx.eng, ctx.geom, ctx.shape, ctx.stats = eng, (rows, ld, inv), tuple(logits.shape), stats
+            ctx.eng, ctx.geom, ctx.shape, ctx.stats, ctx.opts = eng, (rows, ld, inv), tuple(logits.shape), stats, opts
             ctx.side = side if (side is not None and ctx.needs_input_grad[5] and ld == eng.Vpad) else None
         return loss
 
@@ -567,20 +650,23 @@ class _VerbLoss(torch.autograd.Function):
     def backward(ctx, gout):
         x, gt, *rest = ctx.saved_tensors
         total = rest[0] if rest else None
-        eng, (rows, ld, inv), stats, side = ctx.eng, ctx.geom, ctx.stats, ctx.side
+        eng, (rows, ld, inv), stats, side, opts = ctx.eng, ctx.geom, ctx.stats, ctx.side, ctx.opts
         gout = gout.detach().to(torch.float32).contiguous()
         st = ctypes.c_void_p(stats[1]) if stats else None
         ctx.stats = None
+        per_target = opts is not None and opts.reduction == "none"
+        o = None if opts is None else ctypes.byref(opts.struct(grad_per_target=gout if per_target else None))
+        gscale = None if per_target else _lib.ptr(gout)
         if side is not None:
-            _lib.check(eng.lib.srg_verb_loss_backward(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), rows, inv, _lib.ptr(total),
-                                                      _lib.ptr(gout), 1.0, None, ctypes.c_void_p(side.ptr),
-                                                      int(side.written), st, eng.stream()))
+            _lib.check(eng.lib.srg_verb_loss_backward_ex(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), rows, inv,
+                                                         _lib.ptr(total), gscale, 1.0, None, ctypes.c_void_p(side.ptr),
+                                                         int(side.written), st, o, eng.stream()))
             side.written = True
-            return None, None, None, None, None, gout.new_zeros(1), None
+            return None, None, None, None, None, gout.new_zeros(1), None, None
         dl = torch.empty(rows, ld, dtype=torch.float32, device=x.device)
-        _lib.check(eng.lib.srg_verb_loss_backward(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), rows, inv, _lib.ptr(total),
-                                                  _lib.ptr(gout), 1.0, _lib.ptr(dl), None, 0, st, eng.stream()))
-        return None, None, dl[:, :eng.V].view(ctx.shape), None, None, None, None
+        _lib.check(eng.lib.srg_verb_loss_backward_ex(eng.h, _lib.ptr(x), ld, _lib.ptr(gt), rows, inv, _lib.ptr(total),
+                                                     gscale, 1.0, _lib.ptr(dl), None, 0, st, o, eng.stream()))
+        return None, None, dl[:, :eng.V].view(ctx.shape), None, None, None, None, None
 
 
 def _has_batchnorm_in_train(module):
@@ -647,7 +733,7 @@ class FCGGNN(nn.Module):
         self._flat = None                # parallel.attach(): flat gradient / parameter buffers
         self._last_stats = None
         self._last_side = None
-        self._counts_cache = None        # (key, counts, targets) of the last nouns_loss call
+        self._counts_cache = None        # (key, counts, targets, weight) of the last nouns_loss call
 
     # sr.py accesses model.module.* when CUDA is available (DataParallel wrapper in the reference)
     @property
@@ -826,18 +912,31 @@ class FCGGNN(nn.Module):
         tp = getattr(logits, "_srg_tap", None) if stats is not None else None
         return tp if tp is not None else (None, None)
 
-    def verb_loss(self, pred_verb, gt_verb):
+    def verb_loss(self, pred_verb, gt_verb, weight=None, label_smoothing=0.0, reduction="mean"):
+        """CrossEntropy(pred_verb [B, n_verbs], gt_verb [B]) (model.py:182-187) with the keywords of
+        F.cross_entropy: class weights [n_verbs] (data: they must not require grad), label smoothing in [0, 1] and the
+        reduction ("none" gives the [B] per-image losses).  The mean is over the global batch under `loss_group`,
+        weighted: sum of weight[gt_verb] over all ranks.  A zero denominator gives 0 where torch gives NaN."""
+        opts = _LossOpts.make(weight, label_smoothing, reduction, self.encoder.get_num_verbs(), pred_verb.device,
+                              "verb_loss")
         eng_pad = _pad256(self.encoder.get_num_verbs())
         stats = self._stats_ptr(pred_verb, eng_pad) if pred_verb.dim() == 2 else None
         tap, side = self._tap_of(pred_verb, stats)
-        return _VerbLoss.apply(self, torch.is_grad_enabled(), pred_verb, gt_verb.to(pred_verb.device), stats, tap, side)
+        return _VerbLoss.apply(self, torch.is_grad_enabled(), pred_verb, gt_verb.to(pred_verb.device), stats, tap, side,
+                               opts)
 
-    def nouns_loss(self, pred_nouns, gt_nouns):
+    def nouns_loss(self, pred_nouns, gt_nouns, weight=None, label_smoothing=0.0, reduction="mean"):
+        """Sum over the 3 annotations of CrossEntropy(ignore_index = n_labels) (model.py:189-201), with the keywords
+        of F.cross_entropy as verb_loss: weight [n_labels]; "mean" is taken per annotation (denominator: the global
+        sum of weight[y] over its non-ignored targets) and summed; "none" gives [B, 3, R] laid out like gt_nouns, 0 on
+        ignored targets."""
+        opts = _LossOpts.make(weight, label_smoothing, reduction, self.encoder.get_num_labels(), pred_nouns.device,
+                              "nouns_loss")
         eng_pad = _pad256(self.encoder.get_num_labels())
         stats = self._stats_ptr(pred_nouns, eng_pad) if pred_nouns.dim() == 3 else None
         tap, side = self._tap_of(pred_nouns, stats)
         return _NounsLoss.apply(self, torch.is_grad_enabled(), pred_nouns, gt_nouns.to(pred_nouns.device), stats, tap,
-                                side)
+                                side, opts)
 
     # ---- top-k situation decode ----------------------------------------------------------------
     @torch.no_grad()

@@ -20,7 +20,9 @@ ways.  Differences, all forced by the B200-first design:
   * `--finetune_backbone` (extra flag) trains both ResNet-152 backbones with the GGNN stage (bf16 only; the dev
     feature cache is off, and a checkpoint resumes only under the setting it was trained with);
   * `--nbest_situations N` (extra flag, with --test_img) prints the N highest-scoring situations, which may share a
-    verb, and whether that list is certified to be the N best over all verbs.
+    verb, and whether that list is certified to be the N best over all verbs;
+  * `--label_smoothing EPS` and `--class_weights FILE` (extra flags) change the training objective to
+    F.cross_entropy(weight=..., label_smoothing=EPS) on both losses; the logged dev losses stay the plain ones.
 """
 import os
 from argparse import ArgumentParser
@@ -87,9 +89,32 @@ def _global_sizes(loader):
     return sampler.global_sizes() if hasattr(sampler, "global_sizes") else None
 
 
+def load_class_weights(path, encoder):
+    """The class weights of --class_weights: a torch.save'd dict with the optional keys "verb" (fp32 [n_verbs]) and
+    "nouns" (fp32 [n_labels]), indexed by the encoder's verb and label ids.  Returns (verb, nouns), None where absent;
+    raises ValueError when the file does not fit the encoder."""
+    d = torch.load(path, map_location="cpu", weights_only=True)
+    if not isinstance(d, dict) or not set(d) <= {"verb", "nouns"}:
+        raise ValueError("%s: expected a dict with the keys 'verb' and / or 'nouns'" % path)
+    out = []
+    for key, n in (("verb", encoder.get_num_verbs()), ("nouns", encoder.get_num_labels())):
+        w = d.get(key)
+        if w is not None:
+            w = torch.as_tensor(w, dtype=torch.float32)
+            if tuple(w.shape) != (n,):
+                raise ValueError("%s: '%s' weights have shape %s, the encoder has %d classes" %
+                                 (path, key, tuple(w.shape), n))
+            if not torch.isfinite(w).all() or (w < 0).any():
+                raise ValueError("%s: '%s' weights must be finite and non-negative" % (path, key))
+        out.append(w)
+    return tuple(out)
+
+
 def train(model, train_loader, dev_loader, optimizer, max_epoch, encoder, model_saving_name, folder, checkpoint=None,
-          flat=None, plot=True, dev_cache=None):
-    """sr.py:15-162."""
+          flat=None, plot=True, dev_cache=None, verb_loss_kwargs=None, nouns_loss_kwargs=None):
+    """sr.py:15-162.  verb_loss_kwargs / nouns_loss_kwargs: the training objective's weight / label_smoothing (the
+    dev losses stay the reference's plain ones)."""
+    vkw, nkw = verb_loss_kwargs or {}, nouns_loss_kwargs or {}
     model.train()
     hist = {k: [] for k in ('avg_scores', 'verb_losses', 'nouns_losses', 'val_avg_scores', 'val_verb_losses',
                             'val_nouns_losses')}
@@ -125,9 +150,9 @@ def train(model, train_loader, dev_loader, optimizer, max_epoch, encoder, model_
             model.global_batch = sizes[step] if sizes is not None else None
             flat.zero()
             pred_verb, pred_nouns, pred_gt_nouns = model(img, verb)
-            verb_loss = model.verb_loss(pred_verb, verb)
-            nouns_loss = model.nouns_loss(pred_nouns, nouns)
-            gt_nouns_loss = model.nouns_loss(pred_gt_nouns, nouns)
+            verb_loss = model.verb_loss(pred_verb, verb, **vkw)
+            nouns_loss = model.nouns_loss(pred_nouns, nouns, **nkw)
+            gt_nouns_loss = model.nouns_loss(pred_gt_nouns, nouns, **nkw)
             (verb_loss + nouns_loss).backward()
             if not sharded:
                 flat.all_reduce()
@@ -428,6 +453,14 @@ def build_parser():
     parser.add_argument("--nbest_situations", type=int, default=None,
                         help="with --test_img: also print the N best situations (1 <= N <= 16), which may share a verb, "
                              "and whether the list is certified to be the N best over all verbs")
+    parser.add_argument("--label_smoothing", type=float, default=0.0,
+                        help="label smoothing EPS in [0, 1] of the training objective's verb and noun losses (as "
+                             "nn.CrossEntropyLoss(label_smoothing=EPS)); the logged dev losses stay the plain ones, "
+                             "comparable across runs")
+    parser.add_argument("--class_weights", type=str, default="",
+                        help="torch.save'd dict with optional keys 'verb' [n_verbs] and 'nouns' [n_labels]: class weights "
+                             "of the training objective (tools/make_class_weights.py writes one); the logged dev losses "
+                             "stay unweighted")
     return parser
 
 
@@ -450,6 +483,8 @@ def main(argv=None):
             parser.error("--nbest_situations must be in [1, 16], got %d" % args.nbest_situations)
         if not args.test_img:
             parser.error("--nbest_situations needs --test_img")
+    if not 0.0 <= args.label_smoothing <= 1.0:
+        parser.error("--label_smoothing must be in [0, 1], got %g" % args.label_smoothing)
     if args.finetune_backbone and args.precision == "fp32":
         parser.error("--finetune_backbone needs --precision bf16 (precision fp32 is a forward-only parity mode)")
     if not torch.cuda.is_available():
@@ -479,6 +514,7 @@ def main(argv=None):
         _print0("Loading encoder file")
         encoder = torch.load(enc_path, weights_only=False)
 
+    verb_w, nouns_w = load_class_weights(args.class_weights, encoder) if args.class_weights else (None, None)
     train_set = imsitu_loader(args.imgset_dir, train_json, encoder, encoder.train_transform)
     dev_set = imsitu_loader(args.imgset_dir, dev_json, encoder, encoder.dev_transform)
     test_set = imsitu_loader(args.imgset_dir, test_json, encoder, encoder.dev_transform)
@@ -546,8 +582,11 @@ def main(argv=None):
         analize_subset(model, dev_set, encoder, args.subset, args.dataset_folder, args.imgset_dir)
     else:
         _print0('Model training started!')
+        objective = [{"label_smoothing": args.label_smoothing, "weight": None if w is None else w.to(dev)}
+                     for w in (verb_w, nouns_w)]
         train(model, train_loader, dev_loader, optimizer, args.epochs, encoder, args.model_saving_name,
-              folder=args.saving_folder, checkpoint=checkpoint, flat=flat, dev_cache=dev_cache)
+              folder=args.saving_folder, checkpoint=checkpoint, flat=flat, dev_cache=dev_cache,
+              verb_loss_kwargs=objective[0], nouns_loss_kwargs=objective[1])
     if world > 1:
         dist.destroy_process_group()
 
