@@ -155,8 +155,9 @@ def gate_stats(g):
 
 
 def oracle_step(params, batch, tabs, pred_verbs=None, keeps=(None, None, None), feat_grad=False,
-                dtype=torch.float64, device="cpu"):
-    """sr.py's training step (verb_loss + nouns_loss of the predicted-verb path) under fp64 autograd of the oracle.
+                dtype=torch.float64, device="cpu", num_labels=NUM_LABELS):
+    """sr.py's training step (verb_loss + nouns_loss of the predicted-verb path) under fp64 autograd of the oracle;
+    num_labels is the vocabulary size, the noun targets' ignore label.
     Returns (losses (verb, nouns, gt nouns), {param: grad}, logits (verb, pred nouns, gt nouns), (dfeat_v, dfeat_n))."""
     fv, fn, gt_verb, gt_nouns = batch
     t, c = tabs
@@ -166,7 +167,7 @@ def oracle_step(params, batch, tabs, pred_verbs=None, keeps=(None, None, None), 
     kp = tuple(None if k is None else k.to(device) for k in keeps)
     gv, gn = gt_verb.to(device), gt_nouns.to(device)
     pv, pn, gpn = O.forward(ps, xv, xn, gv, t, c, kp, 0.5, None if pred_verbs is None else pred_verbs.to(device))
-    vl, nl, gl = O.verb_loss(pv, gv), O.nouns_loss(pn, gn, NUM_LABELS), O.nouns_loss(gpn, gn, NUM_LABELS)
+    vl, nl, gl = O.verb_loss(pv, gv), O.nouns_loss(pn, gn, num_labels), O.nouns_loss(gpn, gn, num_labels)
     (vl + nl).backward()
     grads = {k: (v.grad if v.grad is not None else torch.zeros_like(v)) for k, v in ps.items()}
     return ((vl.detach(), nl.detach(), gl.detach()), grads, (pv.detach(), pn.detach(), gpn.detach()),
